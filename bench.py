@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the DINO-Soft loss hot path (fwd + bwd), BASELINE.json's metric.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 N = 1 (default): global batch B = 32768 (BASELINE config 3's batch, which fits one B200 because the
 B x B logits are never materialised), D = 512, DINO dim 768, MLP projection head, text-symmetric soft
@@ -18,6 +18,10 @@ SURVEY.md 2a names.  `--impl reference` times only the CPU reference.
 
 Other BASELINE configs: `--batch 4096` (config 2), `--clip-dim 768 --dino-dim 1024 --no-head --batch 65536`
 under torchrun with 8 ranks (config 4).
+
+`--dump-outputs DIR` writes what the last timed step returned on rank 0 (the loss terms and the gradients of the
+image / text features, the logit scale and the head parameters) as DIR/<name>.npy in float32.  The inputs are
+seeded, so two builds run with the same arguments can be compared array for array.
 """
 from __future__ import annotations
 
@@ -37,6 +41,7 @@ import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the benchmark leaves the tree as it found it (it may be read-only)
 
 METRIC = "dino_soft_loss_fwd_bwd_samples_per_sec"
 GLOBAL_B, D_CLIP, D_DINO = 32768, 512, 768
@@ -252,6 +257,38 @@ def load_ncu_traffic():
     return out
 
 
+DUMP_ROWS = 4096  # rows kept of a per-sample gradient: 8 MB at D = 512 (the full one is 64 MB at B = 32768)
+DUMP_MAX_BYTES = 64_000_000
+
+
+def snapshot_outputs(out, leaves):
+    """Host float32 copies of what the caller of a step receives: the loss terms of `out` and the gradients of the
+    (name, tensor) `leaves`.  A gradient with more than DUMP_ROWS rows keeps a fixed seeded sample of its rows, in
+    ascending order, so that two runs keep the same rows."""
+    arrays = {k: out[k] for k in ("total_loss", "classic_loss", "soft_loss", "weighted_loss") if k in out}
+    for name, t in leaves:
+        g = t.grad
+        if g is None:
+            continue
+        if g.dim() > 0 and g.shape[0] > DUMP_ROWS:
+            rows = torch.randperm(g.shape[0], generator=torch.Generator().manual_seed(0))[:DUMP_ROWS].sort().values
+            g = g[rows.to(g.device)]
+        arrays["grad_" + name] = g
+    arrays = {k: v.detach().float().cpu().numpy() for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_MAX_BYTES:
+        raise SystemExit(f"--dump-outputs: {total} bytes of outputs, more than {DUMP_MAX_BYTES}")
+    return arrays
+
+
+def write_outputs(directory, arrays):
+    import numpy as np
+
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), a)
+
+
 # --------------------------------------------------------------------------------------------------
 # clocks sampler
 # --------------------------------------------------------------------------------------------------
@@ -429,6 +466,12 @@ def run_ours(args):
         print(f"[bench] rank {rank}: headline {ms / args.steps:.4f} ms/step, host enqueue {host_ms / args.steps:.4f} "
               "ms/step", file=sys.stderr)
     final_loss = float(out["total_loss"].detach())
+    dumped = None
+    if args.dump_outputs and rank == 0:  # before the passes below overwrite the gradients
+        leaves = [("image", img), ("text", txt), ("logit_scale", scale)]
+        if USE_HEAD:
+            leaves += [("head_" + n.replace(".", "_"), p) for n, p in loss.image_to_dino_proj.named_parameters()]
+        dumped = snapshot_outputs(out, leaves)
 
     # ---- per-kernel pass (same inputs, same loop, clocks still sampled): the product launches the independent
     # tile kernels of a pass on forked streams so they fill each other's last wave; CUDA events around a kernel
@@ -628,6 +671,8 @@ def run_ours(args):
             "gpu_eager_baseline": gpu_eager,
             "loss": final_loss,
         }
+        if dumped is not None:
+            write_outputs(args.dump_outputs, dumped)
         if stdout_fd is not None:
             sys.stdout.flush()
             os.dup2(stdout_fd, 1)
@@ -661,7 +706,14 @@ def main():
                     help="replay the loss forward / backward as CUDA graphs (dinosoft_b200.make_graphed); default: "
                          "only where the step is host-bound (per-rank block <= 2^28 similarity entries)")
     ap.add_argument("--no-graph", action="store_true", help="always time the eager step")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the loss terms and gradients of the last timed step as DIR/<name>.npy (float32; "
+                         f"gradients with more than {DUMP_ROWS} rows keep a fixed seeded sample of rows)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     GLOBAL_B, D_CLIP, D_DINO, USE_HEAD = args.batch, args.clip_dim, args.dino_dim, not args.no_head
     if args.impl == "reference":
         run_reference_arm(args)
