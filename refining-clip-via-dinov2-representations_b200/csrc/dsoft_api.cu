@@ -52,7 +52,6 @@ struct dsoft_plan {
   int have_soft, have_text, have_proj, soft_local, row_only;
   int fwd_sym;         // world == 1 and fast_t: the soft forward computes the upper block triangle only
   int clip_sym;        // world == 1: one CLIP forward pass serves both directions (MODE_CLIP_SYM)
-  int sym16;           // symmetric soft forward with the 16x256b TMEM load shape (MODE_SOFT_SYM16; DSOFT_SYM16)
   // world > 1, global soft scope (DSOFT_SYM_W): the soft Gram matrices are symmetric, so every pair of row blocks
   // is computed by ONE of its two ranks.  Rank r owns, in column coordinates relative to its own first row
   // ("primed"), the blocks [0, W/2) - its diagonal block first - plus half of the contested block W/2 (ranks below
@@ -259,13 +258,8 @@ extern "C" int dsoft_plan_create(const dsoft_shape_t* sh, dsoft_plan_t** out) {
   p->f_wce = choose_split(rbs, 1, ceil_div(p->B, 2 * BN), sms);
   {
     // symmetric forward: needs one rank (the row block is the whole square), the fixed teacher maximum, and more
-    // than one row pair (otherwise there is nothing to save); DSOFT_FWD_SYM=0 keeps the full-square kernel
-    const char* e = getenv("DSOFT_FWD_SYM");
-    p->fwd_sym = soft && (sh->world == 1 || p->sym_w) && p->fast_t && rbs > 2 && !(e && e[0] == '0');
-    if (p->sym_w && !p->fwd_sym) p->sym_w = 0;  // (cannot happen: b % 512 == 0 gives rbs >= 4)
-    // the symmetric forward with the 16x256b TMEM load shape (MODE_SOFT_SYM16); DSOFT_SYM16=0: the 32x32b form
-    const char* e16 = getenv("DSOFT_SYM16");
-    p->sym16 = p->fwd_sym && !(e16 && e16[0] == '0');
+    // than one row pair (otherwise there is nothing to save)
+    p->fwd_sym = soft && (sh->world == 1 || p->sym_w) && p->fast_t && rbs > 2;
     p->f_sym.tps = std::max(4, ceil_div(p->ntiles_s, 10));
     p->f_sym.nsplit = ceil_div(p->ntiles_s, p->f_sym.tps);
   }
@@ -2221,8 +2215,7 @@ static int forward_impl(const dsoft_plan_t* p, const void* gathered, const float
     P.part = X + p->sc_ps;
     if ((rc = fk.lane(lane++, &ks))) return rc;
     if (p->fwd_sym) {
-      // world == 1: upper block triangle only, the other half through column reductions (MODE_SOFT_SYM)
-      if ((rc = set_smem(dsoft_fwd_kernel<MODE_SOFT_SYM, 2>, FWD_SMEM_BYTES))) return rc;
+      // upper block triangle only, the other half through column reductions (dsoft_fwd_kernel<MODE_SOFT_SYM16>)
       if ((rc = set_smem(dsoft_fwd_kernel<MODE_SOFT_SYM16, 2>, FWD_SMEM_BYTES))) return rc;
       P.tri = 1;
       P.tiles_per_split = p->f_sym.tps;
@@ -2236,9 +2229,7 @@ static int forward_impl(const dsoft_plan_t* p, const void* gathered, const float
         P.ntiles_a = p->sw_ncols_a / (2 * BN);
       }
       ProfScope ps(PK_FWD_SOFT, ks);
-      if ((rc = p->sym16 ? launch_fwd_pair(dsoft_fwd_kernel<MODE_SOFT_SYM16, 2>, rbs, p->f_sym.nsplit, ks, tm, P)
-                         : launch_fwd_pair(dsoft_fwd_kernel<MODE_SOFT_SYM, 2>, rbs, p->f_sym.nsplit, ks, tm, P)))
-        return rc;
+      if ((rc = launch_fwd_pair(dsoft_fwd_kernel<MODE_SOFT_SYM16, 2>, rbs, p->f_sym.nsplit, ks, tm, P))) return rc;
       // column sums by PRIMED column: [0, b) are this rank's own rows, the rest belongs to the ranks behind it
       soft_colreduce_kernel<<<dim3(p->Bcol / 32, 6), dim3(32, 16), 0, ks>>>(
           X + p->sc_colpart, 4 * rbs, p->Bcol, p->s_ncols, X + p->sc_colsum, p->sym_w ? p->sw_ncols_a : p->s_ncols,

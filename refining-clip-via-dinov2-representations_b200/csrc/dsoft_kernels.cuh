@@ -51,8 +51,8 @@ constexpr int MODE_WCE_STAT = 5;
 constexpr int MODE_WCE_LSE = 6;
 constexpr int MODE_WCE_DBG = 7;
 constexpr int MODE_WCE_G = 8;
-constexpr int MODE_SOFT_SYM = 9;  // forward soft statistics, world == 1: upper block triangle + column reductions
-constexpr int MODE_SOFT_SYM16 = 13;  // the same with a 16x256b TMEM load shape (4 rows per thread: short butterflies)
+constexpr int MODE_SOFT_SYM16 = 13;  // forward soft statistics, upper block triangle + column reductions, on a
+                                     // 16x256b TMEM load shape (4 rows per thread: short butterflies)
 constexpr int MODE_LINEAR = 11;   // projection head layer: out = act(A . W^T + bias) as bf16 (loss.py:214-238, 322-347)
 constexpr int MODE_PAIRS = 12;    // CLIP-blind pair statistics (open_clip_train/helpers.py:221-285): threshold counts
                                   // and candidate pairs over the upper triangle of two Gram matrices
@@ -128,7 +128,7 @@ struct FwdParams {
   int wsym;                 // weight_text_symmetry (loss.py:449-463)
   float wcc;                // c_clip
   const float* wgout;       // G mode: upstream gradients [6] (device)
-  // ---- symmetric forward (MODE_SOFT_SYM): column partials [6][cp_rows = 4 * row blocks][cp_pitch]
+  // ---- symmetric forward (MODE_SOFT_SYM16): column partials [6][cp_rows = 4 * row blocks][cp_pitch]
   float* colpart;
   int cp_rows, cp_pitch;
   // ---- one-pass CLIP forward (MODE_CLIP_SYM): column partials (reference exponent, sum) [cp_rows][cp_pitch] each,
@@ -214,34 +214,12 @@ __device__ __forceinline__ void st_cs_v8(void* dst, const uint32_t (&w)[8]) {
 
 // Packed fp32 pairs (sm_100 FFMA2 / FMUL2 / FADD2: one issue slot and one pass through the FMA pipe for two lanes'
 // worth of work).  The epilogues are issue-bound (two epilogue warps per scheduler next to the MMA stream), so their
-// element loops are written over column PAIRS.  -DDSOFT_PACKED_F32=0 compiles the same loops with scalar operations
-// (A/B arm; results agree up to the summation order, which is the same in both builds).
-#ifndef DSOFT_PACKED_F32
-#define DSOFT_PACKED_F32 1
-#endif
+// element loops are written over column PAIRS.
 __device__ __forceinline__ float2 pk(float a, float b) { return make_float2(a, b); }
 __device__ __forceinline__ float2 pk1(float a) { return make_float2(a, a); }
-__device__ __forceinline__ float2 pk_mul(float2 a, float2 b) {
-#if DSOFT_PACKED_F32
-  return __fmul2_rn(a, b);
-#else
-  return make_float2(a.x * b.x, a.y * b.y);
-#endif
-}
-__device__ __forceinline__ float2 pk_add(float2 a, float2 b) {
-#if DSOFT_PACKED_F32
-  return __fadd2_rn(a, b);
-#else
-  return make_float2(a.x + b.x, a.y + b.y);
-#endif
-}
-__device__ __forceinline__ float2 pk_fma(float2 a, float2 b, float2 c) {
-#if DSOFT_PACKED_F32
-  return __ffma2_rn(a, b, c);
-#else
-  return make_float2(fmaf(a.x, b.x, c.x), fmaf(a.y, b.y, c.y));
-#endif
-}
+__device__ __forceinline__ float2 pk_mul(float2 a, float2 b) { return __fmul2_rn(a, b); }
+__device__ __forceinline__ float2 pk_add(float2 a, float2 b) { return __fadd2_rn(a, b); }
+__device__ __forceinline__ float2 pk_fma(float2 a, float2 b, float2 c) { return __ffma2_rn(a, b, c); }
 __device__ __forceinline__ float2 pk_exp2(float2 a) { return make_float2(fast_exp2(a.x), fast_exp2(a.y)); }
 
 // Column sums over the 32 rows of a warp: every lane holds x[k] = the value of ITS row in column k; lane l returns
@@ -376,8 +354,7 @@ dsoft_fwd_kernel(const __grid_constant__ TileMaps maps, const __grid_constant__ 
   constexpr bool kWce = (MODE >= MODE_WCE_STAT && MODE <= MODE_WCE_G);
   // "soft-like": 256-column tiles with several products per tile, staged per-column vectors, setmaxnreg
   constexpr bool kPairs = (MODE == MODE_PAIRS);  // two products per tile like the weighted-CE passes, no column vectors
-  constexpr bool kSoftMode = (MODE == MODE_SOFT || MODE == MODE_SOFT_G || MODE == MODE_SOFT_SYM ||
-                              MODE == MODE_SOFT_SYM16 || kWce || kPairs);
+  constexpr bool kSoftMode = (MODE == MODE_SOFT || MODE == MODE_SOFT_G || MODE == MODE_SOFT_SYM16 || kWce || kPairs);
   static_assert(!kSoftMode || CG == 2, "the soft modes are written for CTA pairs");
   // streaming mode: stages of (A box | B boxes); resident mode: 8 A boxes, then B-only stages
   const bool resident = P.resident != 0;
@@ -1446,14 +1423,23 @@ dsoft_fwd_kernel(const __grid_constant__ TileMaps maps, const __grid_constant__ 
       }
     } else if constexpr (MODE == MODE_SOFT_SYM16) {
       // ---------------------------------------------------------------- symmetric forward, 16x256b TMEM loads
-      // Same statistics as MODE_SOFT_SYM below (read its comment first), other register layout: tcgen05.ld
-      // 16x256b gives every thread FOUR rows (g, g + 8, g + 16, g + 24 of the warp's 32; g = lane / 4) and, per
-      // 32-column chunk, the columns 8 j + 2 c2 + {0, 1} (j = 0..3, c2 = lane % 4).  The column sums over the warp's
-      // rows then start with three in-register adds per column and need a three-stage butterfly over the eight row
-      // groups (warp_colsum8: 7 shuffles + 14 selects per quantity and chunk) instead of the five-stage one over 32
-      // lanes (31 + 62), which was about half of the MODE_SOFT_SYM epilogue.  Row sums: every thread accumulates its
-      // four rows per product and tile, the four lanes of a row group combine them (two xor stages) and lane c2 keeps
-      // row g + 8 c2, so the persistent accumulators stay one row per thread.
+      // The teacher, student and text Gram matrices are symmetric, so a row pair only computes the tiles from its
+      // own diagonal tile onwards (P.tri).  A tile right of the diagonal also holds, transposed, the entries the
+      // rows of its COLUMN block need: every quantity is summed over the 32 rows of a warp per column and written
+      // as a column partial [k][rb * 4 + q][column]; soft_colreduce_kernel adds those to the row partials.  All
+      // exponentials use FIXED maxima (teacher: log2(e)/tau_t, valid because fast_t bounds it by 60; student /
+      // text: log2(e)/tau, reached on the diagonal), so row and column partials share one reference and no running
+      // maximum has to be reconciled.  Exponent arguments come out of ONE fma: arg = dot * (row factor * column
+      // factor) - M, with M = NEG_BIG for a dead row (rows past b: 2^arg = 0 without a select, so they never reach
+      // the column sums).  The weighted sums are kept relative to the fixed maxima, sum w (q - M_t) etc.;
+      // finalize_fwd adds M * Zt back.
+      // Register layout: tcgen05.ld 16x256b gives every thread FOUR rows (g, g + 8, g + 16, g + 24 of the warp's 32;
+      // g = lane / 4) and, per 32-column chunk, the columns 8 j + 2 c2 + {0, 1} (j = 0..3, c2 = lane % 4).  The
+      // column sums over the warp's rows then start with three in-register adds per column and need a three-stage
+      // butterfly over the eight row groups (warp_colsum8: 7 shuffles + 14 selects per quantity and chunk) instead of
+      // the five-stage one over 32 lanes that the 32x32b shape needs (31 + 62).  Row sums: every thread accumulates
+      // its four rows per product and tile, the four lanes of a row group combine them (two xor stages) and lane c2
+      // keeps row g + 8 c2, so the persistent accumulators stay one row per thread.
       const float mt2 = P.scal[SC_ITT_L2], ms2 = P.scal[SC_ITS_L2], mx2 = P.scal[SC_ITX_L2];
       const int g = lane >> 2, c2 = lane & 3;
       const int wrow0 = rb * BM + q * 32;  // first local row of this warp
@@ -1568,7 +1554,7 @@ dsoft_fwd_kernel(const __grid_constant__ TileMaps maps, const __grid_constant__ 
             if (offdiag) {  // warp-uniform
               const float s0 = warp_colsum8(cs0, lane);
               const float s1 = warp_colsum8(cs1, lane);
-              // quantities as in MODE_SOFT_SYM: [0] teacher sum, [1] sum w q, [2] sum w p, [3] sum w r,
+              // column partial quantities: [0] teacher sum, [1] sum w q, [2] sum w p, [3] sum w r,
               // [4] student sum, [5] text sum
               const int k0 = kT ? 0 : ((p == 1) ? 4 : 5);
               const int k1 = kT ? 1 : ((p == 1) ? 2 : 3);
@@ -1586,168 +1572,6 @@ dsoft_fwd_kernel(const __grid_constant__ TileMaps maps, const __grid_constant__ 
       const int myrow = wrow0 + g + 8 * c2;
       if (myrow < P.b) {  // same partial layout as MODE_SOFT; the maximum is the fixed one
         const int o = sp * P.b + myrow;
-        const int st = P.npart * P.b;
-        P.part[0 * st + o] = mt2;
-        P.part[1 * st + o] = zt;
-        P.part[2 * st + o] = aq;
-        P.part[3 * st + o] = ap;
-        P.part[4 * st + o] = ar;
-        P.part[5 * st + o] = zs;
-        P.part[6 * st + o] = zx;
-      }
-    } else if constexpr (MODE == MODE_SOFT_SYM) {
-      // ---------------------------------------------------------------- symmetric forward (world == 1)
-      // The teacher, student and text Gram matrices are symmetric, so a row pair only computes the tiles from its
-      // own diagonal tile onwards (P.tri).  A tile right of the diagonal also holds, transposed, the entries the
-      // rows of its COLUMN block need: every quantity is summed over the 32 rows of a warp per column (warp
-      // butterfly, warp_colsum32) and written as a column partial [k][rb * 4 + q][column]; soft_colreduce_kernel
-      // adds those to the row partials.  All exponentials use FIXED maxima (teacher: log2(e)/tau_t, valid because
-      // fast_t bounds it by 60; student / text: log2(e)/tau, reached on the diagonal), so row and column partials
-      // share one reference and no running maximum has to be reconciled.
-      const float mt2 = P.scal[SC_ITT_L2], ms2 = P.scal[SC_ITS_L2], mx2 = P.scal[SC_ITX_L2];
-      const float cq = P.rinv[0][gi] * mt2;
-      const float cp = P.rinv[1][gi] * ms2;
-      const bool has_text = P.nprod == 3;
-      const float cr = has_text ? P.rinv[2][gi] * mx2 : 0.f;
-      const bool live_row = li < P.b;  // rows past b (zero operands) must not reach the column sums
-      // exponent arguments come out of ONE fma: arg = dot * (row factor * column factor) - M, with M = -1e30 for a
-      // dead row (2^arg = 0 without a select).  The weighted sums are kept relative to the fixed maxima,
-      // sum w (q - M_t) etc.; finalize_fwd adds M * Zt back.
-      const float bias_t = live_row ? -mt2 : NEG_BIG;
-      const float2 cq2 = pk1(cq), bias_t2 = pk1(bias_t);
-      float2 zt2 = pk1(0.f), aq2 = pk1(0.f);  // even / odd columns
-      float ap = 0.f, ar = 0.f, zs = 0.f, zx = 0.f;
-      float w[128];  // teacher weights 2^(q - M_t) of this thread's 128 columns, kept across the three products
-      const size_t cp_stride = static_cast<size_t>(P.cp_rows) * P.cp_pitch;  // one quantity of the column partials
-      float* cp_row = P.colpart + static_cast<size_t>(rb * 4 + q) * P.cp_pitch;
-      int it = 0;
-      for (int t = t0; t < t1; ++t, it += P.nprod) {
-        const int jt0 = t * CT + half * 128;
-        const bool ragged = jt0 + 128 > P.ncols;
-        const bool offdiag = t > (rb >> 1);  // this tile also serves the rows of its column block
-        const int cb = (t - t0) % COL_BUFS;
-        mbar_wait(smem_u32(&col_full[cb]), static_cast<uint32_t>((t - t0) / COL_BUFS) & 1);
-        const float* cv = colbuf + cb * COL_VECS * CT + half * 128;
-        {  // ---- teacher
-          const int slot = (it + 0) % 2;
-          mbar_wait(smem_u32(&s_full[slot]), static_cast<uint32_t>((it + 0) / 2) & 1);
-          tc_fence_after();
-          uint32_t rA[32], rB[32];
-          tmem_ld32_nowait(lane_addr + slot * CT + half * 128, rA);
-#pragma unroll
-          for (int c = 0; c < 4; ++c) {
-            const int jrel0 = jt0 + c * 32;
-            uint32_t(&rcur)[32] = (c & 1) ? rB : rA;
-            uint32_t(&rnxt)[32] = (c & 1) ? rA : rB;
-            tmem_ld_wait(rcur);
-            if (c < 3) {
-              tmem_ld32_nowait(lane_addr + slot * CT + half * 128 + (c + 1) * 32, rnxt);
-            } else {
-              tc_fence_before();
-              release_slot(slot);
-            }
-            const float4* rc = reinterpret_cast<const float4*>(cv + c * 32);
-            // primed columns: the diagonal is where the column equals the LOCAL row (== the global one at world 1)
-            const int lw0 = rb * BM + q * 32;
-            const bool need_mask = (lw0 < jrel0 + 32 && jrel0 < lw0 + 32) || (ragged && jrel0 + 32 > P.ncols) || !offdiag;
-            float wq[32];
-#pragma unroll
-            for (int e4 = 0; e4 < 8; ++e4) {
-              const float4 r = rc[e4];
-              const float rr[4] = {r.x, r.y, r.z, r.w};
-#pragma unroll
-              for (int k = 0; k < 4; k += 2) {
-                const int e = 4 * e4 + k;
-                const float2 arg = pk_fma(pk(__uint_as_float(rcur[e]), __uint_as_float(rcur[e + 1])),
-                                          pk_mul(cq2, pk(rr[k], rr[k + 1])), bias_t2);
-                float2 we = pk_exp2(arg);
-                if (need_mask) {  // ragged; teacher diag masked
-                  if (jrel0 + e >= P.ncols || jrel0 + e == li) we.x = 0.f;
-                  if (jrel0 + e + 1 >= P.ncols || jrel0 + e + 1 == li) we.y = 0.f;
-                }
-                const float2 wa = pk_mul(we, arg);
-                w[c * 32 + e] = we.x;
-                w[c * 32 + e + 1] = we.y;
-                wq[e] = wa.x;
-                wq[e + 1] = wa.y;
-                zt2 = pk_add(zt2, we);
-                aq2 = pk_add(aq2, wa);
-              }
-            }
-            if (offdiag) {  // warp-uniform
-              float x0[32];
-#pragma unroll
-              for (int e = 0; e < 32; ++e) x0[e] = w[c * 32 + e];
-              const float s0 = warp_colsum32(x0, lane);
-              const float s1 = warp_colsum32(wq, lane);
-              cp_row[0 * cp_stride + jrel0 + lane] = s0;
-              cp_row[1 * cp_stride + jrel0 + lane] = s1;
-            }
-          }
-        }
-        for (int p = 1; p < P.nprod; ++p) {  // ---- student (p = 1), text (p = 2)
-          const int slot = (it + p) % 2;
-          mbar_wait(smem_u32(&s_full[slot]), static_cast<uint32_t>((it + p) / 2) & 1);
-          tc_fence_after();
-          const float cs = (p == 1) ? cp : cr;
-          const float bias_y = live_row ? -((p == 1) ? ms2 : mx2) : NEG_BIG;
-          const float2 cs2 = pk1(cs), bias_y2 = pk1(bias_y);
-          float2 b0 = pk1(0.f), b1 = pk1(0.f);
-          uint32_t rA[32], rB[32];
-          tmem_ld32_nowait(lane_addr + slot * CT + half * 128, rA);
-#pragma unroll
-          for (int c = 0; c < 4; ++c) {
-            const int jrel0 = jt0 + c * 32;
-            uint32_t(&rcur)[32] = (c & 1) ? rB : rA;
-            uint32_t(&rnxt)[32] = (c & 1) ? rA : rB;
-            tmem_ld_wait(rcur);
-            if (c < 3) {
-              tmem_ld32_nowait(lane_addr + slot * CT + half * 128 + (c + 1) * 32, rnxt);
-            } else {
-              tc_fence_before();
-              release_slot(slot);
-            }
-            const float4* rc = reinterpret_cast<const float4*>(cv + p * CT + c * 32);
-            const bool rag = ragged && jrel0 + 32 > P.ncols;
-            float es[32], wp[32];
-#pragma unroll
-            for (int e4 = 0; e4 < 8; ++e4) {
-              const float4 r = rc[e4];
-              const float rr[4] = {r.x, r.y, r.z, r.w};
-#pragma unroll
-              for (int k = 0; k < 4; k += 2) {
-                const int e = 4 * e4 + k;
-                const float2 arg = pk_fma(pk(__uint_as_float(rcur[e]), __uint_as_float(rcur[e + 1])),
-                                          pk_mul(cs2, pk(rr[k], rr[k + 1])), bias_y2);
-                float2 ex = pk_exp2(arg);
-                if (rag) {
-                  if (jrel0 + e >= P.ncols) ex.x = 0.f;
-                  if (jrel0 + e + 1 >= P.ncols) ex.y = 0.f;
-                }
-                // w is zero on masked entries and in dead rows
-                const float2 wa = pk_mul(pk(w[c * 32 + e], w[c * 32 + e + 1]), arg);
-                es[e] = ex.x;
-                es[e + 1] = ex.y;
-                wp[e] = wa.x;
-                wp[e + 1] = wa.y;
-                b0 = pk_add(b0, ex);
-                b1 = pk_add(b1, wa);
-              }
-            }
-            if (offdiag) {
-              const float s0 = warp_colsum32(es, lane);
-              const float s1 = warp_colsum32(wp, lane);
-              cp_row[(p == 1 ? 4 : 5) * cp_stride + jrel0 + lane] = s0;
-              cp_row[(p == 1 ? 2 : 3) * cp_stride + jrel0 + lane] = s1;
-            }
-          }
-          if (p == 1) { zs += b0.x + b0.y; ap += b1.x + b1.y; } else { zx += b0.x + b0.y; ar += b1.x + b1.y; }
-        }
-        mbar_arrive(smem_u32(&col_empty[cb]));
-      }
-      const float zt = zt2.x + zt2.y, aq = aq2.x + aq2.y;
-      if (li < P.b) {  // same partial layout as MODE_SOFT; the maximum is the fixed one
-        const int o = sp * P.b + li;
         const int st = P.npart * P.b;
         P.part[0 * st + o] = mt2;
         P.part[1 * st + o] = zt;

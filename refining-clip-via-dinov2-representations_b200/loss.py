@@ -148,14 +148,13 @@ class _SymW:
     # independent of both: the chain runs on a high-priority second stream and the CLIP part on the caller's, so the
     # block scheduler places the soft CTAs first, CLIP CTAs fill the partial waves, and what is left of the CLIP part
     # runs beside the exchange (2 GPUs, global batch 32768: 7.36 ms per step against 7.86 ms with everything in
-    # line).  While the kernel recorder is on (bench.py's per-kernel pass) or with DSOFT_SYMW_OVERLAP=0 everything
-    # stays on the caller's stream.
+    # line).  While the kernel recorder is on (bench.py's per-kernel pass) everything stays on the caller's stream.
     _side = {}
 
     def run(self, dev, concurrency, call, exchange):
         """call(phase) issues one phase of the C pass on the current stream; exchange() the collective after 1."""
         call(4)
-        if dev.type != "cuda" or concurrency == 2 or os.environ.get("DSOFT_SYMW_OVERLAP", "1") == "0":
+        if dev.type != "cuda" or concurrency == 2:
             call(1)
             exchange()
             call(3)
@@ -373,14 +372,13 @@ class _FnConfig:
 # kernels (dsoft_head_forward): bf16 operands, fp32 accumulation, bias + ReLU + bf16 rounding in the epilogue -
 # the arithmetic autocast gives nn.Linear - and its output lands in the student columns of the packed buffer, so
 # there is no student tensor, no cast and no pack pass.  The backward of the head (five small GEMMs) stays on
-# cuBLAS, issued directly from _DinoSoftFn.backward.  DSOFT_FUSED_HEAD=0 keeps the PyTorch head.
-FUSED_HEAD: Optional[bool] = None  # None: read DSOFT_FUSED_HEAD at every call (default on); True / False force it
+# cuBLAS, issued directly from _DinoSoftFn.backward.
+FUSED_HEAD: bool = True  # False: the PyTorch head (tests compare the two)
 
 
 def _fusable_head(module, image: torch.Tensor):
     """(w1, b1, w2, b2) of a head dsoft_head_forward can run, else None."""
-    on = FUSED_HEAD if FUSED_HEAD is not None else os.environ.get("DSOFT_FUSED_HEAD", "1") != "0"
-    if not on or module is None or image.device.type != "cuda":
+    if not FUSED_HEAD or module is None or image.device.type != "cuda":
         return None
     if not (torch.is_autocast_enabled("cuda") and torch.get_autocast_dtype("cuda") == torch.bfloat16):
         return None  # fp32 callers get fp32 nn.Linear arithmetic

@@ -1,9 +1,9 @@
 """A/B of kernel variants selected by environment switches that libdsoft.so reads at plan creation
-(DSOFT_CLIP_SYM, DSOFT_CLIP_G16, DSOFT_FWD_SYM, ...), in ONE process on one GPU so that both arms see the same
+(DSOFT_CLIP_SYM, DSOFT_SYM_W, ...), in ONE process on one GPU so that both arms see the same
 board, clocks and power state.  Arms alternate `--rounds` times; per arm: whole-step time (forked streams) and the
 serial per-kernel times of the recorder (dsoft_profile_enable).
 
-  python scripts/ab_kernels.py DSOFT_CLIP_G16=0 DSOFT_CLIP_G16=1 [--batch 32768] [--steps 10] [--rounds 3]
+  python scripts/ab_kernels.py DSOFT_CLIP_SYM=0 DSOFT_CLIP_SYM=1 [--batch 32768] [--steps 10] [--rounds 3]
 """
 import argparse
 import ctypes as C

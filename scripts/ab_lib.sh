@@ -2,7 +2,7 @@
 # A/B of two builds of libdsoft.so on ONE board (gpurun -- bash scripts/ab_lib.sh <variant name> [tag]): the GPU test
 # suite on the in-tree build, then the bench line of each build, alternating twice.
 set -x
-var=${1:-scalar}
+var=${1:-variant}
 tag=${2:-ab}
 mkdir -p gpurun_out
 timeout 900 python -m pytest tests -m gpu -q -x 2>&1 | tail -6 > gpurun_out/${tag}_gpu_tests.log; cat gpurun_out/${tag}_gpu_tests.log

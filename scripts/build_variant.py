@@ -1,7 +1,7 @@
 """Build a variant of libdsoft.so with extra nvcc defines (kernel A/B arms on one board):
 
-    python scripts/build_variant.py scalar -DDSOFT_PACKED_F32=0      # -> gpurun_variants/libdsoft_scalar.so
-    DSOFT_LIB=gpurun_variants/libdsoft_scalar.so python bench.py ...  # that build instead of the in-tree one
+    python scripts/build_variant.py variant -DNAME=VALUE   # prints the path of libdsoft_variant.so (out_dir below)
+    DSOFT_LIB=<that path> python bench.py ...               # that build instead of the in-tree one
 """
 import os
 import subprocess

@@ -1,6 +1,7 @@
 """The column butterflies of the symmetric forward epilogues (csrc/dsoft_kernels.cuh: warp_colsum32 for the 32x32b
-TMEM load shape, warp_colsum8 for the 16x256b one), restated lane by lane in numpy: which column's total a lane ends up
-with, and that the total is the sum over all 32 rows of the warp.  The CUDA kernels are checked end to end by the GPU
+TMEM load shape of the one-pass CLIP forward, dsoft_fwd_kernel<MODE_CLIP_SYM>; warp_colsum8 for the 16x256b one of the
+symmetric soft forward, dsoft_fwd_kernel<MODE_SOFT_SYM16>), restated lane by lane in numpy: which column's total a lane
+ends up with, and that the total is the sum over all 32 rows of the warp.  The CUDA kernels are checked end to end by the GPU
 parity tests; this pins the index algebra the kernel comments state (DESIGN section 3)."""
 import numpy as np
 
