@@ -25,7 +25,8 @@
 extern "C" {
 #endif
 
-#define DSOFT_VERSION 220 /* 0.2.2: phase 4 of the phased calls, dsoft_plan_concurrency */
+#define DSOFT_VERSION 230 /* 0.2.3: weighted CE branch at world > 1 (phases 5 / 6, dsoft_plan_lse_rows,
+                             dsoft_plan_wsigma_info) */
 
 /* error codes */
 #define DSOFT_EINVAL (-1)  /* bad argument / unsupported shape            */
@@ -44,8 +45,10 @@ extern "C" {
                                   the fused backward, faster when the scratch memory can be spared.       */
 
 #define DSOFT_F_WEIGHTED 32u    /* denominator-modulated ("weighted") CE branch, loss.py:416-471 + diagnostics
-                                  479-595: DINO-dissimilarity offsets on the CLIP logits.  Single-rank only, like
-                                  the reference; its backward needs DSOFT_F_GMAT.                        */
+                                  479-595: DINO-dissimilarity offsets on the CLIP logits; its backward needs
+                                  DSOFT_F_GMAT.  world > 1 (the reference only runs it on one rank): this rank's
+                                  rows of the global B x B problem, beta from the row stds of all B rows - see
+                                  dsoft_plan_wsigma_info.  Such plans never share soft tiles (DSOFT_SYM_W). */
 #define DSOFT_F_WSYM 64u        /* weight_text_symmetry: modulate the text direction too (loss.py:449-463) */
 
 /* element types accepted by dsoft_pack */
@@ -125,9 +128,10 @@ int dsoft_pack(const dsoft_plan_t* plan, const void* image_dev, int image_dtype,
 int dsoft_head_forward(const dsoft_plan_t* plan, void* gathered_dev, const void* w1_dev, const float* b1_dev,
                        const void* w2_dev, const float* b2_dev, int32_t hidden_dim, void* hidden_dev, void* stream);
 
-/* Symmetric soft tiles across ranks (world > 1, global soft scope, gather_with_grad, DSOFT_F_GMAT, local batch a
- * multiple of 512 and a per-rank block of more than 2^28 similarity entries; environment DSOFT_SYM_W=0 switches it
- * off, DSOFT_SYM_W=1 drops the size condition).  The teacher / student / text Gram matrices are
+/* Symmetric soft tiles across ranks (world > 1, global soft scope, gather_with_grad, DSOFT_F_GMAT, no
+ * DSOFT_F_WEIGHTED, local batch a multiple of 512 and a per-rank block of more than 2^28 similarity entries;
+ * environment DSOFT_SYM_W=0 switches it off, DSOFT_SYM_W=1 drops the size condition but never applies to weighted
+ * plans).  The teacher / student / text Gram matrices are
  * symmetric, so each pair of row blocks is computed by ONE of its two ranks, and what belongs to the other rank's
  * rows is exchanged by the caller - the reduce-scatter of the gathered-feature gradients that `gather_features`
  * implies (loss.py:59-64, `_AllGather.backward`), restricted to the soft terms:
@@ -147,6 +151,19 @@ int dsoft_head_forward(const dsoft_plan_t* plan, void* gathered_dev, const void*
  * Every call of one pass takes the same arguments.
  * dsoft_forward / dsoft_backward refuse such a plan.  Arguments as for dsoft_forward / dsoft_backward. */
 int dsoft_plan_symw_info(const dsoft_plan_t* plan, long long* out12, int n);
+
+/* Weighted CE branch at world > 1 (DSOFT_F_WEIGHTED): beta is the median of the row stds of ALL B rows, one value on
+ * every rank, so the forward pauses once for the caller's exchange of the row stds:
+ *   dsoft_forward_phase(.., 5)   everything up to the weighted row statistics (row stds into `state`)
+ *   caller: all-gather the row-std block in place - rank r's [b x ndir] floats at state + out3[0] + r * out3[1]
+ *   dsoft_forward_phase(.., 6)   median, modulated log-sum-exps, diagnostics, losses
+ * dsoft_forward refuses such a plan (world 1 accepts both forms).  dsoft_plan_wsigma_info: out3 = {offset of the
+ * block in `state` (floats), floats per rank, directions per row (2 with DSOFT_F_WSYM)}, all zero for other plans.
+ * lse_local of such a plan has dsoft_plan_lse_rows() rows: the five log-sum-exps, then per modulated direction
+ * c, lse~ (log2) and A of the rows, which the backward's column side needs from every rank (one all-gather with the
+ * log-sum-exps, as before).  dsoft_plan_lse_rows returns 5 for every other plan. */
+int dsoft_plan_wsigma_info(const dsoft_plan_t* plan, long long* out3, int n);
+int dsoft_plan_lse_rows(const dsoft_plan_t* plan);
 int dsoft_forward_phase(const dsoft_plan_t* plan, const void* gathered_dev, const float* logit_scale_dev,
                         const float* lambdas, void* state_dev, void* scratch_dev, float* lse_local_dev,
                         float* losses_dev, float* dbg_dev, void* stream, int phase);
@@ -187,20 +204,21 @@ int dsoft_gather_rows(const void* table_dev, int table_dtype, int64_t ld_table, 
 
 /* Forward statistics pass.  logit_scale_dev: one fp32 (already exp'd, reference model.py:571).
  * lambdas (HOST, 4 floats): {lambda_original, lambda_soft, text_lambda, lambda_weighted} (loss.py:387-388,
- * 417, 474).  Outputs: lse_local_dev [5][b] fp32 (log2-domain row log-sum-exps: clip i->t, clip t->i,
- * teacher, student, text) and losses_dev[6] = {classic_loss, soft_imgimg, soft_texttext,
+ * 417, 474).  Outputs: lse_local_dev [dsoft_plan_lse_rows][b] fp32 (rows 0..4: log2-domain row log-sum-exps:
+ * clip i->t, clip t->i, teacher, student, text) and losses_dev[6] = {classic_loss, soft_imgimg, soft_texttext,
  * soft = imgimg + text_lambda * texttext, total = lambda_original * classic + lambda_soft * soft
  * + lambda_weighted * weighted, weighted_loss} (loss.py:317-319, 383, 396-397, 466, 473-477), the first three
  * already divided by b.  With DSOFT_F_WEIGHTED, dbg_dev (32 floats, may be NULL to skip the diagnostics pass)
  * receives the reference's diagnostic scalars (loss.py:479-595): [0,1] pc_err img/txt, [2,3] diag_max, [4..6]
  * delta_img max/mean/std, [7..9] delta_txt, [10,11] l1_prob_shift, [12,13] corr_rhat_dprob, [14..17] ce_img_base,
  * ce_txt_base, ce_img_mod, ce_txt_mod, [18..21] pos/neg_frac img, pos/neg_frac txt, [22,23] beta img/txt,
- * [24] rho, [25] c_clip.  beta stays on the device: no host synchronisation (the reference calls .item()). */
+ * [24] rho, [25] c_clip.  beta stays on the device: no host synchronisation (the reference calls .item()).
+ * At world > 1 the losses and diagnostics are this rank's row block (means over its b rows; beta global). */
 int dsoft_forward(const dsoft_plan_t* plan, const void* gathered_dev, const float* logit_scale_dev,
                   const float* lambdas_host, void* state_dev, void* scratch_dev, float* lse_local_dev,
                   float* losses_dev, float* dbg_dev, void* stream);
 
-/* Backward pass.  lse_all_dev [world][5][b] = all ranks' lse_local (all-gathered by the caller when
+/* Backward pass.  lse_all_dev [world][dsoft_plan_lse_rows][b] = all ranks' lse_local (all-gathered by the caller when
  * world > 1).  gout_dev[6] = upstream gradients of the six forward outputs (the chain rule through
  * `soft` and `total` is applied on the device with the same lambdas).  Outputs (fp32):
  * d_image [b][D], d_text [b][D], d_student [b][Dp] (ignored when Dp == 0), d_logit_scale [1].

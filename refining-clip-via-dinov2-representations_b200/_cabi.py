@@ -65,6 +65,8 @@ PROTOTYPES = {
                             + [C.c_int]),
     "dsoft_backward_phase": (C.c_int, [C.c_void_p] * 6 + [C.POINTER(C.c_float)] + [C.c_void_p] * 5 + [C.c_int]),
     "dsoft_plan_symw_info": (C.c_int, [C.c_void_p, C.POINTER(C.c_longlong), C.c_int]),
+    "dsoft_plan_wsigma_info": (C.c_int, [C.c_void_p, C.POINTER(C.c_longlong), C.c_int]),
+    "dsoft_plan_lse_rows": (C.c_int, [C.c_void_p]),
     "dsoft_selftest_gemm": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p]),
     "dsoft_selftest_chain": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                        C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p]),

@@ -64,7 +64,10 @@ struct dsoft_plan {
   size_t sc_clipM, sc_clipS, sc_lse_ti, st_dbound;
   SplitPlan f_sym;     // its (triangular) column chunks
   size_t sc_colpart, sc_colsum;
-  int weighted, wsym;  // denominator-modulated CE branch (loss.py:416-471), world == 1 only
+  int weighted, wsym;  // denominator-modulated CE branch (loss.py:416-471); world > 1: this rank's row block
+  int wnd;             // directions with a row std (1, or 2 with weight_text_symmetry)
+  int lse_rows;        // per-row statistics rows of lse_local: 5, weighted world > 1 5 + 3 wnd (c, lse~, A)
+  size_t st_wsig;      // weighted, world > 1: row std [B][wnd] by global row (all-gathered by the caller)
   SplitPlan f_wce;     // column split of its tile passes
   int Dz;          // student width (Dp or D)
   // packed row layout (elements)
@@ -181,9 +184,8 @@ extern "C" int dsoft_plan_create(const dsoft_shape_t* sh, dsoft_plan_t** out) {
   if ((sh->flags & DSOFT_F_TEXT) && !(sh->text_temp > 0.f))
     return fail(DSOFT_EINVAL, "text_temp must be > 0");
   if (sh->flags & DSOFT_F_WEIGHTED) {
-    // the reference builds r and the diagonal mask from the LOCAL batch against [b, B] logits and fails in the
-    // first broadcast when world > 1 (loss.py:423-446)
-    if (sh->world != 1) return fail(DSOFT_EINVAL, "the weighted CE branch is single-rank only (loss.py:416-471)");
+    // world > 1 (the reference fails there, loss.py:423-446): this rank's row block of the global B x B problem,
+    // beta from the row stds of all B rows (dsoft_forward_phase 5, exchange, 6)
     if (sh->Dd == 0) return fail(DSOFT_EINVAL, "DSOFT_F_WEIGHTED needs Dd > 0");
     if (!(sh->c_clip > 0.f)) return fail(DSOFT_EINVAL, "c_clip must be > 0");
   }
@@ -205,6 +207,8 @@ extern "C" int dsoft_plan_create(const dsoft_shape_t* sh, dsoft_plan_t** out) {
   p->have_proj = soft && sh->Dp > 0;
   p->weighted = (sh->flags & DSOFT_F_WEIGHTED) != 0;
   p->wsym = p->weighted && (sh->flags & DSOFT_F_WSYM) != 0;
+  p->wnd = p->wsym ? 2 : 1;
+  p->lse_rows = (p->weighted && sh->world > 1) ? 5 + 3 * p->wnd : 5;
   p->soft_local = (sh->flags & DSOFT_F_SOFT_LOCAL) != 0 && sh->world > 1;
   p->row_only = (sh->flags & DSOFT_F_ROW_ONLY) != 0 && sh->world > 1;
   p->Dz = p->have_proj ? sh->Dp : sh->D;
@@ -227,7 +231,8 @@ extern "C" int dsoft_plan_create(const dsoft_shape_t* sh, dsoft_plan_t** out) {
     // CUDA graph 4.20 ms), on 2 GPUs 7.4 ms against 8.85 ms.  DESIGN.md section 6.
     const char* e = getenv("DSOFT_SYM_W");
     const bool big = static_cast<double>(sh->b) * p->B > 268435456.0;
-    p->sym_w = soft && sh->world > 1 && !p->soft_local && !p->row_only && (sh->flags & DSOFT_F_GMAT) &&
+    // weighted plans never share soft tiles (their forward has its own exchange)
+    p->sym_w = soft && sh->world > 1 && !p->soft_local && !p->row_only && (sh->flags & DSOFT_F_GMAT) && !p->weighted &&
                1.4426950408889634 / sh->teacher_temp <= 60.0 && sh->b % 512 == 0 &&
                (e ? e[0] != '0' : big);
     p->sw_ncols_a = 0;
@@ -296,6 +301,7 @@ extern "C" int dsoft_plan_create(const dsoft_shape_t* sh, dsoft_plan_t** out) {
   p->st_colfac = take(static_cast<size_t>(5) * p->Bcol);
   p->st_lsestat = take(2 * 64);
   p->st_wstat = take(p->weighted ? static_cast<size_t>(8) * p->Bcol : 0);
+  p->st_wsig = take(p->weighted && sh->world > 1 ? static_cast<size_t>(p->wnd) * p->B : 0);
   p->st_total = o;
 
   // ---- scratch (floats)
@@ -411,7 +417,8 @@ extern "C" int dsoft_plan_launches_forward(const dsoft_plan_t* p) {
 extern "C" int dsoft_plan_launches_backward(const dsoft_plan_t* p) {
   if (!p) return 0;
   if (p->gmat)
-    return 3 /*lse stats, relayout, fp16 operands*/ + (p->clip_tr ? 1 : 2) /*clip G*/ + 2 /*clip GEMMs*/ +
+    return 3 /*lse stats, relayout, fp16 operands*/ + (p->weighted && !p->clip_tr ? 1 : 0) /*weighted relayout*/ +
+           (p->clip_tr ? 1 : 2) /*clip G*/ + 2 /*clip GEMMs*/ +
            (p->have_soft ? 2 : 0) /*soft G, student GEMM*/ + (p->have_text ? 1 : 0) + 1 /*finalize*/;
   return 3 /*lse stats, relayout, fp16 operands*/ + 2 * chunk_groups(p->nch_clip) + (p->have_soft ? chunk_groups(p->nch_stu) : 0) +
          (p->have_text ? chunk_groups(p->nch_txt) : 0) + 1 /*finalize*/;
@@ -882,14 +889,14 @@ __device__ bool last_block_done(int* ticket) {
 // 2^(x - c) (2^(c - lse_row) + 2^(c - lse_col)) and decides whether that form is safe (every 2^(c - lse) inside
 // fp32: spread <= 200 log2 units; c >= -100 keeps 2^(0 - c) of padded entries finite).
 constexpr int LSE_NB = 64;
-__global__ void __launch_bounds__(256) lse_stats_kernel(const float* __restrict__ lse_all, int W, int b,
+__global__ void __launch_bounds__(256) lse_stats_kernel(const float* __restrict__ lse_all, int W, int b, int nr,
                                                         float* __restrict__ part) {
   __shared__ float smn[8], smx[8];
   float mn = __int_as_float(0x7f800000), mx = -__int_as_float(0x7f800000);
   const int n = W * 2 * b;
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
     const int r = i / (2 * b), k = i % (2 * b);
-    const float v = lse_all[static_cast<size_t>(r) * 5 * b + k];  // kinds 0 and 1 are contiguous
+    const float v = lse_all[static_cast<size_t>(r) * nr * b + k];  // kinds 0 and 1 are contiguous
     mn = fminf(mn, v);
     mx = fmaxf(mx, v);
   }
@@ -907,14 +914,15 @@ __global__ void __launch_bounds__(256) lse_stats_kernel(const float* __restrict_
   }
 }
 
-// [W][5][b] (rank-major, as all-gathered) -> by global column, padded:
+// [W][nr][b] (rank-major, as all-gathered; rows 0..4 used here) -> by global column, padded:
 //   lsec   [5][Bcol]  the log-sum-exps themselves (zero padded; exact CLIP form and the fused backward)
 //   colfac [5][Bcol]  column factors of the factorised logit gradients: 0 / 1 CLIP 2^(c - lse) for the image-rows
 //                     launch (columns = text rows' lse_ti) and the text-rows launch (lse_it); 2 teacher
 //                     2^(M_t - lt) (exact form: lt); 3 student 2^(M_s - ls); 4 text 2^(M_x - lx).  Zero (teacher
 //                     exact form: +1e30, i.e. 2^(q - 1e30) = 0) for padded columns and wherever the column-side
 //                     terms are dropped (gather_with_grad == False).
-__global__ void __launch_bounds__(256) lse_relayout_kernel(const float* __restrict__ lse_all, int W, int b, int Bcol,
+__global__ void __launch_bounds__(256) lse_relayout_kernel(const float* __restrict__ lse_all, int W, int b, int nr,
+                                                           int Bcol,
                                                            float* __restrict__ scal, const float* __restrict__ part,
                                                            int fast_t, int drop_clip, int drop_soft,
                                                            float* __restrict__ out, float* __restrict__ colfac) {
@@ -944,12 +952,12 @@ __global__ void __launch_bounds__(256) lse_relayout_kernel(const float* __restri
     const int k = i / Bcol, j = i % Bcol;
     const bool real = j < W * b;
     float v = 0.f;
-    if (real) v = lse_all[(static_cast<size_t>(j / b) * 5 + k) * b + (j % b)];
+    if (real) v = lse_all[(static_cast<size_t>(j / b) * nr + k) * b + (j % b)];
     out[i] = v;
     float f;
     if (k < 2) {
       // colfac[0] serves the launch whose columns are TEXT rows (their lse is kind 1), colfac[1] the other one
-      const float lo = real ? lse_all[(static_cast<size_t>(j / b) * 5 + (1 - k)) * b + (j % b)] : 0.f;
+      const float lo = real ? lse_all[(static_cast<size_t>(j / b) * nr + (1 - k)) * b + (j % b)] : 0.f;
       f = (real && !drop_clip) ? exp2f(cclip - lo) : 0.f;
     } else if (k == 2) {
       if (fast_t) f = (real && !drop_soft) ? exp2f(scal[SC_ITT_L2] - v) : 0.f;
@@ -998,10 +1006,10 @@ struct FinBwdArgs {
   int b, D, Dz, row0, row_elems, offI, offT, offZ;
   int have_soft, have_text, have_proj, row_only;
   int sym_scaled;  // two-phase backward, world == 1: the soft G matrices carry mant(1/||y_i||) of their ROW as well
-  // weighted CE (world == 1): the CLIP logit-gradient matrix already carries g_c and g_w; the diagonal entry of
-  // both directions is applied here in fp32
+  // weighted CE: the CLIP logit-gradient matrices already carry g_c and g_w; the diagonal entry of both directions
+  // is applied here in fp32
   int weighted, wsym;
-  const float* wstat;  // [2 directions][4][Bcol]: c, lse~, A, (std)
+  const float* wstat;  // [2 directions][4][Bcol] by global row: c, lse~, A, (std)
   int Bcol;
   float lam_w;
   int ns_c, ns_c2, ns_s, ns_x;  // split counts of acc1, acc2, acc3, acc4
@@ -1063,7 +1071,7 @@ __device__ __forceinline__ float4 load_bf16x4(const __nv_bfloat16* p) {
 // small residual), the coefficient of the CLIP part and the diagonal's share of d(logit_scale).
 //   classic:  dg = (p_it_aa - 1) + (p_ti_aa - 1); the matrix is unscaled, g_c s / (2b) is applied here; the row
 //             partials of d(logit_scale) include the diagonal's probabilities, hence the - 2 dot_aa
-//   weighted (world == 1): the matrix already carries g_c and g_w and has no diagonal;
+//   weighted: the matrix already carries g_c and g_w and has no diagonal;
 //             dg = g_c [(p_it_aa - 1) + (p_ti_aa - 1)] + g_w [(p~_it_aa - 1 + beta A_a p_it_aa c_a) + text direction]
 //             (d CE~_a / d x_aa = p~_aa - 1 - beta A_a p_aa (r_aa - c_a) with r_aa = 0, loss.py:416-471)
 struct ClipDiag { float dg_img, dg_txt, coefc, ds_diag; };
@@ -1082,13 +1090,18 @@ __device__ __forceinline__ ClipDiag clip_diag(const FinBwdArgs& a, int i, float 
     const float gw = a.gout[5] + a.lam_w * a.gout[4];
     const float* wi = a.wstat;
     const float* wt = a.wstat + static_cast<size_t>(4) * a.Bcol;
-    const float g_img = expm1f(LN2 * (xd - wi[1 * a.Bcol + i])) +
-                        a.scal[SC_WBETA + 0] * wi[2 * a.Bcol + i] * (dm_it + 1.f) * wi[0 * a.Bcol + i];
-    const float g_txt = a.wsym ? expm1f(LN2 * (xd - wt[1 * a.Bcol + i])) +
-                                     a.scal[SC_WBETA + 1] * wt[2 * a.Bcol + i] * (dm_ti + 1.f) * wt[0 * a.Bcol + i]
+    const int j = a.row0 + i;  // the statistics rows are indexed by global row
+    const float g_img = expm1f(LN2 * (xd - wi[1 * a.Bcol + j])) +
+                        a.scal[SC_WBETA + 0] * wi[2 * a.Bcol + j] * (dm_it + 1.f) * wi[0 * a.Bcol + j];
+    const float g_txt = a.wsym ? expm1f(LN2 * (xd - wt[1 * a.Bcol + j])) +
+                                     a.scal[SC_WBETA + 1] * wt[2 * a.Bcol + j] * (dm_ti + 1.f) * wt[0 * a.Bcol + j]
                                : dm_ti;
     const float dg = gc * (dm_it + dm_ti) + gw * (g_img + g_txt);
     r.dg_img = r.dg_txt = dg;
+    if (a.row_only) {  // world > 1, gathered columns detached: each direction's own row term only
+      r.dg_img = gc * dm_it + gw * g_img;
+      r.dg_txt = gc * dm_ti + gw * g_txt;
+    }
     r.coefc = a.scal[SC_SCALE] * 0.5f * inv_b;
     r.ds_diag = dg * a.diag[i];
   }
@@ -1728,23 +1741,30 @@ static void fill_clip_fwd(const dsoft_plan* p, FwdParams& P, int amap, int bmap,
 }
 
 // ------------------------------------------------------------------------------------------------
-// denominator-modulated ("weighted") CE branch, loss.py:416-471 + diagnostics loss.py:479-595 (world == 1)
+// denominator-modulated ("weighted") CE branch, loss.py:416-471 + diagnostics loss.py:479-595
 // ------------------------------------------------------------------------------------------------
 // Per direction (image rows x text columns; text rows x image columns when weight_text_symmetry):
 //   STAT tile pass -> wce_rows<0> (c_a, row std) -> wce_median (beta) -> LSE tile pass -> wce_rows<1> (lse~, A_a,
 //   row CE) -> DBG tile pass -> wce_rows<2> (diagnostic rows);  then wce_final assembles the loss and the dbg
 //   scalars.  Nothing of size B x B is stored; beta stays on the device (the reference's `.item()` syncs are gone).
+// World > 1: every pass runs over this rank's [b x B] row block (row0 = rank * b).  beta is the median over all B
+// rows, so the row stds leave through the caller's all-gather between wce_rows<0> and wce_median (phases 5 / 6),
+// and c, lse~ and A travel with the LSE all-gather (lse_local rows 5 ..) for the backward's column side.
 enum { WS_C = 0, WS_LSET = 1, WS_A = 2, WS_STD = 3 };       // state rows per direction: [dir * 4 + k][Bcol]
 enum { WR_CE_MOD = 0, WR_CE_BASE, WR_PC, WR_L1, WR_CORR, WR_SABS, WR_SSQ, WR_MAX, WR_POS, WR_DIAG, WR_N };
 enum { DBG_N = 32 };
 
 struct WceRowsArgs {
   int b, np, dir;
+  int row0, ncols;     // global index of local row 0; columns per row (B)
+  float* sig;          // row std of local row i -> sig[(row0 + i) * sig_stride]
+  int sig_stride;
+  float* ext;          // world > 1: lse_local rows of this direction [3][b] (c, lse~, A), else null
   const float* part;   // [k][np][b]
   const float* lse;    // [b] log2 LSE of the unmodified logits of this direction
   const float* diag;   // [b] raw diagonal dot products
   const float* scal;
-  float* wstat;        // state rows of this direction [4][Bcol]
+  float* wstat;        // state rows of this direction [4][Bcol], by global row
   int Bcol;
   float* wrows;        // [WR_N][b] of this direction
   float cc;
@@ -1756,7 +1776,7 @@ __global__ void __launch_bounds__(256) wce_rows_kernel(WceRowsArgs a) {
   if (i >= a.b) return;
   const float LN2 = 0.6931471805599453f;
   const int st = a.np * a.b;
-  float* ws = a.wstat;
+  float* ws = a.wstat + a.row0;
   if constexpr (PHASE == 0) {
     float c = 0.f;
     double s1 = 0.0, s2 = 0.0;  // sums of x and x^2 in log2 units; fp64 for the E[x^2] - E[x]^2 cancellation
@@ -1765,10 +1785,12 @@ __global__ void __launch_bounds__(256) wce_rows_kernel(WceRowsArgs a) {
       s1 += static_cast<double>(a.part[1 * st + k * a.b + i]);
       s2 += static_cast<double>(a.part[2 * st + k * a.b + i]);
     }
-    const double n = a.b;  // square logits: one column per row
+    const double n = a.ncols;
     const double var = (s2 - s1 * s1 / n) / (n - 1.0);  // torch.std: unbiased (loss.py:440)
     ws[WS_C * a.Bcol + i] = c;
-    ws[WS_STD * a.Bcol + i] = static_cast<float>(sqrt(var > 0.0 ? var : 0.0)) * LN2;  // natural-log units
+    a.sig[static_cast<size_t>(a.row0 + i) * a.sig_stride] =
+        static_cast<float>(sqrt(var > 0.0 ? var : 0.0)) * LN2;  // natural-log units
+    if (a.ext) a.ext[i] = c;
   } else if constexpr (PHASE == 1) {
     float m = M_FLOOR;
     for (int k = 0; k < a.np; ++k) m = fmaxf(m, a.part[0 * st + k * a.b + i]);
@@ -1781,6 +1803,10 @@ __global__ void __launch_bounds__(256) wce_rows_kernel(WceRowsArgs a) {
     const float lset = m + log2f(s);
     ws[WS_LSET * a.Bcol + i] = lset;
     ws[WS_A * a.Bcol + i] = si / s;
+    if (a.ext) {
+      a.ext[1 * a.b + i] = lset;
+      a.ext[2 * a.b + i] = si / s;
+    }
     const float xd = a.scal[SC_SCALE] * a.diag[i];
     a.wrows[WR_CE_MOD * a.b + i] = LN2 * lset - xd;       // loss.py:447 / 463: CE row of the modified logits
     a.wrows[WR_CE_BASE * a.b + i] = LN2 * a.lse[i] - xd;  // loss.py:541-542
@@ -1792,7 +1818,7 @@ __global__ void __launch_bounds__(256) wce_rows_kernel(WceRowsArgs a) {
         v = (q == 9) ? fmaxf(v, a.part[q * st + k * a.b + i]) : v + a.part[q * st + k * a.b + i];
       acc[q] = v;
     }
-    const float n = static_cast<float>(a.b);
+    const float n = static_cast<float>(a.ncols);
     // rowwise Pearson correlation of r^ and (p~ - p), loss.py:528-536
     const float cov = acc[6] - acc[2] * acc[4] / n;
     const float vr = fmaxf(acc[3] - acc[2] * acc[2] / n, 0.f), vd = fmaxf(acc[5] - acc[4] * acc[4] / n, 0.f);
@@ -1807,11 +1833,11 @@ __global__ void __launch_bounds__(256) wce_rows_kernel(WceRowsArgs a) {
   }
 }
 
-// beta = rho * max(median_row(std), 1e-6) / c_clip (loss.py:440-443).  torch.median returns the LOWER of the two
-// middle values: the element of rank (b - 1) / 2.  One block, four 8-bit radix-select passes over the bit
-// patterns (non-negative floats order like unsigned integers).
-__global__ void __launch_bounds__(1024) wce_median_kernel(const float* __restrict__ v, int b, float rho, float cc,
-                                                          float* __restrict__ scal, int dir) {
+// beta = rho * max(median_row(std), 1e-6) / c_clip (loss.py:440-443) over the b values v[i * stride].  torch.median
+// returns the LOWER of the two middle values: the element of rank (b - 1) / 2.  One block, four 8-bit radix-select
+// passes over the bit patterns (non-negative floats order like unsigned integers).
+__global__ void __launch_bounds__(1024) wce_median_kernel(const float* __restrict__ v, int b, int stride, float rho,
+                                                          float cc, float* __restrict__ scal, int dir) {
   __shared__ unsigned hist[256];
   __shared__ unsigned s_prefix, s_rank;
   if (threadIdx.x == 0) { s_prefix = 0u; s_rank = static_cast<unsigned>((b - 1) / 2); }
@@ -1822,7 +1848,7 @@ __global__ void __launch_bounds__(1024) wce_median_kernel(const float* __restric
     const unsigned prefix = s_prefix;
     const unsigned mask = shift == 24 ? 0u : (0xffffffffu << (shift + 8));
     for (int i = threadIdx.x; i < b; i += blockDim.x) {
-      const unsigned key = __float_as_uint(v[i]);
+      const unsigned key = __float_as_uint(v[static_cast<size_t>(i) * stride]);
       if ((key & mask) == prefix) atomicAdd(&hist[(key >> shift) & 255u], 1u);
     }
     __syncthreads();
@@ -1847,6 +1873,7 @@ __global__ void __launch_bounds__(1024) wce_median_kernel(const float* __restric
 
 struct WceFinalArgs {
   int b, sym;
+  int ncols;           // columns per row (B): the diagnostics over all entries count b x ncols
   const float* wrows;  // [2][WR_N][b]
   const float* lse;    // [5][b] (only the text direction's base CE needs it when !sym)
   const float* diag;
@@ -1890,7 +1917,7 @@ __global__ void __launch_bounds__(1024) wce_final_kernel(WceFinalArgs a) {
     }
   }
   if (threadIdx.x != 0) return;
-  const double n = a.b, nn = n * n, off = nn - n;
+  const double n = a.b, nn = n * a.ncols, off = nn - n;
   const double ce_img_mod = res[0][WR_CE_MOD] / n, ce_img_base = res[0][WR_CE_BASE] / n;
   const double ce_txt_base = res[1][WR_CE_BASE] / n;
   const double ce_txt_mod = a.sym ? res[1][WR_CE_MOD] / n : ce_txt_base;
@@ -1903,7 +1930,7 @@ __global__ void __launch_bounds__(1024) wce_final_kernel(WceFinalArgs a) {
   for (int d = 0; d < (a.sym ? 2 : 1); ++d) {
     const double beta = a.scal[SC_WBETA + d];
     const double sabs = beta * res[d][WR_SABS], ssq = beta * beta * res[d][WR_SSQ];
-    const double var = (ssq - sabs * sabs / nn) / (nn - 1.0);  // std of |Delta| over all B^2 entries (diag = 0)
+    const double var = (ssq - sabs * sabs / nn) / (nn - 1.0);  // std of |Delta| over all b x B entries (diag = 0)
     g[0 + d] = static_cast<float>(res[d][WR_PC] / n);          // pc_err
     g[2 + d] = static_cast<float>(res[d][WR_DIAG]);            // diag_max
     g[4 + 3 * d] = static_cast<float>(beta * res[d][WR_MAX]);  // delta max / mean / std
@@ -1923,6 +1950,19 @@ __global__ void __launch_bounds__(1024) wce_final_kernel(WceFinalArgs a) {
   g[25] = a.cc;
 }
 
+// world > 1, backward: c, lse~ and A of every rank's rows ([W][nr][b] rows 5 + 3 d + k, as all-gathered) -> the
+// state rows [d][k][Bcol] by global row (zero padded), where the column side of the logit-gradient kernels reads them
+__global__ void __launch_bounds__(256) wce_relayout_kernel(const float* __restrict__ lse_all, int W, int b, int nr,
+                                                           int Bcol, int nd, float* __restrict__ wstat) {
+  static_assert(WS_C == 0 && WS_LSET == 1 && WS_A == 2, "lse_local carries c, lse~, A in state-row order");
+  const int total = 3 * nd * Bcol;
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < total; i += gridDim.x * blockDim.x) {
+    const int dk = i / Bcol, j = i % Bcol, d = dk / 3, k = dk % 3;
+    wstat[(static_cast<size_t>(d) * 4 + k) * Bcol + j] =
+        j < W * b ? lse_all[(static_cast<size_t>(j / b) * nr + 5 + dk) * b + (j % b)] : 0.f;
+  }
+}
+
 template <typename K>
 static int launch_fwd_pair(K kernel, int rbs, int nsplit, cudaStream_t st, const TileMaps& tm, const FwdParams& P,
                            int threads);
@@ -1938,7 +1978,7 @@ static void fill_wce(const dsoft_plan* p, FwdParams& P, int dir, float* S, float
   P.a_map[1] = P.b_map[1] = 3;    // DINO cosine (symmetric: r^T = r, loss.py:453)
   P.kchunks[0] = ceil_div(p->sh.D, BK);
   P.kchunks[1] = ceil_div(p->sh.Dd, BK);
-  P.row0 = 0;
+  P.row0 = p->sh.rank * p->sh.b;
   P.b = p->sh.b;
   P.col0 = 0;
   P.ncols = p->B;
@@ -1953,41 +1993,58 @@ static void fill_wce(const dsoft_plan* p, FwdParams& P, int dir, float* S, float
   P.wcc = p->sh.c_clip;
 }
 
-// forward of the weighted branch; runs after finalize_fwd_kernel (needs the CLIP row LSEs and the diagonal)
-static int weighted_forward(const dsoft_plan* p, const TileMaps& tm, float* S, float* X, const float* lse_local,
-                            float lam_w, float* losses, float* dbg, cudaStream_t st) {
-  const int b = p->sh.b, rbs = ceil_div(b, BM), ns = p->f_wce.nsplit;
+// forward of the weighted branch; runs after finalize_fwd_kernel (needs the CLIP row LSEs and the diagonal).
+// part_a: the row statistics up to the row stds; part_b: median onward.  World > 1 runs them as two calls with the
+// caller's all-gather of the row stds in between.
+static int weighted_forward(const dsoft_plan* p, const TileMaps& tm, float* S, float* X, float* lse_local,
+                            float lam_w, float* losses, float* dbg, cudaStream_t st, bool part_a, bool part_b) {
+  const int b = p->sh.b, rbs = ceil_div(b, BM), ns = p->f_wce.nsplit, row0 = p->sh.rank * b;
+  const bool multi = p->sh.world > 1;
   int rc;
   if ((rc = set_smem(dsoft_fwd_kernel<MODE_WCE_STAT, 2>, FWD_SMEM_BYTES))) return rc;
   if ((rc = set_smem(dsoft_fwd_kernel<MODE_WCE_LSE, 2>, FWD_SMEM_BYTES))) return rc;
   if ((rc = set_smem(dsoft_fwd_kernel<MODE_WCE_DBG, 2>, FWD_SMEM_BYTES))) return rc;
   float* part = X + p->sc_wpart;
-  for (int d = 0; d < (p->wsym ? 2 : 1); ++d) {
-    float* ws = S + p->st_wstat + static_cast<size_t>(d) * 4 * p->Bcol;
-    FwdParams P;
-    fill_wce(p, P, d, S, part);
-    P.wrow[0] = lse_local + d * b;
-    P.wrow[1] = ws + WS_C * p->Bcol;
-    P.wrow[2] = ws + WS_LSET * p->Bcol;
-    WceRowsArgs ra;
-    ra.b = b; ra.np = 2 * ns; ra.dir = d; ra.part = part; ra.lse = lse_local + d * b; ra.diag = S + p->st_diag;
-    ra.scal = S + p->st_scal; ra.wstat = ws; ra.Bcol = p->Bcol; ra.wrows = X + p->sc_wrows + static_cast<size_t>(d) * WR_N * b;
-    ra.cc = p->sh.c_clip;
-    const int rg = ceil_div(b, 256);
-    if ((rc = launch_fwd_pair(dsoft_fwd_kernel<MODE_WCE_STAT, 2>, rbs, ns, st, tm, P))) return rc;
-    wce_rows_kernel<0><<<rg, 256, 0, st>>>(ra);
-    wce_median_kernel<<<1, 1024, 0, st>>>(ws + WS_STD * p->Bcol, b, p->sh.rho, p->sh.c_clip, S + p->st_scal, d);
-    if ((rc = launch_fwd_pair(dsoft_fwd_kernel<MODE_WCE_LSE, 2>, rbs, ns, st, tm, P))) return rc;
-    wce_rows_kernel<1><<<rg, 256, 0, st>>>(ra);
-    if (dbg) {
-      if ((rc = launch_fwd_pair(dsoft_fwd_kernel<MODE_WCE_DBG, 2>, rbs, ns, st, tm, P))) return rc;
-      wce_rows_kernel<2><<<rg, 256, 0, st>>>(ra);
+  const int rg = ceil_div(b, 256);
+  for (int stage = 0; stage < 2; ++stage) {
+    if (!(stage == 0 ? part_a : part_b)) continue;
+    for (int d = 0; d < p->wnd; ++d) {
+      float* ws = S + p->st_wstat + static_cast<size_t>(d) * 4 * p->Bcol;
+      FwdParams P;
+      fill_wce(p, P, d, S, part);
+      P.wrow[0] = lse_local + d * b;
+      P.wrow[1] = ws + WS_C * p->Bcol + row0;
+      P.wrow[2] = ws + WS_LSET * p->Bcol + row0;
+      WceRowsArgs ra;
+      ra.b = b; ra.np = 2 * ns; ra.dir = d; ra.part = part; ra.lse = lse_local + d * b; ra.diag = S + p->st_diag;
+      ra.scal = S + p->st_scal; ra.wstat = ws; ra.Bcol = p->Bcol; ra.wrows = X + p->sc_wrows + static_cast<size_t>(d) * WR_N * b;
+      ra.cc = p->sh.c_clip;
+      ra.row0 = row0;
+      ra.ncols = p->B;
+      ra.sig = multi ? S + p->st_wsig + d : ws + WS_STD * p->Bcol;
+      ra.sig_stride = multi ? p->wnd : 1;
+      ra.ext = multi ? lse_local + static_cast<size_t>(5 + 3 * d) * b : nullptr;
+      if (stage == 0) {
+        if ((rc = launch_fwd_pair(dsoft_fwd_kernel<MODE_WCE_STAT, 2>, rbs, ns, st, tm, P))) return rc;
+        wce_rows_kernel<0><<<rg, 256, 0, st>>>(ra);
+      } else {
+        // over all B rows: ra.sig is the start of the (all-gathered) block, indexed by global row
+        wce_median_kernel<<<1, 1024, 0, st>>>(ra.sig, p->B, ra.sig_stride, p->sh.rho, p->sh.c_clip, S + p->st_scal, d);
+        if ((rc = launch_fwd_pair(dsoft_fwd_kernel<MODE_WCE_LSE, 2>, rbs, ns, st, tm, P))) return rc;
+        wce_rows_kernel<1><<<rg, 256, 0, st>>>(ra);
+        if (dbg) {
+          if ((rc = launch_fwd_pair(dsoft_fwd_kernel<MODE_WCE_DBG, 2>, rbs, ns, st, tm, P))) return rc;
+          wce_rows_kernel<2><<<rg, 256, 0, st>>>(ra);
+        }
+      }
+      CUDA_TRY(cudaGetLastError());
     }
-    CUDA_TRY(cudaGetLastError());
   }
+  if (!part_b) return 0;
   WceFinalArgs fa;
   fa.b = b; fa.sym = p->wsym; fa.wrows = X + p->sc_wrows; fa.lse = lse_local; fa.diag = S + p->st_diag;
   fa.scal = S + p->st_scal; fa.rho = p->sh.rho; fa.cc = p->sh.c_clip; fa.lam_w = lam_w; fa.losses = losses; fa.dbg = dbg;
+  fa.ncols = p->B;
   wce_final_kernel<<<1, 1024, 0, st>>>(fa);
   CUDA_TRY(cudaGetLastError());
   return 0;
@@ -2118,7 +2175,8 @@ extern "C" int dsoft_pair_stats(const void* clip_a, const void* clip_b, int32_t 
 }
 
 // phase 0: the whole forward; of a DSOFT_SYM_W plan: 4 = operand statistics, 1 = the soft part up to the column-sum
-// exchange, 3 = the CLIP part (independent of 1 and of the exchange), 2 = finalize
+// exchange, 3 = the CLIP part (independent of 1 and of the exchange), 2 = finalize; of a weighted plan: 5 = up to the
+// weighted row statistics (row stds), 6 = median onward
 static int forward_impl(const dsoft_plan_t* p, const void* gathered, const float* logit_scale,
                         const float* lambdas, void* state, void* scratch, float* lse_local,
                         float* losses, float* dbg, void* stream, int phase);
@@ -2129,13 +2187,21 @@ extern "C" int dsoft_forward(const dsoft_plan_t* p, const void* gathered, const 
   if (p && p->sym_w)
     return fail(DSOFT_EINVAL, "this plan shares the symmetric soft tiles across ranks (DSOFT_SYM_W): call "
                               "dsoft_forward_phase 4, 1, 3 (next to the column-sum exchange), 2");
+  if (p && p->weighted && p->sh.world > 1)
+    return fail(DSOFT_EINVAL, "the weighted CE branch at world > 1 needs the row stds of all ranks: call "
+                              "dsoft_forward_phase 5, all-gather the row-std block, then phase 6");
   return forward_impl(p, gathered, logit_scale, lambdas, state, scratch, lse_local, losses, dbg, stream, 0);
 }
 
 extern "C" int dsoft_forward_phase(const dsoft_plan_t* p, const void* gathered, const float* logit_scale,
                                    const float* lambdas, void* state, void* scratch, float* lse_local,
                                    float* losses, float* dbg, void* stream, int phase) {
-  if (phase < 1 || phase > 4) return fail(DSOFT_EINVAL, "phase must be 4, 1, 3 or 2");
+  if (!p) return fail(DSOFT_EINVAL, "null argument");
+  // 1..4: the symmetric soft tiles' schedule; 5 / 6: around the row-std exchange of the weighted branch
+  const bool wmulti = p->weighted && p->sh.world > 1;
+  if (phase < 1 || phase > 6 || (phase >= 5 && !p->weighted) || (phase <= 4 && wmulti))
+    return fail(DSOFT_EINVAL, wmulti ? "a weighted plan at world > 1 takes phases 5 and 6"
+                                     : (p->weighted ? "phase must be 1..6" : "phase must be 4, 1, 3 or 2"));
   return forward_impl(p, gathered, logit_scale, lambdas, state, scratch, lse_local, losses, dbg, stream, phase);
 }
 
@@ -2155,9 +2221,11 @@ static int forward_impl(const dsoft_plan_t* p, const void* gathered, const float
   if (rc) return rc;
 
   // phases of a DSOFT_SYM_W plan: 4 = operand statistics, 1 = soft tile kernel + column reduction, 3 = CLIP kernels
-  // (the caller's column-sum exchange runs next to them), 2 = finalize; 0 = everything
-  const bool do_pro = phase == 0 || phase == 4, do_soft = phase == 0 || phase == 1, do_clip = phase == 0 || phase == 3;
-  if (phase != 2) {
+  // (the caller's column-sum exchange runs next to them), 2 = finalize; 0 = everything.  Weighted plans: 5 = all of
+  // phase 0 up to the weighted row stds, 6 = the rest of the weighted branch (after the caller's row-std all-gather)
+  const bool whole = phase == 0 || phase == 5;
+  const bool do_pro = whole || phase == 4, do_soft = whole || phase == 1, do_clip = whole || phase == 3;
+  if (phase != 2 && phase != 6) {
   if (do_pro) {
   prep_scalars_kernel<<<1, 32, 0, st>>>(logit_scale, p->have_soft ? p->sh.teacher_temp : 0.f,
                                         p->have_text ? p->sh.text_temp : 0.f, S + p->st_scal);
@@ -2277,8 +2345,9 @@ static int forward_impl(const dsoft_plan_t* p, const void* gathered, const float
   }
   }  // do_clip
   if ((rc = fk.join())) return rc;
-  }  // phase != 2
-  if (phase != 0 && phase != 2) return 0;
+  }  // phase != 2 && phase != 6
+  if (phase == 1 || phase == 3 || phase == 4) return 0;
+  if (phase == 6) return weighted_forward(p, tm, S, X, lse_local, lambdas[3], losses, dbg, st, false, true);
 
   FinFwdArgs fa;
   fa.b = b;
@@ -2303,7 +2372,7 @@ static int forward_impl(const dsoft_plan_t* p, const void* gathered, const float
   fa.losses = losses;
   finalize_fwd_kernel<<<ceil_div(b, 128), 128, 0, st>>>(fa);
   CUDA_TRY(cudaGetLastError());
-  if (p->weighted) return weighted_forward(p, tm, S, X, lse_local, lambdas[3], losses, dbg, st);
+  if (p->weighted) return weighted_forward(p, tm, S, X, lse_local, lambdas[3], losses, dbg, st, true, phase != 5);
   return 0;
 }
 
@@ -2489,38 +2558,48 @@ static int backward_two_phase(const dsoft_plan* p, const void* gathered, float* 
   if (!do_clip) return fk.join();
   if (p->weighted) {
     // world == 1: ONE logit-gradient matrix carries  g_c * classic CE + g_w * weighted CE  of both directions
-    // (loss.py:416-471 backward); the two gradient GEMMs below are the classic ones
+    // (loss.py:416-471 backward); the two gradient GEMMs below are the classic ones.  World > 1: one matrix per
+    // direction, like the CLIP launches below: the row side is this rank's rows of direction d, the column side the
+    // other direction's rows of all ranks (statistics relayouted from lse_all by wce_relayout_kernel)
     if ((rc = set_smem(dsoft_fwd_kernel<MODE_WCE_G, 2>, FWD_SMEM_BYTES))) return rc;
-    if ((rc = fk.lane(lane++, &ks))) return rc;
-    fill_wce(p, P, 0, S, nullptr);
-    const float* wi = S + p->st_wstat;
-    const float* wt = wi + static_cast<size_t>(4) * p->Bcol;
-    P.wrow[0] = lse_loc;
-    P.wrow[1] = wi + WS_C * p->Bcol;
-    P.wrow[2] = wi + WS_LSET * p->Bcol;
-    P.wrow[3] = wi + WS_A * p->Bcol;
-    P.ncolvec = 5;
-    P.colvec[1] = lsec + static_cast<size_t>(1) * p->Bcol;  // lse of the text direction, by column
-    P.colvec[2] = wt + WS_LSET * p->Bcol;                   // (only read when weight_text_symmetry)
-    P.colvec[3] = wt + WS_C * p->Bcol;
-    P.colvec[4] = wt + WS_A * p->Bcol;
-    P.wsym = p->wsym;
-    P.wgout = gout;
-    P.wlam[0] = lambdas[0];
-    P.wlam[1] = lambdas[3];
-    P.gout[0] = Gci;
-    P.g_pitch = p->pitch_c;
-    P.npart = 2 * p->f_wce.nsplit;
-    P.ds_part = X + p->sc_ds1;
-    if ((rc = make_gstore_map(p, &tm.g[0], Gci, p->pitch_c))) return rc;
-    tm.g[1] = tm.g[0];
-    {
-      ProfScope ps(PK_BWD_GCLIP, ks);
-      if ((rc = launch_fwd_pair(dsoft_fwd_kernel<MODE_WCE_G, 2>, rbs, p->f_wce.nsplit, ks, tm, P))) return rc;
-    }
-    {
-      ProfScope ps(PK_BWD_CLIP_I, ks);
-      if ((rc = launch_gy(p, Gci, p->pitch_c, v16, p->v_offT, p->sh.D, 0, p->g_clip, X + p->sc_acc1, ks))) return rc;
+    const size_t r0 = static_cast<size_t>(p->sh.rank) * b;
+    for (int d = 0; d < (p->clip_tr ? 1 : 2); ++d) {
+      if ((rc = fk.lane(lane++, &ks))) return rc;
+      fill_wce(p, P, d, S, nullptr);
+      const float* wr = S + p->st_wstat + static_cast<size_t>(d) * 4 * p->Bcol;      // row-side direction
+      const float* wc = S + p->st_wstat + static_cast<size_t>(1 - d) * 4 * p->Bcol;  // column-side direction
+      P.wrow[0] = lse_loc + d * b;
+      P.wrow[1] = wr + WS_C * p->Bcol + r0;
+      P.wrow[2] = wr + WS_LSET * p->Bcol + r0;
+      P.wrow[3] = wr + WS_A * p->Bcol + r0;
+      P.ncolvec = 5;
+      P.colvec[1] = lsec + static_cast<size_t>(1 - d) * p->Bcol;  // lse of the other direction, by column
+      P.colvec[2] = wc + WS_LSET * p->Bcol;                       // (only read when that direction is modulated)
+      P.colvec[3] = wc + WS_C * p->Bcol;
+      P.colvec[4] = wc + WS_A * p->Bcol;
+      P.wsym = d == 0 ? p->wsym : 1;
+      P.wrow_plain = d == 1 && !p->wsym;
+      P.wsplit = !p->clip_tr;
+      P.row_only = p->row_only;
+      P.wgout = gout;
+      P.wlam[0] = lambdas[0];
+      P.wlam[1] = lambdas[3];
+      P.gout[0] = d == 0 ? Gci : Gct;
+      P.g_pitch = p->pitch_c;
+      P.npart = 2 * p->f_wce.nsplit;
+      P.ds_part = X + (d == 0 ? p->sc_ds1 : p->sc_ds2);
+      if ((rc = make_gstore_map(p, &tm.g[0], P.gout[0], p->pitch_c))) return rc;
+      tm.g[1] = tm.g[0];
+      {
+        ProfScope ps(PK_BWD_GCLIP, ks);
+        if ((rc = launch_fwd_pair(dsoft_fwd_kernel<MODE_WCE_G, 2>, rbs, p->f_wce.nsplit, ks, tm, P))) return rc;
+      }
+      {
+        ProfScope ps(d == 0 ? PK_BWD_CLIP_I : PK_BWD_CLIP_T, ks);
+        if ((rc = launch_gy(p, P.gout[0], p->pitch_c, v16, d == 0 ? p->v_offT : p->v_offI, p->sh.D, 0, p->g_clip,
+                            X + (d == 0 ? p->sc_acc1 : p->sc_acc2), ks)))
+          return rc;
+      }
     }
   }
   for (int d = 0; d < (p->weighted ? 0 : (p->clip_tr ? 1 : 2)); ++d) {  // d = 0: image rows (dI = G . T), d = 1: text rows
@@ -2592,6 +2671,22 @@ extern "C" int dsoft_backward_phase(const dsoft_plan_t* p, const void* gathered,
 //  [7] the same for the text term [s_ncols - b][D], [8] D (0: no text term)
 //  [9] offset of this rank's own student partial sums (split 0: [b][Dz]), [10] of the text ones ([b][D])
 //  [11] number of K splits of those partial sums (received products are added to split 0)
+// Rows of the per-row statistics lse_local / lse_all carry (5, more for a weighted plan at world > 1)
+extern "C" int dsoft_plan_lse_rows(const dsoft_plan_t* p) { return p ? p->lse_rows : 0; }
+
+// Row-std block of a weighted plan at world > 1 (out[3], in floats): [0] offset in `state`, [1] floats per rank
+// (rank r's block starts at [0] + r * [1]), [2] directions per row.  All zero for every other plan.
+extern "C" int dsoft_plan_wsigma_info(const dsoft_plan_t* p, long long* out, int n) {
+  if (!p || !out || n < 3) return fail(DSOFT_EINVAL, "need 3 slots");
+  for (int k = 0; k < n; ++k) out[k] = 0;
+  if (p->weighted && p->sh.world > 1) {
+    out[0] = static_cast<long long>(p->st_wsig);
+    out[1] = static_cast<long long>(p->wnd) * p->sh.b;
+    out[2] = p->wnd;
+  }
+  return 0;
+}
+
 extern "C" int dsoft_plan_symw_info(const dsoft_plan_t* p, long long* out, int n) {
   if (!p || !out || n < 12) return fail(DSOFT_EINVAL, "need 12 slots");
   for (int k = 0; k < n; ++k) out[k] = 0;
@@ -2629,19 +2724,24 @@ static int backward_impl(const dsoft_plan_t* p, const void* gathered, const void
   if (rc) return rc;
 
   float* lsec = S + p->st_lsecols;
-  const float* lse_loc = lse_all + static_cast<size_t>(p->sh.rank) * 5 * b;
+  const float* lse_loc = lse_all + static_cast<size_t>(p->sh.rank) * p->lse_rows * b;
   // phases of a DSOFT_SYM_W plan: 1 = statistics relayout + fp16 operands + soft lane (G kernel, GEMMs incl. the
   // transposed products), 3 = CLIP lanes (the caller's exchange of the transposed products runs next to them),
   // 2 = finalize; 0 = everything
   if (phase != 2) {
   __half* v16 = reinterpret_cast<__half*>(X + p->sc_v16);
   if (phase == 0 || phase == 4) {
-  lse_stats_kernel<<<LSE_NB, 256, 0, st>>>(lse_all, p->sh.world, b, S + p->st_lsestat);
+  lse_stats_kernel<<<LSE_NB, 256, 0, st>>>(lse_all, p->sh.world, b, p->lse_rows, S + p->st_lsestat);
   CUDA_TRY(cudaGetLastError());
   lse_relayout_kernel<<<ceil_div(5 * p->Bcol, 1024), 256, 0, st>>>(
-      lse_all, p->sh.world, b, p->Bcol, S + p->st_scal, S + p->st_lsestat, p->fast_t, p->row_only,
+      lse_all, p->sh.world, b, p->lse_rows, p->Bcol, S + p->st_scal, S + p->st_lsestat, p->fast_t, p->row_only,
       p->row_only && !p->soft_local, lsec, S + p->st_colfac);
   CUDA_TRY(cudaGetLastError());
+  if (p->weighted && p->sh.world > 1) {
+    wce_relayout_kernel<<<ceil_div(3 * p->wnd * p->Bcol, 1024), 256, 0, st>>>(lse_all, p->sh.world, b, p->lse_rows,
+                                                                             p->Bcol, p->wnd, S + p->st_wstat);
+    CUDA_TRY(cudaGetLastError());
+  }
   make_v16_kernel<<<ceil_div(p->B, 8), 256, 0, st>>>(
       static_cast<const __nv_bfloat16*>(gathered), p->row_elems, p->B, p->sh.D, p->Dz, p->offI, p->offT,
       p->offZ, p->have_soft, p->have_text, S + p->st_rinv_z, S + p->st_rinv_t, v16, p->v_row, p->v_offT, p->v_offI,

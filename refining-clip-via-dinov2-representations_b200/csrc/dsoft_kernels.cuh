@@ -120,12 +120,17 @@ struct FwdParams {
   int g_pitch;              // columns of G (multiple of 64 >= ncols)
   int row_only;             // clip, exact form: gather_with_grad == False drops the column-side terms
   float* ds_part;           // clip: d(logit_scale) row partials [npart][b]
-  // ---- weighted-CE modes (MODE_WCE_*): world == 1
+  // ---- weighted-CE modes (MODE_WCE_*): one rank's [b x B] row block (row0 = rank * b, col0 = 0)
   int ncolvec;              // per-column vectors staged per tile: colvec[0 .. ncolvec)
-  const float* colvec[6];   // [0] 1/||dino_j||; G mode: [1] lse_ti, [2] lse~ (text dir), [3] c' (text dir), [4] A'
+  const float* colvec[6];   // [0] 1/||dino_j||; G mode, by global column, of the OTHER direction: [1] lse,
+                            // [2] lse~, [3] c', [4] A'
   const float* wrow[4];     // per row: [0] lse of the unmodified logits (log2), [1] c_a, [2] lse~ (log2), [3] A_a
   int wdir;                 // 0: image rows x text columns, 1: text rows x image columns
-  int wsym;                 // weight_text_symmetry (loss.py:449-463)
+  int wsym;                 // G mode: the column-side direction is modulated (image rows: weight_text_symmetry,
+                            // loss.py:449-463; text rows: always)
+  int wrow_plain;           // G mode: the row-side direction is the classic CE (text rows without weight_text_symmetry)
+  int wsplit;               // G mode, world > 1: the d(logit_scale) row partial takes the row-side term only (the
+                            // text rows' launch holds the rest), and row_only drops the column-side term
   float wcc;                // c_clip
   const float* wgout;       // G mode: upstream gradients [6] (device)
   // ---- symmetric forward (MODE_SOFT_SYM16): column partials [6][cp_rows = 4 * row blocks][cp_pitch]
@@ -1195,8 +1200,9 @@ dsoft_fwd_kernel(const __grid_constant__ TileMaps maps, const __grid_constant__ 
     } else if constexpr (kWce) {
       // ---------------------------------------------------------------- denominator-modulated CE, loss.py:416-471
       // Products per 256-column tile: [0] CLIP logits x (row operand = image rows, or text rows for the text
-      // direction), [1] DINO cosine -> dissimilarity r = 1 - clamp(cos), r_aa = 0 (loss.py:424-429).  One world-
-      // size-1 problem (the reference's branch is single-rank): global row == local row, col0 == 0.
+      // direction), [1] DINO cosine -> dissimilarity r = 1 - clamp(cos), r_aa = 0 (loss.py:424-429).  The rows are
+      // this rank's block [row0, row0 + b) of the global B x B problem, the columns all of it (col0 == 0), so the
+      // diagonal of local row li sits at column row0 + li.  World size 1 is the reference's square problem.
       //   STAT : c_a = sum_j p_aj r_aj with p = soft-max of the UNMODIFIED row (loss.py:434-435), and the row sums
       //          of x and x^2 behind the row std of the logits (loss.py:440-441)
       //   LSE  : log-sum-exp of x~ = x + beta clamp(r - c_a, +-c_clip) (diagonal unshifted, loss.py:445-447) and
@@ -1204,7 +1210,9 @@ dsoft_fwd_kernel(const __grid_constant__ TileMaps maps, const __grid_constant__ 
       //   DBG  : the row statistics behind the reference's diagnostics (loss.py:479-595)
       //   G    : the fp16 logit gradient of  g_c * classic CE  +  g_w * weighted CE  for BOTH directions in one
       //          matrix (rows = image, columns = text; the text direction's entry is the transposed one and reads
-      //          its row statistics per column):  d CE~_a / d x_ak = p~_ak - delta_ak - beta A_a p_ak (r_ak - c_a)
+      //          its row statistics per column):  d CE~_a / d x_ak = p~_ak - delta_ak - beta A_a p_ak (r_ak - c_a).
+      //          World > 1: one launch per direction (wdir = row side); the column side reads the other
+      //          direction's all-gathered row statistics by global column, as MODE_CLIP_G does.
       const int lic = min(li, P.b - 1);
       const float s2 = P.scal[SC_SCALE_L2];
       const float rda = P.colvec[0][min(gi, P.ncols - 1)];
@@ -1226,9 +1234,9 @@ dsoft_fwd_kernel(const __grid_constant__ TileMaps maps, const __grid_constant__ 
       if constexpr (MODE == MODE_WCE_G) {
         gcl = P.wgout[0] + P.wlam[0] * P.wgout[4];
         gwt = P.wgout[5] + P.wlam[1] * P.wgout[4];
-        beta_i = P.scal[SC_WBETA + 0];
-        beta_t = P.scal[SC_WBETA + 1];
-        beta2_t = P.scal[SC_WBETA2 + 1];
+        beta_i = P.scal[SC_WBETA + P.wdir];  // row-side direction
+        beta_t = P.scal[SC_WBETA + 1 - P.wdir];
+        beta2_t = P.scal[SC_WBETA2 + 1 - P.wdir];
         aa_a = P.wrow[3][lic];
       }
       int it = 0;
@@ -1375,18 +1383,23 @@ dsoft_fwd_kernel(const __grid_constant__ TileMaps maps, const __grid_constant__ 
                   const float x = xq[c * 32 + e];
                   const float za = r[e] - c_a;
                   const float e1 = fast_exp2(x - lse_a);
-                  const float pt = fast_exp2(fmaf(beta2, fminf(fmaxf(za, -cc), cc), x) - lset_a);
-                  const float gimg = pt - beta_i * aa_a * e1 * za;
-                  const float e2 = fast_exp2(x - lti[k]);
+                  float gimg = e1;  // row-side direction (the image direction unless wdir == 1)
+                  if (!P.wrow_plain) {
+                    const float pt = fast_exp2(fmaf(beta2, fminf(fmaxf(za, -cc), cc), x) - lset_a);
+                    gimg = pt - beta_i * aa_a * e1 * za;
+                  }
+                  float e2 = fast_exp2(x - lti[k]);
                   float gtxt = e2;
                   if (P.wsym) {
                     const float zj = r[e] - cj[k];
                     const float ptj = fast_exp2(fmaf(beta2_t, fminf(fmaxf(zj, -cc), cc), x) - ltt[k]);
                     gtxt = ptj - beta_t * aj[k] * e2 * zj;
                   }
+                  if (P.wsplit && P.row_only) e2 = gtxt = 0.f;  // gathered columns carry no gradient
                   float g = gcl * (e1 + e2) + gwt * (gimg + gtxt);
-                  if (need_mask && ((jrel0 + e == gi) || (jrel0 + e >= P.ncols) || !live_row)) g = 0.f;
-                  acc[0] = fmaf(g, x, acc[0]);  // d(logit_scale) row term in log2 units of x (off-diagonal part)
+                  float gr = P.wsplit ? gcl * e1 + gwt * gimg : g;  // this rank's own loss terms
+                  if (need_mask && ((jrel0 + e == gi) || (jrel0 + e >= P.ncols) || !live_row)) g = gr = 0.f;
+                  acc[0] = fmaf(gr, x, acc[0]);  // d(logit_scale) row term in log2 units of x (off-diagonal part)
                   g4[k] = g;
                 }
                 w16[2 * e4 + 0] = pack_f16x2(g4[0], g4[1]);

@@ -18,8 +18,10 @@ Differences from the reference that are deliberate and documented in DESIGN.md:
     is rounded with a straight-through gradient); all soft-max / KL arithmetic is fp32;
   * at world_size > 1 the soft terms default to the *global* row block (``soft_scope="global"``);
     ``soft_scope="local"`` reproduces the reference's local b x b block;
-  * the weighted-CE branch (loss.py:416-471, lambda_weighted > 0; one rank only, off by default) runs in the
-    same fused kernels (fp32 logits also under autocast, beta kept on the device instead of `.item()`);
+  * the weighted-CE branch (loss.py:416-471, lambda_weighted > 0, off by default) runs in the same fused kernels
+    (fp32 logits also under autocast, beta kept on the device instead of `.item()`).  The reference only runs it on
+    one rank; at world_size > 1 it raises like the reference unless ``weighted_scope="global"``, which gives rank r
+    the rows [r b, (r+1) b) of the branch on the concatenated batch (beta from the row stds of all B rows);
   * Horovod is not supported (``use_horovod=True`` raises).
 """
 from __future__ import annotations
@@ -101,7 +103,7 @@ _DTYPES = {torch.float32: _cabi.DT_F32, torch.bfloat16: _cabi.DT_BF16, torch.flo
 
 class _Plan:
     __slots__ = ("handle", "row_elems", "state_numel", "scratch_numel", "fwd_scratch_numel", "flops",
-                 "launches_fwd", "launches_bwd", "shape", "dino_col", "symw")
+                 "launches_fwd", "launches_bwd", "shape", "dino_col", "symw", "lse_rows", "wsig")
 
 
 class _SymW:
@@ -244,6 +246,12 @@ class CudaBackend:
             info = (C.c_longlong * 12)()
             _cabi.check(self._lib.dsoft_plan_symw_info(h, info, 12), "dsoft_plan_symw_info")
             p.symw = _SymW(list(info), shape.world, shape.rank) if info[0] else None
+            # weighted CE at world > 1: the row-std block in `state` (offset, floats per rank, directions) that the
+            # forward all-gathers between phases 5 and 6, and the widened per-row statistics of lse_local
+            ws = (C.c_longlong * 3)()
+            _cabi.check(self._lib.dsoft_plan_wsigma_info(h, ws, 3), "dsoft_plan_wsigma_info")
+            p.wsig = (int(ws[0]), int(ws[1]), int(ws[2])) if ws[1] else None
+            p.lse_rows = int(self._lib.dsoft_plan_lse_rows(h))
             p.shape = shape
             self._plans[key] = p
         return p
@@ -289,7 +297,8 @@ class CudaBackend:
         return (C.c_float * 4)(*[float(x) for x in lambdas])
 
     def forward(self, plan, gathered, logit_scale, lambdas, state, scratch, lse_local, losses, dbg=None, phase=0):
-        """phase 0: whole forward; a plan with `symw`: 4 operand statistics, 1 soft part, 3 CLIP part, 2 finalize."""
+        """phase 0: whole forward; a plan with `symw`: 4 operand statistics, 1 soft part, 3 CLIP part, 2 finalize;
+        a plan with `wsig`: 5 up to the weighted row stds, 6 the rest."""
         a = (plan.handle, _ptr(gathered), _ptr(logit_scale), self._lam(lambdas), _ptr(state), _ptr(scratch),
              _ptr(lse_local), _ptr(losses), _ptr(dbg), self._stream(gathered))
         if phase == 0:
@@ -448,7 +457,7 @@ class _DinoSoftFn(torch.autograd.Function):
             dist.all_gather_into_tensor(gathered.view(-1), gathered[r * b:(r + 1) * b].view(-1), group=cfg.group)
         state = torch.empty(plan.state_numel, dtype=torch.float32, device=dev)
         scratch = torch.empty(plan.fwd_scratch_numel, dtype=torch.float32, device=dev)
-        lse_all = torch.empty((W, 5, b), dtype=torch.float32, device=dev)
+        lse_all = torch.empty((W, getattr(plan, "lse_rows", 5), b), dtype=torch.float32, device=dev)
         losses = torch.empty(6, dtype=torch.float32, device=dev)
         dbg = torch.empty(_cabi.DBG_N if weighted else 0, dtype=torch.float32, device=dev)
         ls = logit_scale.detach().to(device=dev, dtype=torch.float32).reshape(1).contiguous()
@@ -458,10 +467,20 @@ class _DinoSoftFn(torch.autograd.Function):
             fargs = (plan, gathered, ls, cfg.lambdas, state, scratch, lse_all[r], losses, None)
             plan.symw.run(dev, be.concurrency(plan), lambda ph: be.forward(*fargs, phase=ph),
                           lambda: plan.symw.exchange_forward(scratch, cfg.group))
+        elif getattr(plan, "wsig", None) is not None:
+            # weighted CE at world > 1: beta is the median of the row stds of all B rows, so the forward pauses once
+            # for their all-gather (ndir floats per sample), in place in `state`
+            fargs = (plan, gathered, ls, cfg.lambdas, state, scratch, lse_all[r], losses, dbg)
+            be.forward(*fargs, phase=5)
+            off, n, _ = plan.wsig
+            sig = state[off:off + W * n]
+            dist.all_gather_into_tensor(sig, sig[r * n:(r + 1) * n], group=cfg.group)
+            be.forward(*fargs, phase=6)
         else:
             be.forward(plan, gathered, ls, cfg.lambdas, state, scratch, lse_all[r], losses, dbg if weighted else None)
         if W > 1 and needs_grad:
-            # column-side soft-max statistics of the other ranks' rows (5 floats per sample)
+            # column-side soft-max statistics of the other ranks' rows (5 floats per sample; weighted CE: 3 more per
+            # modulated direction)
             dist.all_gather_into_tensor(lse_all.view(-1), lse_all[r].view(-1), group=cfg.group)
         ctx.save_for_backward(gathered, state, lse_all, hidden, w1b, w2b)
         ctx.plan, ctx.cfg = plan, cfg
@@ -534,7 +553,10 @@ class _DinoSoftFn(torch.autograd.Function):
 # Runs inside libdsoft.so (DSOFT_F_WEIGHTED): three tile passes per direction over the CLIP and DINO Gram tiles
 # (row statistics c_a = sum_j p r and the row std of the logits -> device-side median -> beta; log-sum-exp of the
 # shifted logits; diagnostics) and one logit-gradient pass in the backward.  Nothing of size B x B is stored and beta
-# never visits the host (the reference calls `.item()` twice per step).  Single-rank only, like the reference.
+# never visits the host (the reference calls `.item()` twice per step).  At world_size > 1 (`weighted_scope="global"`)
+# every rank runs its row block of the global problem: one extra all-gather of the row stds in the forward, and the
+# per-row statistics the backward's column side needs travel with the existing LSE all-gather.  The loss terms and
+# diagnostics are per rank (means over the rank's rows); beta_img / beta_txt are the global values.
 DBG_KEYS = (  # index into the dbg array of dsoft_forward (include/dsoft.h)
     ("pc_err_img", 0), ("pc_err_txt", 1), ("diag_max_img", 2), ("diag_max_txt", 3),
     ("delta_img_max", 4), ("delta_img_mean", 5), ("delta_img_std", 6),
@@ -573,6 +595,7 @@ class ClipLossWithDINOEnhancements(nn.Module):
         soft_scope: str = "global",
         process_group=None,
         sync_projection: bool = True,
+        weighted_scope: Optional[str] = None,
     ):
         super().__init__()
         self.local_loss = local_loss
@@ -584,6 +607,11 @@ class ClipLossWithDINOEnhancements(nn.Module):
         if soft_scope not in ("global", "local"):
             raise ValueError(f"soft_scope must be 'global' or 'local', got {soft_scope!r}")
         self.soft_scope = soft_scope
+        if weighted_scope not in (None, "global"):
+            raise ValueError(f"weighted_scope must be None or 'global', got {weighted_scope!r}")
+        # None: the reference's behaviour (the lambda_weighted branch fails at world_size > 1); "global": rank r
+        # computes rows [r b, (r+1) b) of the branch on the concatenated batch (DESIGN.md section 1)
+        self.weighted_scope = weighted_scope
         self.process_group = process_group
         self.sync_projection = sync_projection
 
@@ -676,7 +704,7 @@ class ClipLossWithDINOEnhancements(nn.Module):
             )
         lambda_weighted = float(g(args, "lambda_weighted", 0.0))
         weighted_on = lambda_weighted > 0.0 and dino_features is not None and B > 1  # loss.py:422
-        if weighted_on and self.world_size > 1:
+        if weighted_on and self.world_size > 1 and self.weighted_scope is None:
             # the reference builds r and the diagonal mask from the LOCAL batch against [b, B] logits
             # (loss.py:423-446) and fails in the first broadcast; keep the failure
             raise RuntimeError(
