@@ -25,8 +25,8 @@
 extern "C" {
 #endif
 
-#define DSOFT_VERSION 230 /* 0.2.3: weighted CE branch at world > 1 (phases 5 / 6, dsoft_plan_lse_rows,
-                             dsoft_plan_wsigma_info) */
+#define DSOFT_VERSION 240 /* 0.2.4: weighted plans accept the fused backward (no DSOFT_F_GMAT); 0.2.3: weighted
+                             CE branch at world > 1 (phases 5 / 6, dsoft_plan_lse_rows, dsoft_plan_wsigma_info) */
 
 /* error codes */
 #define DSOFT_EINVAL (-1)  /* bad argument / unsupported shape            */
@@ -45,10 +45,13 @@ extern "C" {
                                   the fused backward, faster when the scratch memory can be spared.       */
 
 #define DSOFT_F_WEIGHTED 32u    /* denominator-modulated ("weighted") CE branch, loss.py:416-471 + diagnostics
-                                  479-595: DINO-dissimilarity offsets on the CLIP logits; its backward needs
-                                  DSOFT_F_GMAT.  world > 1 (the reference only runs it on one rank): this rank's
-                                  rows of the global B x B problem, beta from the row stds of all B rows - see
-                                  dsoft_plan_wsigma_info.  Such plans never share soft tiles (DSOFT_SYM_W). */
+                                  479-595: DINO-dissimilarity offsets on the CLIP logits.  Both backward forms:
+                                  with DSOFT_F_GMAT one fp16 logit-gradient matrix per direction (world 1: one),
+                                  without it the fused backward, whose two CLIP launches (bwd clip image / text
+                                  rows) then also recompute the DINO tile.  world > 1 (the reference only runs
+                                  it on one rank): this rank's rows of the global B x B problem, beta from the
+                                  row stds of all B rows - see dsoft_plan_wsigma_info.  Such plans never share
+                                  soft tiles (DSOFT_SYM_W). */
 #define DSOFT_F_WSYM 64u        /* weight_text_symmetry: modulate the text direction too (loss.py:449-463) */
 
 /* element types accepted by dsoft_pack */
@@ -99,7 +102,8 @@ size_t dsoft_plan_forward_scratch_bytes(const dsoft_plan_t* plan);
 double dsoft_plan_algorithmic_flops(const dsoft_plan_t* plan);
 /* FLOPs of the tile-kernel launches of one fwd+bwd for this rank, in dsoft_profile_read order (n >= 7;
  * 9 slots are filled when available): fwd clip i->t, fwd clip t->i, fwd soft, bwd clip (image rows), bwd
- * clip (text rows), bwd student, bwd text, [7] CLIP logit-gradient kernel(s), [8] soft logit-gradient kernel
+ * clip (text rows) - of a weighted plan the fused weighted CE kernel, CLIP and DINO products -, bwd student,
+ * bwd text, [7] CLIP logit-gradient kernel(s), [8] soft logit-gradient kernel
  * (the last two only with DSOFT_F_GMAT, where slots 3..6 are the gradient GEMMs).  `algorithmic` follows
  * SURVEY.md 8(d) (each distinct product once, no recompute); `executed` is what the tensor cores really do
  * (tile recompute included). */
@@ -232,7 +236,7 @@ int dsoft_backward(const dsoft_plan_t* plan, const void* gathered_dev, const voi
 /* Optional timing of the tile kernels with CUDA events on the launching stream (bench.py roofline).
  * dsoft_profile_read synchronises the device, returns summed milliseconds and launch counts per kernel
  * kind since the last read, and resets the recorder.  9 slots: the 7 kinds above (with DSOFT_F_GMAT slots
- * 3..6 are the gradient GEMMs) followed by the CLIP (2 launches) and the soft logit-gradient kernels. */
+ * 3..6 are the gradient GEMMs; without it slots 3 / 4 of a weighted plan are the fused weighted CE kernel) followed by the CLIP (2 launches) and the soft logit-gradient kernels. */
 int dsoft_profile_enable(int on);
 int dsoft_profile_read(double* ms_sum, int* counts, int n);
 

@@ -386,6 +386,8 @@ extern "C" int dsoft_plan_kernel_flops(const dsoft_plan_t* p, double* algorithmi
   }
   algorithmic[3] = algorithmic[4] = 2.0 * b * Bc * D;
   executed[3] = executed[4] = 2.0 * b * Bc * D * (chunk_groups(p->nch_clip) + 1.0);
+  if (p->weighted)  // fused weighted CE backward: the CLIP and the DINO product per chunk group, then G . Y
+    executed[3] = executed[4] = 2.0 * b * Bc * (chunk_groups(p->nch_clip) * (D + Dd) + D);
   if (p->have_soft) {
     algorithmic[2] = executed[2] = 2.0 * b * Bs * (Dz + Dd + (p->have_text ? D : 0.0));
     if (p->fwd_sym) executed[2] *= 0.5 * (1.0 + 256.0 / std::max(256.0, Bs));  // upper block triangle + diagonal tiles
@@ -420,7 +422,8 @@ extern "C" int dsoft_plan_launches_backward(const dsoft_plan_t* p) {
     return 3 /*lse stats, relayout, fp16 operands*/ + (p->weighted && !p->clip_tr ? 1 : 0) /*weighted relayout*/ +
            (p->clip_tr ? 1 : 2) /*clip G*/ + 2 /*clip GEMMs*/ +
            (p->have_soft ? 2 : 0) /*soft G, student GEMM*/ + (p->have_text ? 1 : 0) + 1 /*finalize*/;
-  return 3 /*lse stats, relayout, fp16 operands*/ + 2 * chunk_groups(p->nch_clip) + (p->have_soft ? chunk_groups(p->nch_stu) : 0) +
+  return 3 /*lse stats, relayout, fp16 operands*/ + (p->weighted && p->sh.world > 1 ? 1 : 0) /*weighted relayout*/ +
+         2 * chunk_groups(p->nch_clip) /*clip, or weighted CE*/ + (p->have_soft ? chunk_groups(p->nch_stu) : 0) +
          (p->have_text ? chunk_groups(p->nch_txt) : 0) + 1 /*finalize*/;
 }
 
@@ -1375,6 +1378,8 @@ __global__ void __launch_bounds__(256, 2) finalize_bwd_warp_kernel(FinBwdArgs a)
 // ------------------------------------------------------------------------------------------------
 // optional per-kernel timing (bench.py's roofline): CUDA events around each tile-kernel launch
 // ------------------------------------------------------------------------------------------------
+// PK_BWD_CLIP_I / _T: the fused backward's CLIP launches (of a weighted plan dsoft_bwd_kernel<MODE_WCE_X>, CLIP and
+// DINO products), or with DSOFT_F_GMAT the CLIP gradient GEMMs
 enum { PK_FWD_CLIP_IT = 0, PK_FWD_CLIP_TI, PK_FWD_SOFT, PK_BWD_CLIP_I, PK_BWD_CLIP_T, PK_BWD_STU, PK_BWD_TXT,
        PK_BWD_GCLIP, PK_BWD_GSOFT, PK_COUNT };
 static const int PROF_MAX = 4096;
@@ -2711,8 +2716,6 @@ static int backward_impl(const dsoft_plan_t* p, const void* gathered, const void
   if (!p || !gathered || !state || !scratch || !lse_all || !gout || !lambdas || !d_image || !d_text || !d_scale)
     return fail(DSOFT_EINVAL, "null argument");
   if (p->have_proj && !d_student) return fail(DSOFT_EINVAL, "d_student is null but the plan has Dp > 0");
-  if (p->weighted && !p->gmat)
-    return fail(DSOFT_EINVAL, "the weighted CE branch needs the two-phase backward (DSOFT_F_GMAT)");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   // state is logically const for the caller; the relayouted LSE columns live in it
   float* S = const_cast<float*>(static_cast<const float*>(state));
@@ -2760,6 +2763,7 @@ static int backward_impl(const dsoft_plan_t* p, const void* gathered, const void
   } else {
   if ((rc = set_smem(dsoft_bwd_kernel<MODE_CLIP>, BWD_SMEM_BYTES))) return rc;
   if ((rc = set_smem(dsoft_bwd_kernel<MODE_SOFT>, BWD_SMEM_BYTES))) return rc;
+  if (p->weighted && (rc = set_smem(dsoft_bwd_kernel<MODE_WCE_X>, BWD_SMEM_BYTES))) return rc;
 
   BwdParams P;
   auto base = [&](const SplitPlan& sp, int col0, int ncols, int ntiles) {
@@ -2831,6 +2835,37 @@ static int backward_impl(const dsoft_plan_t* p, const void* gathered, const void
     }
   }
 
+  // weighted CE branch: the CLIP launches below run MODE_WCE_X instead, whose G carries g_c * classic CE + g_w *
+  // weighted CE of the pair's two directions (MODE_WCE_G's entry), from a CLIP and a DINO tile per column tile.  Row
+  // side = this rank's rows of direction d, column side = the other direction's per-row statistics by global column
+  // (world 1: st_wstat by global row is that view; world > 1: wce_relayout_kernel above).  There is no transposed
+  // GEMM here, so each launch takes its own direction's d(logit_scale) row term (wsplit) at every world size.
+  auto set_wce = [&](int d) {
+    const size_t r0 = static_cast<size_t>(p->sh.rank) * b;
+    const float* wr = S + p->st_wstat + static_cast<size_t>(d) * 4 * p->Bcol;      // row-side direction
+    const float* wc = S + p->st_wstat + static_cast<size_t>(1 - d) * 4 * p->Bcol;  // column-side direction
+    P.nprod = 2;
+    P.a_map[1] = P.b_map[1] = 3;  // DINO cosine
+    P.kchunks[1] = ceil_div(p->sh.Dd, BK);
+    P.rinv_d = S + p->st_rinv_d;
+    P.wrow[0] = lse_loc + d * b;
+    P.wrow[1] = wr + WS_C * p->Bcol + r0;
+    P.wrow[2] = wr + WS_LSET * p->Bcol + r0;
+    P.wrow[3] = wr + WS_A * p->Bcol + r0;
+    P.wcol[0] = lsec + static_cast<size_t>(1 - d) * p->Bcol;  // lse of the other direction, by column
+    P.wcol[1] = wc + WS_LSET * p->Bcol;                       // (only read when that direction is modulated)
+    P.wcol[2] = wc + WS_C * p->Bcol;
+    P.wcol[3] = wc + WS_A * p->Bcol;
+    P.wdir = d;
+    P.wsym = d == 0 ? p->wsym : 1;
+    P.wrow_plain = d == 1 && !p->wsym;
+    P.wsplit = 1;
+    P.wcc = p->sh.c_clip;
+    P.wlam[0] = lambdas[0];
+    P.wlam[1] = lambdas[3];
+    P.wgout = gout;
+  };
+  auto clip_kernel = p->weighted ? dsoft_bwd_kernel<MODE_WCE_X> : dsoft_bwd_kernel<MODE_CLIP>;
   // ---- CLIP, image rows: d image = s/(2b) sum_j (p_it[a,j] + p_ti[j,a]) T_j - ...
   base(p->b_clip, 0, p->B, p->ntiles_g);
   P.nprod = 1;
@@ -2844,10 +2879,11 @@ static int backward_impl(const dsoft_plan_t* p, const void* gathered, const void
   P.lse_col = lsec + 1 * p->Bcol;
   P.acc_part = X + p->sc_acc1;
   P.ds_part = X + p->sc_ds1;
+  if (p->weighted) set_wce(0);
   if ((rc = fk.lane(lane++, &ks))) return rc;
   {
     ProfScope ps(PK_BWD_CLIP_I, ks);
-    if ((rc = launch_bwd(dsoft_bwd_kernel<MODE_CLIP>, p->nch_clip, rbs, p->b_clip.nsplit, ks, tm, vmap, P))) return rc;
+    if ((rc = launch_bwd(clip_kernel, p->nch_clip, rbs, p->b_clip.nsplit, ks, tm, vmap, P))) return rc;
   }
   CUDA_TRY(cudaGetLastError());
   // ---- CLIP, text rows
@@ -2858,10 +2894,11 @@ static int backward_impl(const dsoft_plan_t* p, const void* gathered, const void
   P.lse_col = lsec + 0 * p->Bcol;
   P.acc_part = X + p->sc_acc2;
   P.ds_part = X + p->sc_ds2;
+  if (p->weighted) set_wce(1);
   if ((rc = fk.lane(lane++, &ks))) return rc;
   {
     ProfScope ps(PK_BWD_CLIP_T, ks);
-    if ((rc = launch_bwd(dsoft_bwd_kernel<MODE_CLIP>, p->nch_clip, rbs, p->b_clip.nsplit, ks, tm, vmap, P))) return rc;
+    if ((rc = launch_bwd(clip_kernel, p->nch_clip, rbs, p->b_clip.nsplit, ks, tm, vmap, P))) return rc;
   }
   CUDA_TRY(cudaGetLastError());
 

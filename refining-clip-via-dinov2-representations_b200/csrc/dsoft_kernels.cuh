@@ -51,6 +51,7 @@ constexpr int MODE_WCE_STAT = 5;
 constexpr int MODE_WCE_LSE = 6;
 constexpr int MODE_WCE_DBG = 7;
 constexpr int MODE_WCE_G = 8;
+constexpr int MODE_WCE_X = 9;  // fused backward (dsoft_bwd_kernel) of the same logit gradient: no G matrix in HBM
 constexpr int MODE_SOFT_SYM16 = 13;  // forward soft statistics, upper block triangle + column reductions, on a
                                      // 16x256b TMEM load shape (4 rows per thread: short butterflies)
 constexpr int MODE_LINEAR = 11;   // projection head layer: out = act(A . W^T + bias) as bf16 (loss.py:214-238, 322-347)
@@ -189,7 +190,53 @@ struct BwdParams {
   const float* rinv_y;
   float* acc_part;         // [nsplit][b][dout] fp32
   float* ds_part;          // [nsplit * C * 2][b]
+  // ---- weighted CE (MODE_WCE_X): products [0] CLIP (row side = direction wdir), [1] DINO; the fields mean what the
+  // MODE_WCE_G fields of FwdParams mean (rinv_d: 1/||dino|| by global index, read for rows and columns)
+  const float* wrow[4];    // per local row: [0] lse (log2), [1] c_a, [2] lse~ (log2), [3] A_a
+  const float* wcol[4];    // by global column, of the OTHER direction: [0] lse, [1] lse~, [2] c', [3] A'
+  int wdir, wsym, wrow_plain, wsplit;
+  float wcc;
+  float wlam[2];           // lambda_original, lambda_weighted
+  const float* wgout;      // upstream gradients [6] (device)
 };
+
+// Weighted CE logit gradient of one pair (row a of direction wdir, column j), MODE_WCE_G and MODE_WCE_X:
+//   g  = g_c (e1 + e2) + g_w (gimg + gtxt),  d CE~_a / d x_aj = p~_aj - beta A_a p_aj (r_aj - c_a)  (j != a)
+//   gr = this row's own loss terms (world > 1 or the fused backward: the other direction's launch holds the rest)
+// e1 / gimg are the row side's classic / modulated terms, e2 / gtxt the column side's (the other direction's entry of
+// the same pair, statistics by column); x is the CLIP logit in log2 units, r the DINO dissimilarity.  The switches
+// (wrow_plain, wsym, wsplit, row_only) are read from the kernel parameters P (FwdParams or BwdParams) at each use, as
+// the kernel-parameter bank costs no registers.
+struct WceRowK {
+  float lse, c, lset, aa;      // row side: lse, c_a, lse~, A_a
+  float beta, beta2;           // row side: beta, beta log2(e)
+  float beta_t, beta2_t;       // column side
+  float cc, gcl, gwt;          // c_clip, g_c, g_w
+};
+struct WcePair { float g, gr; };
+template <class Params>
+__device__ __forceinline__ WcePair wce_pair(const Params& P, const WceRowK& k, float x, float r, float lse_j,
+                                            float lset_j, float c_j, float aa_j) {
+  const float za = r - k.c;
+  const float e1 = fast_exp2(x - k.lse);
+  float gimg = e1;  // row-side direction (the image direction unless wdir == 1)
+  if (!P.wrow_plain) {
+    const float pt = fast_exp2(fmaf(k.beta2, fminf(fmaxf(za, -k.cc), k.cc), x) - k.lset);
+    gimg = pt - k.beta * k.aa * e1 * za;
+  }
+  float e2 = fast_exp2(x - lse_j);
+  float gtxt = e2;
+  if (P.wsym) {
+    const float zj = r - c_j;
+    const float ptj = fast_exp2(fmaf(k.beta2_t, fminf(fmaxf(zj, -k.cc), k.cc), x) - lset_j);
+    gtxt = ptj - k.beta_t * aa_j * e2 * zj;
+  }
+  if (P.wsplit && P.row_only) e2 = gtxt = 0.f;  // gathered columns carry no gradient
+  WcePair o;
+  o.g = k.gcl * (e1 + e2) + k.gwt * (gimg + gtxt);
+  o.gr = P.wsplit ? k.gcl * e1 + k.gwt * gimg : o.g;
+  return o;
+}
 
 __device__ __forceinline__ uint8_t* align_1024(uint8_t* p) {
   uintptr_t a = reinterpret_cast<uintptr_t>(p);
@@ -1230,14 +1277,19 @@ dsoft_fwd_kernel(const __grid_constant__ TileMaps maps, const __grid_constant__ 
       for (int k = 0; k < 11; ++k) acc[k] = 0.f;
       float mrun = M_FLOOR;
       // G mode: upstream gradients and the text direction's knobs
-      float gcl = 0.f, gwt = 0.f, beta_i = 0.f, beta_t = 0.f, beta2_t = 0.f, aa_a = 0.f;
+      WceRowK wk{};
       if constexpr (MODE == MODE_WCE_G) {
-        gcl = P.wgout[0] + P.wlam[0] * P.wgout[4];
-        gwt = P.wgout[5] + P.wlam[1] * P.wgout[4];
-        beta_i = P.scal[SC_WBETA + P.wdir];  // row-side direction
-        beta_t = P.scal[SC_WBETA + 1 - P.wdir];
-        beta2_t = P.scal[SC_WBETA2 + 1 - P.wdir];
-        aa_a = P.wrow[3][lic];
+        wk.lse = lse_a;
+        wk.c = c_a;
+        wk.lset = lset_a;
+        wk.aa = P.wrow[3][lic];
+        wk.beta = P.scal[SC_WBETA + P.wdir];  // row-side direction
+        wk.beta2 = beta2;
+        wk.beta_t = P.scal[SC_WBETA + 1 - P.wdir];
+        wk.beta2_t = P.scal[SC_WBETA2 + 1 - P.wdir];
+        wk.cc = cc;
+        wk.gcl = P.wgout[0] + P.wlam[0] * P.wgout[4];
+        wk.gwt = P.wgout[5] + P.wlam[1] * P.wgout[4];
       }
       int it = 0;
       for (int t = t0; t < t1; ++t, it += 2) {
@@ -1381,23 +1433,9 @@ dsoft_fwd_kernel(const __grid_constant__ TileMaps maps, const __grid_constant__ 
                 for (int k = 0; k < 4; ++k) {
                   const int e = 4 * e4 + k;
                   const float x = xq[c * 32 + e];
-                  const float za = r[e] - c_a;
-                  const float e1 = fast_exp2(x - lse_a);
-                  float gimg = e1;  // row-side direction (the image direction unless wdir == 1)
-                  if (!P.wrow_plain) {
-                    const float pt = fast_exp2(fmaf(beta2, fminf(fmaxf(za, -cc), cc), x) - lset_a);
-                    gimg = pt - beta_i * aa_a * e1 * za;
-                  }
-                  float e2 = fast_exp2(x - lti[k]);
-                  float gtxt = e2;
-                  if (P.wsym) {
-                    const float zj = r[e] - cj[k];
-                    const float ptj = fast_exp2(fmaf(beta2_t, fminf(fmaxf(zj, -cc), cc), x) - ltt[k]);
-                    gtxt = ptj - beta_t * aj[k] * e2 * zj;
-                  }
-                  if (P.wsplit && P.row_only) e2 = gtxt = 0.f;  // gathered columns carry no gradient
-                  float g = gcl * (e1 + e2) + gwt * (gimg + gtxt);
-                  float gr = P.wsplit ? gcl * e1 + gwt * gimg : g;  // this rank's own loss terms
+                  const WcePair wp = wce_pair(P, wk, x, r[e], lti[k], ltt[k], cj[k], aj[k]);
+                  float g = wp.g;
+                  float gr = wp.gr;  // this rank's own loss terms
                   if (need_mask && ((jrel0 + e == gi) || (jrel0 + e >= P.ncols) || !live_row)) g = gr = 0.f;
                   acc[0] = fmaf(gr, x, acc[0]);  // d(logit_scale) row term in log2 units of x (off-diagonal part)
                   g4[k] = g;
@@ -1740,6 +1778,9 @@ dsoft_fwd_kernel(const __grid_constant__ TileMaps maps, const __grid_constant__ 
 //             -2 one-hot part and the s/(2b) factor are applied in fp32 by the finalize kernel)
 //  MODE_SOFT: G_aj = [(2^(p-ls_a) + 2^(p-ls_j)) - (2^(q-lt_a) + 2^(q-lt_j))] / (||y_j|| sigma), j != a
 //             (diagonal dropped: it is parallel to y_a and vanishes in the normalise backward)
+//  MODE_WCE_X: G_aj = the weighted CE entry of MODE_WCE_G (wce_pair) for the rows of one direction, from a CLIP
+//             tile and a DINO tile per column tile (diagonal dropped, applied in fp32 by the finalize kernel); one
+//             launch per direction, each with the row-side d(logit_scale) term only (wsplit), as MODE_CLIP
 //  row_only drops the *_j (column-side) terms: gathered features are constants (gather_with_grad=0).
 //  G is stored as fp16 (10-bit mantissa) and multiplied with an EXACT fp16 copy of the gradient operand
 //  (bf16 features times a power of two sigma): bf16 G costs 8x the rounding error, mixed fp16 x bf16
@@ -1981,11 +2022,28 @@ dsoft_bwd_kernel(const __grid_constant__ TileMaps maps, const __grid_constant__ 
     } else if constexpr (MODE == MODE_CLIP) {
       c_a = P.scal[SC_SCALE_L2];
       l_a = P.lse_row[lic];
+    } else if constexpr (MODE == MODE_WCE_X) {
+      c_a = P.scal[SC_SCALE_L2];
+      c_b = P.rinv_d[gi];
     } else {
       c_a = P.rinv_d[gi] * P.scal[SC_ITT_L2];  // teacher
       l_a = P.lse_t_row[lic];
       c_b = P.rinv_y[gi] * P.scal[P.tau_idx];  // student / text
       l_b = P.lse_y_row[lic];
+    }
+    WceRowK wk{};
+    if constexpr (MODE == MODE_WCE_X) {
+      wk.lse = P.wrow[0][lic];
+      wk.c = P.wrow[1][lic];
+      wk.lset = P.wrow[2][lic];
+      wk.aa = P.wrow[3][lic];
+      wk.beta = P.scal[SC_WBETA + P.wdir];
+      wk.beta2 = P.scal[SC_WBETA2 + P.wdir];
+      wk.beta_t = P.scal[SC_WBETA + 1 - P.wdir];
+      wk.beta2_t = P.scal[SC_WBETA2 + 1 - P.wdir];
+      wk.cc = P.wcc;
+      wk.gcl = P.wgout[0] + P.wlam[0] * P.wgout[4];
+      wk.gwt = P.wgout[5] + P.wlam[1] * P.wgout[4];
     }
 
     // 32 fp32 -> fp16, 4 x 16-byte swizzled stores into the K-major SW128 A-operand layout
@@ -2008,7 +2066,60 @@ dsoft_bwd_kernel(const __grid_constant__ TileMaps maps, const __grid_constant__ 
       const int slot0 = it % B_SLOTS;
       const int jt0 = t * BN + half * 64;  // first column (relative to col0) of this thread's 64 columns
 
-      if constexpr (MODE == MODE_SOFT) {
+      if constexpr (MODE == MODE_WCE_X) {
+        // ---- CLIP tile first: the raw dot products stay in registers and the TMEM slot is handed back at once,
+        // as in MODE_SOFT
+        float Xd[64];
+        const int slot1 = (it + 1) % B_SLOTS;
+        mbar_wait(smem_u32(&s_full[slot0]), static_cast<uint32_t>(it / B_SLOTS) & 1);
+        tc_fence_after();
+#pragma unroll
+        for (int c = 0; c < 2; ++c) {
+          tmem_ld32(lane_addr + slot0 * BN + half * 64 + c * 32, v);
+#pragma unroll
+          for (int e = 0; e < 32; ++e) Xd[c * 32 + e] = v[e];
+        }
+        tc_fence_before();
+        mbar_arrive(smem_u32(&s_empty[slot0]));
+        // ---- DINO tile: r = 1 - clamp(cos), then the pair's weighted logit gradient (MODE_WCE_G's arithmetic)
+        mbar_wait(smem_u32(&s_full[slot1]), static_cast<uint32_t>((it + 1) / B_SLOTS) & 1);
+        tc_fence_after();
+        if (r > 0) mbar_wait(smem_u32(g_free), static_cast<uint32_t>(r - 1) & 1);
+#pragma unroll
+        for (int c = 0; c < 2; ++c) {
+          const int jrel0 = jt0 + c * 32;
+          const int gj0 = P.col0 + jrel0;
+          float g[32];
+          tmem_ld32(lane_addr + slot1 * BN + half * 64 + c * 32, v);
+          const float4* rc = reinterpret_cast<const float4*>(P.rinv_d + gj0);
+          const float4* l1c = reinterpret_cast<const float4*>(P.wcol[0] + gj0);
+          const float4* l2c = reinterpret_cast<const float4*>(P.wcol[1] + gj0);
+          const float4* ccc = reinterpret_cast<const float4*>(P.wcol[2] + gj0);
+          const float4* aac = reinterpret_cast<const float4*>(P.wcol[3] + gj0);
+#pragma unroll
+          for (int e4 = 0; e4 < 8; ++e4) {
+            const float4 r4 = __ldg(rc + e4), a4 = __ldg(l1c + e4), b4 = __ldg(l2c + e4);
+            const float4 c4 = __ldg(ccc + e4), d4 = __ldg(aac + e4);
+            const float rr[4] = {r4.x, r4.y, r4.z, r4.w};
+            const float lj[4] = {a4.x, a4.y, a4.z, a4.w}, ltj[4] = {b4.x, b4.y, b4.z, b4.w};
+            const float cj[4] = {c4.x, c4.y, c4.z, c4.w}, aj[4] = {d4.x, d4.y, d4.z, d4.w};
+#pragma unroll
+            for (int k = 0; k < 4; ++k) {
+              const int e = 4 * e4 + k;
+              const float rd = 1.f - fminf(fmaxf(v[e] * c_b * rr[k], -1.f), 1.f);
+              const float dot = Xd[c * 32 + e];
+              const WcePair wp = wce_pair(P, wk, dot * c_a, rd, lj[k], ltj[k], cj[k], aj[k]);
+              // diagonal (r_aa = 0: applied in fp32 by finalize_bwd_kernel) and ragged columns dropped
+              const bool dead = (gj0 + e == gi) || (jrel0 + e >= P.ncols);
+              dsacc = fmaf(dead ? 0.f : wp.gr, dot, dsacc);
+              g[e] = dead ? 0.f : wp.g;
+            }
+          }
+          store_g(g, c);
+        }
+        tc_fence_before();
+        mbar_arrive(smem_u32(&s_empty[slot1]));
+      } else if constexpr (MODE == MODE_SOFT) {
         // ---- teacher tile first: E = -(2^(q-lt_a) + 2^(q-lt_j)) stays in registers and the TMEM slot is
         // handed back at once, so the next tile's teacher MMAs overlap the rest of this epilogue
         float E[64];
@@ -2152,7 +2263,7 @@ dsoft_bwd_kernel(const __grid_constant__ TileMaps maps, const __grid_constant__ 
     }
     // d(logit_scale) row term: this CTA saw only its own column tiles -> one partial per (split, cluster
     // rank, half); written by the CTAs of the first chunk group only
-    if (MODE == MODE_CLIP && P.want_ds && P.chunk0 == 0 && li < P.b)
+    if ((MODE == MODE_CLIP || MODE == MODE_WCE_X) && P.want_ds && P.chunk0 == 0 && li < P.b)
       P.ds_part[((split * csize + crank) * 2 + half) * P.b + li] = dsacc;
   }
 

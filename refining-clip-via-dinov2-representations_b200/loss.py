@@ -424,9 +424,11 @@ class _DinoSoftFn(torch.autograd.Function):
         needs_grad = any(ctx.needs_input_grad[:4]) or any(ctx.needs_input_grad[6:])
         fused_head = w1 is not None  # the head runs inside (dsoft_head_forward); `student` is None
         flags = cfg.flags
-        # the weighted branch's backward exists in the two-phase form only
-        if needs_grad and (weighted or _gmat_fits(b, W, soft, bool(flags & _cabi.DSOFT_F_TEXT),
-                                                  bool(flags & _cabi.DSOFT_F_SOFT_LOCAL), dev)):
+        # weighted plans take the two-phase backward unless GMAT == "never" (the memory rule does not cover their
+        # matrices); when its scratch cannot be allocated, the backward below falls back to the fused form
+        if needs_grad and ((weighted and GMAT != "never") or
+                           _gmat_fits(b, W, soft, bool(flags & _cabi.DSOFT_F_TEXT),
+                                      bool(flags & _cabi.DSOFT_F_SOFT_LOCAL), dev)):
             flags |= _cabi.DSOFT_F_GMAT
         shape = _cabi.Shape(
             b=b, world=W, rank=r, D=D,
@@ -508,7 +510,7 @@ class _DinoSoftFn(torch.autograd.Function):
             # the fp16 logit-gradient matrices fitted when this shape was first seen but do not now: the saved
             # forward state does not depend on the backward implementation, so run the fused backward instead
             s = plan.shape
-            if not (s.flags & _cabi.DSOFT_F_GMAT) or (s.flags & _cabi.DSOFT_F_WEIGHTED):
+            if not (s.flags & _cabi.DSOFT_F_GMAT):
                 raise
             for key in [k for k in _gmat_decisions if k[0] == s.b and k[1] == s.world]:
                 _gmat_decisions[key] = False
