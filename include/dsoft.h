@@ -25,7 +25,8 @@
 extern "C" {
 #endif
 
-#define DSOFT_VERSION 240 /* 0.2.4: weighted plans accept the fused backward (no DSOFT_F_GMAT); 0.2.3: weighted
+#define DSOFT_VERSION 250 /* 0.2.5: retrieval ranks (dsoft_retrieval_ranks); 0.2.4: weighted plans accept the fused
+                             backward (no DSOFT_F_GMAT); 0.2.3: weighted
                              CE branch at world > 1 (phases 5 / 6, dsoft_plan_lse_rows, dsoft_plan_wsigma_info) */
 
 /* error codes */
@@ -188,6 +189,24 @@ int dsoft_pair_stats(const void* clip_a_dev, const void* clip_b_dev, int32_t k_c
                      const void* dino_b_dev, int32_t k_dino, int32_t n, const float* cmin, const float* dmax,
                      int32_t n_thr, unsigned long long* counts_dev, float gap_floor, void* cand_dev,
                      uint32_t cand_cap, uint32_t* cand_count_dev, void* stream);
+
+/* Retrieval ranks of open_clip's get_clip_metrics (open_clip_train/train.py) without the [n_img x n_txt] logit
+ * matrix.  s_ij = <img_i, txt_j> (bf16 operands [n][k] row-major, fp32 accumulation, features used as given); t(j) =
+ * text_image_dev[j], the image caption j belongs to (NULL: t(j) = j, which needs n_img == n_txt).
+ *   rank_img_dev[i] = #{j : t(j) != i, s_ij > p_i},  p_i = max over the captions of image i of s_ij
+ *   rank_txt_dev[j] = #{i : i != t(j), s_ij > s_t(j),j}
+ * i.e. the 0-based position of the (first) positive in a descending sort, ties counted in the query's favour (strict
+ * >).  The positives s_t(j),j and p_i come from an fp32 pre-pass over the same operands; the tile pass masks the
+ * positives themselves, so a positive never counts against its own query.  Pass a == b-style split operands
+ * img = [hi | lo | hi], txt = [hi | hi | lo] (k = 3 d) for fp32 features at ~1e-5 score accuracy, as for
+ * dsoft_pair_stats.  Every map entry must lie in [0, n_img) and every image must have a caption (not checked on
+ * the device: an entry out of range makes that caption count nothing, an image without caption gets rank n_txt).  Both rank arrays are written (no zeroing by the caller).  Operands and scratch 16-byte
+ * aligned, k a multiple of 8; scratch_dev holds dsoft_retrieval_scratch_bytes(n_img, n_txt) bytes, O(n_img + n_txt).
+ * Asynchronous on `stream`, no host synchronisation (graph-capturable). */
+size_t dsoft_retrieval_scratch_bytes(int32_t n_img, int32_t n_txt);
+int dsoft_retrieval_ranks(const void* img_dev, const void* txt_dev, int32_t k, int32_t n_img, int32_t n_txt,
+                          const int32_t* text_image_dev, int32_t* rank_img_dev, int32_t* rank_txt_dev,
+                          void* scratch_dev, void* stream);
 
 /* Column (in elements) of the DINO block inside a packed row: where dsoft_gather_rows must write when the caller
  * fills the DINO columns of `gathered` itself (dsoft_pack with dino_dev == NULL). */

@@ -10,6 +10,7 @@ Import as ``dinosoft_b200`` (see the shim at the repo root).  Contents:
                  moment matrices (SURVEY 8f-4)
     graphed.py   CUDA-graph capture of the loss forward + backward (launch-bound small batches)
     pair_stats.py  CLIP-blind pair statistics on the Gram-tile kernel (helpers.py:221-285, SURVEY 8f-4)
+    retrieval.py  retrieval ranks and R@K (open_clip get_clip_metrics) on the Gram-tile kernel, no N x N logits
     _cabi.py     ctypes binding of libdsoft.so (include/dsoft.h)
     _build.py    nvcc recipe for csrc/ (sm_100a only)
     csrc/        hand-written tcgen05 / TMEM / TMA kernels + the C ABI
@@ -20,6 +21,7 @@ from .feature_store import DinoFeatureStore, DinoRows, lookup as dino_lookup, to
 from .cyclip import CyCLIPLoss
 from .graphed import make_graphed
 from .pair_stats import pair_stats
+from .retrieval import clip_metrics, retrieval_ranks
 from .loss import (
     ClipLossWithDINOEnhancements,
     CudaBackend,
@@ -43,6 +45,8 @@ __all__ = [
     "to_device_table",
     "dino_lookup",
     "pair_stats",
+    "retrieval_ranks",
+    "clip_metrics",
     "CyCLIPLoss",
     "make_graphed",
 ]

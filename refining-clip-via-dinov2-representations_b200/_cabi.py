@@ -58,6 +58,9 @@ PROTOTYPES = {
     "dsoft_pair_stats": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32,
                                    C.POINTER(C.c_float), C.POINTER(C.c_float), C.c_int32, C.c_void_p, C.c_float,
                                    C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p]),
+    "dsoft_retrieval_scratch_bytes": (C.c_size_t, [C.c_int32, C.c_int32]),
+    "dsoft_retrieval_ranks": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_void_p,
+                                        C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "dsoft_head_forward": (C.c_int, [C.c_void_p] * 6 + [C.c_int32, C.c_void_p, C.c_void_p]),
     "dsoft_forward": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(C.c_float)] + [C.c_void_p] * 6),
     "dsoft_backward": (C.c_int, [C.c_void_p] * 6 + [C.POINTER(C.c_float)] + [C.c_void_p] * 5),

@@ -2179,6 +2179,137 @@ extern "C" int dsoft_pair_stats(const void* clip_a, const void* clip_b, int32_t 
   return launch_fwd_pair(dsoft_fwd_kernel<MODE_PAIRS, 2>, ceil_div(n, BM), nsplit, st, tm, P);
 }
 
+// ------------------------------------------------------------------------------------------------
+// Retrieval ranks (open_clip get_clip_metrics, open_clip_train/train.py) on the Gram-tile kernel: MODE_RANKS counts,
+// per image and per caption, the non-positive scores above the positive's.  The thresholds come from a small fp32
+// pre-pass over the same bf16 operands; nothing of size n_img x n_txt exists.
+// Scratch: thr [n_txt padded to 256] fp32 | t(j) [same] int32 | p [n_img padded to 64] fp32
+// ------------------------------------------------------------------------------------------------
+static size_t rk_cols(int n_txt) { return static_cast<size_t>(ceil_div(n_txt, 2 * BN)) * (2 * BN); }
+
+extern "C" size_t dsoft_retrieval_scratch_bytes(int32_t n_img, int32_t n_txt) {
+  if (n_img <= 0 || n_txt <= 0) return 0;
+  return 4 * (2 * rk_cols(n_txt) + align_up(static_cast<size_t>(n_img), 64));
+}
+
+// thr = +inf and t(j) = -1 past n_txt (nothing counts there), p = -inf, ranks = 0
+__global__ void rk_init_kernel(const int32_t* __restrict__ tmap_in, int n_img, int n_txt, int ncols_pad,
+                               float* __restrict__ thr, int* __restrict__ tmap, float* __restrict__ p,
+                               int* __restrict__ rank_img, int* __restrict__ rank_txt) {
+  const int n = max(ncols_pad, n_img);
+  for (int k = blockIdx.x * blockDim.x + threadIdx.x; k < n; k += gridDim.x * blockDim.x) {
+    if (k < ncols_pad) {
+      thr[k] = __int_as_float(0x7f800000);
+      tmap[k] = (k < n_txt && tmap_in) ? tmap_in[k] : -1;
+      if (k < n_txt) rank_txt[k] = 0;
+    }
+    if (k < n_img) {
+      p[k] = __int_as_float(static_cast<int>(0xff800000u));
+      rank_img[k] = 0;
+    }
+  }
+}
+
+// float maximum through integer atomics (order-independent): non-negative floats order as signed ints, negative ones
+// in reverse as unsigned ints; -0.0 takes the unsigned path so that it still replaces -inf
+__device__ __forceinline__ void atomic_max_f32(float* a, float v) {
+  if (!signbit(v)) atomicMax(reinterpret_cast<int*>(a), __float_as_int(v));
+  else atomicMin(reinterpret_cast<unsigned int*>(a), __float_as_uint(v));
+}
+
+// one warp per caption j: thr_j = <img[t(j)], txt[j]> in fp32 from the bf16 operands, p_t(j) = max(p_t(j), thr_j).
+// A map entry outside [0, n_img) leaves thr_j = +inf (the caption counts nothing) instead of reading out of bounds.
+__global__ void rk_thr_kernel(const __nv_bfloat16* __restrict__ img, const __nv_bfloat16* __restrict__ txt, int k,
+                              int n_img, int n_txt, const int* __restrict__ tmap, int mapped, float* __restrict__ thr,
+                              float* __restrict__ p) {
+  const int j = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  const int lane = threadIdx.x & 31;
+  if (j >= n_txt) return;
+  const int i = mapped ? tmap[j] : j;
+  if (i < 0 || i >= n_img) return;
+  const uint4* a = reinterpret_cast<const uint4*>(img + static_cast<size_t>(i) * k);
+  const uint4* b = reinterpret_cast<const uint4*>(txt + static_cast<size_t>(j) * k);
+  float acc = 0.f;
+  for (int c = lane; c < k / 8; c += 32) {
+    const uint4 x = __ldg(a + c), y = __ldg(b + c);
+    const __nv_bfloat162* xa = reinterpret_cast<const __nv_bfloat162*>(&x);
+    const __nv_bfloat162* ya = reinterpret_cast<const __nv_bfloat162*>(&y);
+#pragma unroll
+    for (int h = 0; h < 4; ++h) {
+      const float2 xf = __bfloat1622float2(xa[h]), yf = __bfloat1622float2(ya[h]);
+      acc = fmaf(xf.x, yf.x, acc);
+      acc = fmaf(xf.y, yf.y, acc);
+    }
+  }
+#pragma unroll
+  for (int o = 16; o; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
+  if (lane == 0) {
+    thr[j] = acc;
+    if (mapped) atomic_max_f32(p + i, acc);
+    else p[i] = acc;
+  }
+}
+
+extern "C" int dsoft_retrieval_ranks(const void* img, const void* txt, int32_t k, int32_t n_img, int32_t n_txt,
+                                     const int32_t* text_image, int32_t* rank_img, int32_t* rank_txt, void* scratch,
+                                     void* stream) {
+  if (!img || !txt || !rank_img || !rank_txt || !scratch) return fail(DSOFT_EINVAL, "null argument");
+  if (n_img <= 0 || n_txt <= 0 || k <= 0 || k % 8)
+    return fail(DSOFT_EINVAL, "need n_img, n_txt > 0 and a feature width that is a positive multiple of 8 "
+                              "(n_img=%d n_txt=%d k=%d)", n_img, n_txt, k);
+  if (!text_image && n_img != n_txt)
+    return fail(DSOFT_EINVAL, "without a caption -> image map n_img must equal n_txt (%d, %d)", n_img, n_txt);
+  for (const void* q : {img, txt, static_cast<const void*>(scratch)})
+    if (reinterpret_cast<uintptr_t>(q) % 16) return fail(DSOFT_EINVAL, "operands and scratch must be 16-byte aligned");
+  int sms = 0, rc = query_num_sms(&sms);
+  if (rc) return rc;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const int ncols_pad = static_cast<int>(rk_cols(n_txt));
+  float* thr = static_cast<float*>(scratch);
+  int* tmap = reinterpret_cast<int*>(thr + ncols_pad);
+  float* pmax = reinterpret_cast<float*>(tmap + ncols_pad);
+  const int mapped = text_image != nullptr;
+  const int ninit = std::max(ncols_pad, static_cast<int>(n_img));
+  rk_init_kernel<<<std::min(ceil_div(ninit, 256), 4 * sms), 256, 0, st>>>(text_image, n_img, n_txt, ncols_pad, thr,
+                                                                          tmap, pmax, rank_img, rank_txt);
+  CUDA_TRY(cudaGetLastError());
+  const __nv_bfloat16* a = static_cast<const __nv_bfloat16*>(img);
+  const __nv_bfloat16* b = static_cast<const __nv_bfloat16*>(txt);
+  rk_thr_kernel<<<ceil_div(n_txt, 8), 256, 0, st>>>(a, b, k, n_img, n_txt, tmap, mapped, thr, pmax);
+  CUDA_TRY(cudaGetLastError());
+
+  TileMaps tm;
+  const CUtensorMapDataType bf = CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
+  if ((rc = make_map(&tm.m[0], img, n_img, k, static_cast<size_t>(k), bf, 64))) return rc;
+  if ((rc = make_map(&tm.m[1], txt, n_txt, k, static_cast<size_t>(k), bf, 64))) return rc;
+  tm.m[2] = tm.m[3] = tm.g[0] = tm.g[1] = tm.m[0];
+  FwdParams P;
+  memset(&P, 0, sizeof(P));
+  P.nprod = 1;
+  P.a_map[0] = 0;
+  P.b_map[0] = 1;
+  P.kchunks[0] = ceil_div(k, BK);
+  P.bn = 2 * BN;
+  P.row0 = 0;
+  P.b = n_img;
+  P.col0 = 0;
+  P.ncols = n_txt;
+  P.ntiles = ceil_div(n_txt, 2 * BN);
+  const int rbs = ceil_div(n_img, BM);
+  const SplitPlan sp = choose_split(rbs, 1, P.ntiles, sms);
+  P.tiles_per_split = sp.tps;
+  P.npart = 2 * sp.nsplit;
+  P.ncolvec = mapped ? 2 : 1;
+  P.colvec[0] = thr;
+  P.colvec[1] = reinterpret_cast<const float*>(tmap);
+  P.rk_p = pmax;
+  P.rk_img = rank_img;
+  P.rk_txt = rank_txt;
+  P.rk_mapped = mapped;
+  if ((rc = set_smem(dsoft_fwd_kernel<MODE_RANKS, 2>, FWD_SMEM_BYTES))) return rc;
+  return launch_fwd_pair(dsoft_fwd_kernel<MODE_RANKS, 2>, rbs, sp.nsplit, st, tm, P);
+}
+
 // phase 0: the whole forward; of a DSOFT_SYM_W plan: 4 = operand statistics, 1 = the soft part up to the column-sum
 // exchange, 3 = the CLIP part (independent of 1 and of the exchange), 2 = finalize; of a weighted plan: 5 = up to the
 // weighted row statistics (row stds), 6 = median onward

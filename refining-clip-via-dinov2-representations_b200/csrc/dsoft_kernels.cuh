@@ -60,6 +60,8 @@ constexpr int MODE_PAIRS = 12;    // CLIP-blind pair statistics (open_clip_train
 constexpr int MODE_CLIP_SYM = 10; // forward CLIP statistics of BOTH directions from one pass over I . T^T: row
                                   // log-sum-exp partials as MODE_CLIP + per-warp column partials (the text -> image
                                   // direction is the transpose: loss.py:267/273 recomputes it)
+constexpr int MODE_RANKS = 14;    // retrieval ranks (open_clip get_clip_metrics): per image and per caption, the number
+                                  // of non-positive scores of I . T^T above its positive, over the full rectangle
 
 // scalar block computed on device by prep_scalars_kernel (no host sync on logit_scale)
 enum {
@@ -166,6 +168,12 @@ struct FwdParams {
   int wrap;                 // 0, or B: global column of primed tile t = (col0 + t * 256) mod wrap  (col0 == row0)
   int rb_half, ntiles_a;    // row blocks rb < rb_half own the primed tiles [diagonal, ntiles_a) only, the others
                             // [diagonal, ntiles): the contested half block of the rank pair (r, r + W/2)
+  // ---- retrieval ranks (MODE_RANKS): rows = images (b = n_img), columns = captions (ncols = n_txt); colvec[0] =
+  // the caption's threshold s_t(j),j (+inf past n_txt), colvec[1] = t(j) as int bits (rk_mapped only)
+  const float* rk_p;        // per image: p_i = max over its captions of s_ij
+  int* rk_img;              // += #{j : t(j) != i, s_ij > p_i}   (caller-zeroed)
+  int* rk_txt;              // += #{i : i != t(j), s_ij > s_t(j),j}
+  int rk_mapped;            // 0: t(j) = j (the positives are the diagonal), 1: t(j) from colvec[1]
 };
 
 struct BwdParams {
@@ -406,7 +414,9 @@ dsoft_fwd_kernel(const __grid_constant__ TileMaps maps, const __grid_constant__ 
   constexpr bool kWce = (MODE >= MODE_WCE_STAT && MODE <= MODE_WCE_G);
   // "soft-like": 256-column tiles with several products per tile, staged per-column vectors, setmaxnreg
   constexpr bool kPairs = (MODE == MODE_PAIRS);  // two products per tile like the weighted-CE passes, no column vectors
-  constexpr bool kSoftMode = (MODE == MODE_SOFT || MODE == MODE_SOFT_G || MODE == MODE_SOFT_SYM16 || kWce || kPairs);
+  constexpr bool kRanks = (MODE == MODE_RANKS);  // one product per tile, column vectors from P.colvec
+  constexpr bool kSoftMode = (MODE == MODE_SOFT || MODE == MODE_SOFT_G || MODE == MODE_SOFT_SYM16 || kWce || kPairs ||
+                              kRanks);
   static_assert(!kSoftMode || CG == 2, "the soft modes are written for CTA pairs");
   // streaming mode: stages of (A box | B boxes); resident mode: 8 A boxes, then B-only stages
   const bool resident = P.resident != 0;
@@ -494,7 +504,7 @@ dsoft_fwd_kernel(const __grid_constant__ TileMaps maps, const __grid_constant__ 
   // the register hand-over sits INSIDE the role branches: ptxas budgets the code dominated by a setmaxnreg with
   // its value (placed before the branch it compiled the whole kernel, epilogues included, for 56 registers)
   if (warp < EPI_WARP0) {
-  if constexpr (kSoftMode) setmaxnreg_dec<40>();
+  if constexpr (kSoftMode && !kRanks) setmaxnreg_dec<40>();  // the ranks epilogue fits the even split: no spills
   if (warp == 0) {
     // ------------------------------------------------------------------ TMA producer (warp-uniform loop)
     int stage = 0;
@@ -525,11 +535,11 @@ dsoft_fwd_kernel(const __grid_constant__ TileMaps maps, const __grid_constant__ 
         mbar_wait(smem_u32(&col_empty[cb]), ((static_cast<uint32_t>(n / COL_BUFS)) & 1) ^ 1);
         if (elect_one()) {
           const uint32_t full = smem_u32(&col_full[cb]);
-          const int nvec = (kWce || kPairs) ? P.ncolvec : (MODE == MODE_SOFT_G ? 2 : 1) * P.nprod;
+          const int nvec = (kWce || kPairs || kRanks) ? P.ncolvec : (MODE == MODE_SOFT_G ? 2 : 1) * P.nprod;
           mbar_arrive_expect_tx(full, nvec * CT * 4);
           float* dst = colbuf + cb * COL_VECS * CT;
           const size_t c0 = static_cast<size_t>(gcol(t));  // CT == bn == 256 in the soft modes
-          if constexpr (kWce || kPairs) {
+          if constexpr (kWce || kPairs || kRanks) {
             for (int k = 0; k < P.ncolvec; ++k) bulk_copy_g2s(smem_u32(dst + k * CT), P.colvec[k] + c0, CT * 4, full);
           } else {
             for (int p = 0; p < P.nprod; ++p) {
@@ -606,7 +616,7 @@ dsoft_fwd_kernel(const __grid_constant__ TileMaps maps, const __grid_constant__ 
   }
   } else {
     // ------------------------------------------------------------------ epilogue
-    if constexpr (kSoftMode) setmaxnreg_inc<232>();
+    if constexpr (kSoftMode && !kRanks) setmaxnreg_inc<232>();
     const int q = warp & 3;
     const int half = (warp - EPI_WARP0) >> 2;
     const int row = q * 32 + lane;
@@ -821,6 +831,75 @@ dsoft_fwd_kernel(const __grid_constant__ TileMaps maps, const __grid_constant__ 
           }
         }
       }
+    } else if constexpr (kRanks) {
+      // ---------------------------------------------------------------- retrieval ranks
+      // open_clip get_clip_metrics as counts over s = I . T^T (rows = images, columns = captions): a pair (i, j) is
+      // the positive when t(j) == i (1:1: the diagonal, warp-uniform per 32 x 32 chunk); every other pair counts
+      //   for image i   when s_ij > p_i       (row count, a register across this CTA's tiles, one atomic at the end)
+      //   for caption j when s_ij > thr_j     (ballot over the warp's 32 rows, summed over the CTA's 4 warps of a
+      //                                        column strip in shared memory, one atomic per column and tile)
+      // Integer sums: the result does not depend on the order of the atomics.  colsum is double-buffered by tile
+      // parity, so one named barrier per tile separates the shared sums of a tile from their flush.
+      int* colsum = reinterpret_cast<int*>(smem + 6 * 2 * TILE_BYTES + 16384);  // [2][256], behind colbuf
+      const int et = threadIdx.x - 32 * EPI_WARP0;                              // 0 .. 255
+      colsum[et] = 0;
+      colsum[CT + et] = 0;
+      named_bar_sync(1, NUM_EPI_THREADS);
+      const bool live_row = li < P.b;
+      const float prow = live_row ? P.rk_p[li] : 0.f;
+      const bool mapped = P.rk_mapped != 0;
+      unsigned int rcount = 0;
+      int it = 0;
+      for (int t = t0; t < t1; ++t, ++it) {
+        const int slot = it % nslots;
+        const int cb = it % COL_BUFS;
+        mbar_wait(smem_u32(&col_full[cb]), static_cast<uint32_t>(it / COL_BUFS) & 1);
+        mbar_wait(smem_u32(&s_full[slot]), static_cast<uint32_t>(it / nslots) & 1);
+        tc_fence_after();
+        const float* thr = colbuf + cb * COL_VECS * CT;
+        const int* tmap = reinterpret_cast<const int*>(thr + CT);
+        int* csum = colsum + (it & 1) * CT;
+#pragma unroll 1
+        for (int c = 0; c < 4; ++c) {
+          const int jt = half * 128 + c * 32;  // column in the tile
+          const int gj0 = t * CT + jt;
+          tmem_ld32(lane_addr + slot * CT + jt, v);
+          if (c == 3) {
+            tc_fence_before();
+            release_slot(slot);
+          }
+          if (gj0 >= P.ncols) continue;                 // warp-uniform
+          const bool ragged = gj0 + 32 > P.ncols;      // warp-uniform
+          unsigned int mine = 0;
+          if (mapped) {
+#pragma unroll
+            for (int e = 0; e < 32; ++e) {
+              const bool other = tmap[jt + e] != gi && (!ragged || gj0 + e < P.ncols);
+              rcount += (other && v[e] > prow) ? 1u : 0u;
+              const unsigned int bal = __ballot_sync(0xffffffffu, other && live_row && v[e] > thr[jt + e]);
+              if (lane == e) mine = __popc(bal);
+            }
+          } else {
+            const bool diag = gj0 == gw0;  // warp-uniform: rows and chunks are both 32-aligned
+#pragma unroll
+            for (int e = 0; e < 32; ++e) {
+              const bool other = !(diag && lane == e) && (!ragged || gj0 + e < P.ncols);
+              rcount += (other && v[e] > prow) ? 1u : 0u;
+              const unsigned int bal = __ballot_sync(0xffffffffu, other && live_row && v[e] > thr[jt + e]);
+              if (lane == e) mine = __popc(bal);
+            }
+          }
+          if (mine) atomicAdd(csum + jt + lane, static_cast<int>(mine));
+        }
+        mbar_arrive(smem_u32(&col_empty[cb]));
+        named_bar_sync(1, NUM_EPI_THREADS);
+        const int s = csum[et];
+        if (s) {
+          atomicAdd(P.rk_txt + t * CT + et, s);  // s > 0 only for columns < ncols (thr = +inf past them)
+          csum[et] = 0;
+        }
+      }
+      if (live_row && rcount) atomicAdd(P.rk_img + li, static_cast<int>(rcount));
     } else if constexpr (MODE == MODE_LINEAR) {
       // ---------------------------------------------------------------- projection-head layer
       // Row operand = the samples (image rows of the packed buffer, or the hidden activations), column operand =

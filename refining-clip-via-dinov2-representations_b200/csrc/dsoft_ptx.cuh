@@ -467,6 +467,11 @@ __device__ __forceinline__ void setmaxnreg_dec() {
   asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" ::"n"(N));
 }
 
+// Named barrier over a subset of the block's warps (nthreads a multiple of 32; id 0 is __syncthreads).
+__device__ __forceinline__ void named_bar_sync(uint32_t id, uint32_t nthreads) {
+  asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(nthreads) : "memory");
+}
+
 // Warp-wide float maximum / minimum in one instruction (sm_100a: redux.sync on f32, result in a uniform register)
 __device__ __forceinline__ float warp_max_f32(float x) {
   float r;

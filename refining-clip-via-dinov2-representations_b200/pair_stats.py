@@ -25,21 +25,38 @@ _CAND_CAP = 1 << 20
 
 def _operands(z: torch.Tensor) -> Tuple[torch.Tensor, torch.Tensor, int]:
     """(row operand, column operand, K) as contiguous bf16 matrices whose product is z z^T."""
-    if z.dim() != 2:
-        raise ValueError("expected a [N, d] matrix")
-    n, d = z.shape
+    return _operands_ab(z, z)
+
+
+def _operands_ab(x: torch.Tensor, y: torch.Tensor) -> Tuple[torch.Tensor, torch.Tensor, int]:
+    """(row operand, column operand, K) as contiguous bf16 matrices whose product is x y^T.
+
+    Two bf16 inputs are used as they are (widths zero-padded to a multiple of 8).  Anything else (fp32, and fp16,
+    which bf16 does not hold exactly) is split into bf16 (hi, lo) and multiplied as [hi | lo | hi] . [hi | hi | lo]^T.
+    """
+    if x.dim() != 2 or y.dim() != 2:
+        raise ValueError("expected [N, d] matrices")
+    if x.shape[1] != y.shape[1]:
+        raise ValueError(f"feature widths differ ({x.shape[1]} and {y.shape[1]})")
+    d = x.shape[1]
     pad = (-d) % 8
-    if z.dtype == torch.bfloat16:
-        a = torch.nn.functional.pad(z, (0, pad)).contiguous() if pad else z.contiguous()
-        return a, a, d + pad
-    z32 = z.float()
-    hi = z32.to(torch.bfloat16)
-    lo = (z32 - hi.float()).to(torch.bfloat16)
-    if pad:
-        hi = torch.nn.functional.pad(hi, (0, pad))
-        lo = torch.nn.functional.pad(lo, (0, pad))
-    a = torch.cat([hi, lo, hi], dim=1).contiguous()
-    b = torch.cat([hi, hi, lo], dim=1).contiguous()
+
+    def padded(t):
+        return torch.nn.functional.pad(t, (0, pad)) if pad else t
+
+    if x.dtype == torch.bfloat16 and y.dtype == torch.bfloat16:
+        a = padded(x).contiguous()
+        return a, (a if y is x else padded(y).contiguous()), d + pad
+
+    def split(t):
+        t32 = t.float()
+        hi = t32.to(torch.bfloat16)
+        return padded(hi), padded((t32 - hi.float()).to(torch.bfloat16))
+
+    xh, xl = split(x)
+    yh, yl = (xh, xl) if y is x else split(y)
+    a = torch.cat([xh, xl, xh], dim=1).contiguous()
+    b = torch.cat([yh, yh, yl], dim=1).contiguous()
     return a, b, 3 * (d + pad)
 
 
