@@ -25,7 +25,8 @@
 extern "C" {
 #endif
 
-#define DSOFT_VERSION 250 /* 0.2.5: retrieval ranks (dsoft_retrieval_ranks); 0.2.4: weighted plans accept the fused
+#define DSOFT_VERSION 260 /* 0.2.6: SigLIP loss (DSOFT_F_SIGLIP, dsoft_siglip_*); 0.2.5: retrieval ranks
+                             (dsoft_retrieval_ranks); 0.2.4: weighted plans accept the fused
                              backward (no DSOFT_F_GMAT); 0.2.3: weighted
                              CE branch at world > 1 (phases 5 / 6, dsoft_plan_lse_rows, dsoft_plan_wsigma_info) */
 
@@ -54,6 +55,10 @@ extern "C" {
                                   row stds of all B rows - see dsoft_plan_wsigma_info.  Such plans never share
                                   soft tiles (DSOFT_SYM_W). */
 #define DSOFT_F_WSYM 64u        /* weight_text_symmetry: modulate the text direction too (loss.py:449-463) */
+#define DSOFT_F_SIGLIP 128u     /* SigLIP sigmoid loss (open_clip SigLipLoss) instead of the DINO-Soft terms: only
+                                  with Dp = Dd = 0 and no other flag (else DSOFT_EINVAL); runs through
+                                  dsoft_siglip_forward / dsoft_siglip_backward, which dsoft_forward /
+                                  dsoft_backward refuse.  dsoft_pack and the gathered layout are unchanged. */
 
 /* element types accepted by dsoft_pack */
 #define DSOFT_DT_F32 0
@@ -207,6 +212,31 @@ size_t dsoft_retrieval_scratch_bytes(int32_t n_img, int32_t n_txt);
 int dsoft_retrieval_ranks(const void* img_dev, const void* txt_dev, int32_t k, int32_t n_img, int32_t n_txt,
                           const int32_t* text_image_dev, int32_t* rank_img_dev, int32_t* rank_txt_dev,
                           void* scratch_dev, void* stream);
+
+/* SigLIP sigmoid loss of a DSOFT_F_SIGLIP plan (open_clip SigLipLoss).  z_ij = s <I_i, T_j> + beta over the bf16
+ * image | text columns of `gathered` (fp32 accumulation, s and beta applied in fp32), l_ij = +1 for j == i (global
+ * index), -1 otherwise:
+ *   loss = (1/b) sum_{i in this rank's rows} sum_{j < B} softplus(-l_ij z_ij)
+ * dsoft_siglip_forward: logit_scale_dev = s (already exp'd), logit_bias_dev = beta (NULL: 0), both one fp32 on the
+ *   device.  loss_dev: one fp32.  g_dev: NULL for a forward without gradient, else dsoft_siglip_g_bytes(plan) bytes
+ *   (16-byte aligned) that receive this rank's fp16 logit-gradient matrix G 2^14 (G = d loss / d z times b, blocked
+ *   layout), 2 bytes per element of the [b x B] row block.  The forward also leaves the sums of G x and G in `state`.
+ *   Scratch: dsoft_plan_forward_scratch_bytes.
+ * dsoft_siglip_backward: the same gathered / state and g_dev of the forward; gout_dev = the upstream gradient of the
+ *   loss (one fp32).  Outputs fp32, 16-byte aligned: d_image [b][D] and d_text [b][D] = the derivative of the SUM of
+ *   all ranks' losses with respect to this rank's rows (what an all-gather with gradient delivers), d_scale [1] and
+ *   d_bias [1] (NULL: skipped) = the derivative of this rank's own loss; this assumes the same s, beta and upstream
+ *   gradient on every rank.  Scratch: dsoft_plan_scratch_bytes (at world > 1 it holds the text rows' G, another
+ *   2 b B bytes, computed here).  No statistic crosses ranks: the backward needs no collective.
+ * Profile slots: 0 = forward tile kernel, 3 / 4 = the gradient GEMMs (image / text rows), 7 = the text rows' G kernel
+ * (world > 1).  Both calls are asynchronous on `stream`, make no host synchronisation and can be captured in a graph. */
+size_t dsoft_siglip_g_bytes(const dsoft_plan_t* plan);
+int dsoft_siglip_forward(const dsoft_plan_t* plan, const void* gathered_dev, const float* logit_scale_dev,
+                         const float* logit_bias_dev, void* state_dev, void* scratch_dev, void* g_dev, float* loss_dev,
+                         void* stream);
+int dsoft_siglip_backward(const dsoft_plan_t* plan, const void* gathered_dev, const void* state_dev, void* scratch_dev,
+                          const void* g_dev, const float* gout_dev, float* d_image_dev, float* d_text_dev,
+                          float* d_scale_dev, float* d_bias_dev, void* stream);
 
 /* Column (in elements) of the DINO block inside a packed row: where dsoft_gather_rows must write when the caller
  * fills the DINO columns of `gathered` itself (dsoft_pack with dino_dev == NULL). */

@@ -11,6 +11,8 @@ Import as ``dinosoft_b200`` (see the shim at the repo root).  Contents:
     graphed.py   CUDA-graph capture of the loss forward + backward (launch-bound small batches)
     pair_stats.py  CLIP-blind pair statistics on the Gram-tile kernel (helpers.py:221-285, SURVEY 8f-4)
     retrieval.py  retrieval ranks and R@K (open_clip get_clip_metrics) on the Gram-tile kernel, no N x N logits
+    siglip.py    SigLipLoss drop-in (open_clip SigLipLoss): sigmoid loss and its logit gradient in one tile pass,
+                 backward = the two gradient GEMMs, no B x B logit matrix
     _cabi.py     ctypes binding of libdsoft.so (include/dsoft.h)
     _build.py    nvcc recipe for csrc/ (sm_100a only)
     csrc/        hand-written tcgen05 / TMEM / TMA kernels + the C ABI
@@ -22,6 +24,7 @@ from .cyclip import CyCLIPLoss
 from .graphed import make_graphed
 from .pair_stats import pair_stats
 from .retrieval import clip_metrics, retrieval_ranks
+from .siglip import SigLipLoss
 from .loss import (
     ClipLossWithDINOEnhancements,
     CudaBackend,
@@ -48,5 +51,6 @@ __all__ = [
     "retrieval_ranks",
     "clip_metrics",
     "CyCLIPLoss",
+    "SigLipLoss",
     "make_graphed",
 ]

@@ -95,6 +95,10 @@ struct dsoft_plan {
   SplitPlan g_clip, g_stu, g_txt;  // K splits of the gradient GEMMs (tps = K steps per split)
   SplitPlan g_clip_t;              // world == 1: dT = G^T . I, K runs over G's rows
   int clip_tr;                     // world == 1 two-phase: one CLIP logit-gradient matrix serves both directions
+  // DSOFT_F_SIGLIP: SigLIP sigmoid loss on the image | text columns of `gathered` (its own state / scratch layout)
+  int siglip;
+  size_t sg_part, sg_blk;  // forward scratch: row partials [3][npart][b], per-block sums [3][blocks]
+  size_t sg_Gt;            // backward scratch, world > 1: the text rows' fp16 G [bpad][pitch_c]
 };
 
 static int ceil_div(int a, int b) { return (a + b - 1) / b; }
@@ -189,6 +193,8 @@ extern "C" int dsoft_plan_create(const dsoft_shape_t* sh, dsoft_plan_t** out) {
     if (sh->Dd == 0) return fail(DSOFT_EINVAL, "DSOFT_F_WEIGHTED needs Dd > 0");
     if (!(sh->c_clip > 0.f)) return fail(DSOFT_EINVAL, "c_clip must be > 0");
   }
+  if ((sh->flags & DSOFT_F_SIGLIP) && (sh->flags != DSOFT_F_SIGLIP || sh->Dp != 0 || sh->Dd != 0))
+    return fail(DSOFT_EINVAL, "DSOFT_F_SIGLIP takes no other flag and needs Dp = Dd = 0");
   if (static_cast<long>(sh->b) * sh->world > (1L << 30)) return fail(DSOFT_EINVAL, "batch too large");
   if (sh->D > 2048 || sh->Dp > 2048) return fail(DSOFT_EINVAL, "feature dims above 2048 are not supported");
 
@@ -291,6 +297,33 @@ extern "C" int dsoft_plan_create(const dsoft_shape_t* sh, dsoft_plan_t** out) {
   // ---- state (floats)
   size_t o = 0;
   auto take = [&](size_t n) { size_t r = o; o = align_up(o + n, 64); return r; };
+  if (sh->flags & DSOFT_F_SIGLIP) {
+    // state: the scalar block (s, beta, the forward's sums of G x and G).  Forward scratch: the row partials.
+    // Backward scratch: the gradient GEMMs' split partials, the fp16 text | image operands and, at world > 1, the
+    // text rows' G.  The image rows' G is the caller's (dsoft_siglip_g_bytes).
+    const int pairs = ceil_div(rbs, 2);
+    p->siglip = 1;
+    p->clip_tr = sh->world == 1;
+    p->g_clip = choose_gy_split(pairs * ceil_div(sh->D, GY_N), p->pitch_c / 64, sms, sh->b, sh->D);
+    p->g_clip_t = choose_gy_split(pairs * ceil_div(sh->D, GY_N), rbs * 2, sms, sh->b, sh->D);
+    p->st_scal = take(SC_COUNT);
+    p->st_total = o;
+    o = 0;
+    p->sg_part = take(static_cast<size_t>(3) * 2 * p->f_clip.nsplit * sh->b);
+    p->sg_blk = take(static_cast<size_t>(3) * ceil_div(sh->b, 128));
+    p->sc_fwd_total = o;
+    const size_t ns_t = p->clip_tr ? p->g_clip_t.nsplit : p->g_clip.nsplit;
+    p->sc_acc1 = take(static_cast<size_t>(p->g_clip.nsplit) * sh->b * sh->D);
+    p->sc_acc2 = take(ns_t * sh->b * sh->D);
+    p->v_offT = 0;
+    p->v_offI = sh->D;
+    p->v_row = 2 * sh->D;
+    p->sc_v16 = take(static_cast<size_t>(p->B) * p->v_row / 2 + 1);
+    p->sg_Gt = take(p->clip_tr ? 0 : static_cast<size_t>(rbs) * BM * p->pitch_c / 2);
+    p->sc_total = o;
+    *out = p;
+    return 0;
+  }
   p->st_scal = take(SC_COUNT);
   p->st_rinv_t = take(p->Bcol);
   p->st_rinv_z = take(p->Bcol);
@@ -363,6 +396,7 @@ extern "C" size_t dsoft_plan_forward_scratch_bytes(const dsoft_plan_t* p) { retu
 
 extern "C" double dsoft_plan_algorithmic_flops(const dsoft_plan_t* p) {
   if (!p) return 0.0;
+  if (p->siglip) return 2.0 * p->sh.b * p->B * (3.0 * p->sh.D);  // I . T^T, G . T, G^T . I
   // SURVEY.md 8(d): F_alg = 2 B^2 (3D + 2Dp + Dd [+ 2D]) for the whole job; this rank's share is 1/W.
   const double b = p->sh.b, cols_c = p->B, cols_s = p->sym_w ? p->B : p->s_ncols;
   double f = 2.0 * b * cols_c * (3.0 * p->sh.D);
@@ -377,6 +411,11 @@ extern "C" int dsoft_plan_kernel_flops(const dsoft_plan_t* p, double* algorithmi
   const double b = p->sh.b, Bc = p->B, Bs = p->sym_w ? p->B : p->s_ncols, D = p->sh.D, Dz = p->Dz, Dd = p->sh.Dd;
   const double sw = p->sym_w ? 0.5 : 1.0;  // symmetric ownership across ranks: half of the soft tiles per rank
   for (int k = 0; k < n; ++k) algorithmic[k] = executed[k] = 0.0;
+  if (p->siglip) {  // [0] forward tile kernel, [3] / [4] gradient GEMMs, [7] world > 1: the text rows' G kernel
+    algorithmic[0] = executed[0] = algorithmic[3] = executed[3] = algorithmic[4] = executed[4] = 2.0 * b * Bc * D;
+    if (n > 7 && !p->clip_tr) executed[7] = 2.0 * b * Bc * D;
+    return 0;
+  }
   // forward CLIP: the two directions are exact transposes -> one algorithmic product, two executed
   algorithmic[0] = algorithmic[1] = b * Bc * D;
   executed[0] = executed[1] = 2.0 * b * Bc * D;
@@ -413,11 +452,13 @@ extern "C" int dsoft_plan_kernel_flops(const dsoft_plan_t* p, double* algorithmi
 
 extern "C" int dsoft_plan_launches_forward(const dsoft_plan_t* p) {
   if (!p) return 0;
+  if (p->siglip) return 3;  // scalars, tile kernel, finalize
   return 1 /*pack*/ + 1 /*scalars*/ + 1 /*norms*/ + 2 /*clip x2*/ + (p->have_soft ? 1 : 0) + (p->fwd_sym ? 1 : 0) +
          1 /*finalize*/ + (p->weighted ? (p->wsym ? 2 : 1) * 7 + 1 : 0);
 }
 extern "C" int dsoft_plan_launches_backward(const dsoft_plan_t* p) {
   if (!p) return 0;
+  if (p->siglip) return p->clip_tr ? 4 : 5;  // fp16 operands, [text rows' G,] two gradient GEMMs, finalize
   if (p->gmat)
     return 3 /*lse stats, relayout, fp16 operands*/ + (p->weighted && !p->clip_tr ? 1 : 0) /*weighted relayout*/ +
            (p->clip_tr ? 1 : 2) /*clip G*/ + 2 /*clip GEMMs*/ +
@@ -2346,6 +2387,7 @@ static int forward_impl(const dsoft_plan_t* p, const void* gathered, const float
                         float* losses, float* dbg, void* stream, int phase) {
   if (!p || !gathered || !logit_scale || !lambdas || !state || !scratch || !lse_local || !losses)
     return fail(DSOFT_EINVAL, "null argument");
+  if (p->siglip) return fail(DSOFT_EINVAL, "a DSOFT_F_SIGLIP plan runs through dsoft_siglip_forward");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   float* S = static_cast<float*>(state);
   float* X = static_cast<float*>(scratch);
@@ -2846,6 +2888,7 @@ static int backward_impl(const dsoft_plan_t* p, const void* gathered, const void
                          float* d_text, float* d_student, float* d_scale, void* stream, int phase) {
   if (!p || !gathered || !state || !scratch || !lse_all || !gout || !lambdas || !d_image || !d_text || !d_scale)
     return fail(DSOFT_EINVAL, "null argument");
+  if (p->siglip) return fail(DSOFT_EINVAL, "a DSOFT_F_SIGLIP plan runs through dsoft_siglip_backward");
   if (p->have_proj && !d_student) return fail(DSOFT_EINVAL, "d_student is null but the plan has Dp > 0");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   // state is logically const for the caller; the relayouted LSE columns live in it
@@ -3104,6 +3147,210 @@ static int backward_impl(const dsoft_plan_t* p, const void* gathered, const void
       finalize_bwd_kernel<4><<<dim3(std::min(b, p->num_sms * 16)), 128, 0, st>>>(fa);
     }
   }
+  CUDA_TRY(cudaGetLastError());
+  return 0;
+}
+
+// ------------------------------------------------------------------------------------------------
+// SigLIP sigmoid loss (open_clip SigLipLoss) on the Gram-tile kernels: dsoft_fwd_kernel<MODE_SIGLIP> computes every
+// pair's loss term and logit gradient from the pair's own logit, so the forward writes the fp16 G tile as it goes and
+// the backward is the two gradient GEMMs.  Rank r owns image rows [r b, (r+1) b) against all B captions; at world > 1
+// the text rows' G (T_local . I_all^T, same pairs transposed) is computed by a second launch in the backward, so the
+// forward-to-backward interval holds one [b x B] G, and a forward without gradient needs none.
+// ------------------------------------------------------------------------------------------------
+__global__ void siglip_prep_kernel(const float* __restrict__ logit_scale, const float* __restrict__ logit_bias,
+                                   float* __restrict__ scal) {
+  if (threadIdx.x != 0 || blockIdx.x != 0) return;
+  scal[SC_SCALE] = *logit_scale;
+  scal[SC_SIG_BIAS] = logit_bias ? *logit_bias : 0.f;
+  scal[SC_SIG_GX] = scal[SC_SIG_G] = 0.f;
+  scal[SC_TICKET_S] = 0.f;  // all-zero bits == integer 0
+}
+
+struct SgFinFwdArgs {
+  int b, npart;
+  const float* part;  // [3][npart][b]: loss, G x, G
+  float* blk;         // [3][gridDim.x]
+  float* scal;
+  float* loss;
+  int* ticket;
+};
+
+// loss = sum / b; the sums of G x and G stay in the state for the backward.  Rows -> per-block fp32 sums in a fixed
+// order, then the last block adds the blocks in fp64 (deterministic, as finalize_fwd_kernel).
+__global__ void __launch_bounds__(128) siglip_finalize_fwd_kernel(SgFinFwdArgs a) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  float r[3] = {0.f, 0.f, 0.f};
+  if (i < a.b)
+    for (int k = 0; k < 3; ++k)
+      for (int s = 0; s < a.npart; ++s) r[k] += a.part[(static_cast<size_t>(k) * a.npart + s) * a.b + i];
+  __shared__ float shp[3][4];
+#pragma unroll
+  for (int k = 0; k < 3; ++k) {
+    float v = r[k];
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+    if ((threadIdx.x & 31) == 0) shp[k][threadIdx.x >> 5] = v;
+  }
+  __syncthreads();
+  if (threadIdx.x < 3)
+    a.blk[threadIdx.x * gridDim.x + blockIdx.x] =
+        (shp[threadIdx.x][0] + shp[threadIdx.x][1]) + (shp[threadIdx.x][2] + shp[threadIdx.x][3]);
+  if (last_block_done(a.ticket)) {
+    __shared__ double sums[3];
+    block_reduce_rows(a.blk, gridDim.x, 3, sums);
+    if (threadIdx.x == 0) {
+      a.loss[0] = static_cast<float>(sums[0] / a.b);
+      a.scal[SC_SIG_GX] = static_cast<float>(sums[1]);
+      a.scal[SC_SIG_G] = static_cast<float>(sums[2]);
+    }
+  }
+}
+
+struct SgFinBwdArgs {
+  int b, D, ns1, ns2;
+  const float* acc1;  // [ns1][b][D]  sum_j (G 2^k)_ij T_j   (image rows)
+  const float* acc2;  // [ns2][b][D]  sum_i (G 2^k)_ij I_i   (text rows)
+  const float* scal;
+  const float* gout;
+  float* d_image;
+  float* d_text;
+  float* d_scale;
+  float* d_bias;
+};
+
+// d image / d text = gout s / (b 2^k) x the summed split partials; d s = gout / b sum G x, d beta = gout / b sum G
+__global__ void __launch_bounds__(256) siglip_finalize_bwd_kernel(SgFinBwdArgs a) {
+  const float g = a.gout[0] / static_cast<float>(a.b);
+  const float coef = g * a.scal[SC_SCALE] * (1.f / static_cast<float>(1 << SIG_GK));
+  const int q = a.D / 4;
+  const size_t n = static_cast<size_t>(a.b) * q;
+  for (size_t idx = blockIdx.x * static_cast<size_t>(blockDim.x) + threadIdx.x; idx < n;
+       idx += static_cast<size_t>(gridDim.x) * blockDim.x) {
+    const int i = static_cast<int>(idx / q);
+    const int f = static_cast<int>(idx % q) * 4;
+    float4 u = sum_splits4(a.acc1, a.ns1, a.b, a.D, i, f);
+    *reinterpret_cast<float4*>(a.d_image + static_cast<size_t>(i) * a.D + f) =
+        make_float4(u.x * coef, u.y * coef, u.z * coef, u.w * coef);
+    u = sum_splits4(a.acc2, a.ns2, a.b, a.D, i, f);
+    *reinterpret_cast<float4*>(a.d_text + static_cast<size_t>(i) * a.D + f) =
+        make_float4(u.x * coef, u.y * coef, u.z * coef, u.w * coef);
+  }
+  if (blockIdx.x == 0 && threadIdx.x == 0) {
+    a.d_scale[0] = g * a.scal[SC_SIG_GX];
+    if (a.d_bias) a.d_bias[0] = g * a.scal[SC_SIG_G];
+  }
+}
+
+extern "C" size_t dsoft_siglip_g_bytes(const dsoft_plan_t* p) {
+  if (!p || !p->siglip) return 0;
+  return static_cast<size_t>(ceil_div(p->sh.b, BM)) * BM * p->pitch_c * 2;
+}
+
+extern "C" int dsoft_siglip_forward(const dsoft_plan_t* p, const void* gathered, const float* logit_scale,
+                                    const float* logit_bias, void* state, void* scratch, void* g, float* loss,
+                                    void* stream) {
+  if (!p || !gathered || !logit_scale || !state || !scratch || !loss) return fail(DSOFT_EINVAL, "null argument");
+  if (!p->siglip) return fail(DSOFT_EINVAL, "dsoft_siglip_forward needs a DSOFT_F_SIGLIP plan");
+  if (reinterpret_cast<uintptr_t>(g) % 16) return fail(DSOFT_EINVAL, "g must be 16-byte aligned");
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  float* S = static_cast<float*>(state);
+  float* X = static_cast<float*>(scratch);
+  const int b = p->sh.b;
+  TileMaps tm;
+  int rc = make_maps(p, gathered, &tm, 64);
+  if (rc) return rc;
+  siglip_prep_kernel<<<1, 32, 0, st>>>(logit_scale, logit_bias, S + p->st_scal);
+  CUDA_TRY(cudaGetLastError());
+  FwdParams P;
+  fill_clip_fwd(p, P, 0, 1, S + p->st_scal, X + p->sg_part, nullptr);
+  P.gout[0] = static_cast<__half*>(g);
+  P.g_pitch = p->pitch_c;
+  if (g && (rc = make_gstore_map(p, &tm.g[0], static_cast<const __half*>(g), p->pitch_c))) return rc;
+  tm.g[1] = tm.g[0];
+  if ((rc = set_smem(dsoft_fwd_kernel<MODE_SIGLIP, 2>, FWD_SMEM_BYTES))) return rc;
+  {
+    ProfScope ps(PK_FWD_CLIP_IT, st);
+    if ((rc = launch_fwd_pair(dsoft_fwd_kernel<MODE_SIGLIP, 2>, ceil_div(b, BM), p->f_clip.nsplit, st, tm, P)))
+      return rc;
+  }
+  SgFinFwdArgs fa;
+  fa.b = b;
+  fa.npart = P.npart;
+  fa.part = X + p->sg_part;
+  fa.blk = X + p->sg_blk;
+  fa.scal = S + p->st_scal;
+  fa.loss = loss;
+  fa.ticket = reinterpret_cast<int*>(S + p->st_scal + SC_TICKET_S);
+  siglip_finalize_fwd_kernel<<<ceil_div(b, 128), 128, 0, st>>>(fa);
+  CUDA_TRY(cudaGetLastError());
+  return 0;
+}
+
+extern "C" int dsoft_siglip_backward(const dsoft_plan_t* p, const void* gathered, const void* state, void* scratch,
+                                     const void* g, const float* gout, float* d_image, float* d_text, float* d_scale,
+                                     float* d_bias, void* stream) {
+  if (!p || !gathered || !state || !scratch || !g || !gout || !d_image || !d_text || !d_scale)
+    return fail(DSOFT_EINVAL, "null argument");
+  if (!p->siglip) return fail(DSOFT_EINVAL, "dsoft_siglip_backward needs a DSOFT_F_SIGLIP plan");
+  if (reinterpret_cast<uintptr_t>(g) % 16 || reinterpret_cast<uintptr_t>(d_image) % 16 ||
+      reinterpret_cast<uintptr_t>(d_text) % 16)
+    return fail(DSOFT_EINVAL, "g, d_image and d_text must be 16-byte aligned");
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  float* S = const_cast<float*>(static_cast<const float*>(state));
+  float* X = static_cast<float*>(scratch);
+  const int b = p->sh.b;
+  const __half* G = static_cast<const __half*>(g);
+  __half* v16 = reinterpret_cast<__half*>(X + p->sc_v16);
+  TileMaps tm;
+  int rc = make_maps(p, gathered, &tm, 64);
+  if (rc) return rc;
+  make_v16_kernel<<<ceil_div(p->B, 8), 256, 0, st>>>(
+      static_cast<const __nv_bfloat16*>(gathered), p->row_elems, p->B, p->sh.D, p->Dz, p->offI, p->offT, p->offZ, 0, 0,
+      nullptr, nullptr, v16, p->v_row, p->v_offT, p->v_offI, 0, 0);
+  CUDA_TRY(cudaGetLastError());
+  if ((rc = set_smem(dsoft_gy_kernel<false>, GY_SMEM_BYTES))) return rc;
+  if ((rc = set_smem(dsoft_gy_kernel<true>, GY_SMEM_BYTES))) return rc;
+  const __half* Gt = G;  // world == 1: the text rows' G is the transpose of the image rows' one
+  if (!p->clip_tr) {
+    __half* Gw = reinterpret_cast<__half*>(X + p->sg_Gt);
+    FwdParams P;
+    fill_clip_fwd(p, P, 1, 0, S + p->st_scal, nullptr, nullptr);
+    P.gout[0] = Gw;
+    P.g_pitch = p->pitch_c;
+    if ((rc = make_gstore_map(p, &tm.g[0], Gw, p->pitch_c))) return rc;
+    tm.g[1] = tm.g[0];
+    if ((rc = set_smem(dsoft_fwd_kernel<MODE_SIGLIP, 2>, FWD_SMEM_BYTES))) return rc;
+    ProfScope ps(PK_BWD_GCLIP, st);
+    if ((rc = launch_fwd_pair(dsoft_fwd_kernel<MODE_SIGLIP, 2>, ceil_div(b, BM), p->f_clip.nsplit, st, tm, P)))
+      return rc;
+    Gt = Gw;
+  }
+  {
+    ProfScope ps(PK_BWD_CLIP_I, st);
+    if ((rc = launch_gy(p, G, p->pitch_c, v16, p->v_offT, p->sh.D, 0, p->g_clip, X + p->sc_acc1, st))) return rc;
+  }
+  {
+    ProfScope ps(PK_BWD_CLIP_T, st);
+    if ((rc = launch_gy(p, Gt, p->pitch_c, v16, p->v_offI, p->sh.D, 0, p->clip_tr ? p->g_clip_t : p->g_clip,
+                        X + p->sc_acc2, st, p->clip_tr)))
+      return rc;
+  }
+  SgFinBwdArgs fa;
+  fa.b = b;
+  fa.D = p->sh.D;
+  fa.ns1 = p->g_clip.nsplit;
+  fa.ns2 = p->clip_tr ? p->g_clip_t.nsplit : p->g_clip.nsplit;
+  fa.acc1 = X + p->sc_acc1;
+  fa.acc2 = X + p->sc_acc2;
+  fa.scal = S + p->st_scal;
+  fa.gout = gout;
+  fa.d_image = d_image;
+  fa.d_text = d_text;
+  fa.d_scale = d_scale;
+  fa.d_bias = d_bias;
+  const size_t work = static_cast<size_t>(b) * (p->sh.D / 4);
+  siglip_finalize_bwd_kernel<<<static_cast<int>(std::min<size_t>((work + 255) / 256, p->num_sms * 8)), 256, 0, st>>>(fa);
   CUDA_TRY(cudaGetLastError());
   return 0;
 }

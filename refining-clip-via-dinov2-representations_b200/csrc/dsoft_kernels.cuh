@@ -62,6 +62,9 @@ constexpr int MODE_CLIP_SYM = 10; // forward CLIP statistics of BOTH directions 
                                   // direction is the transpose: loss.py:267/273 recomputes it)
 constexpr int MODE_RANKS = 14;    // retrieval ranks (open_clip get_clip_metrics): per image and per caption, the number
                                   // of non-positive scores of I . T^T above its positive, over the full rectangle
+constexpr int MODE_SIGLIP = 15;   // SigLIP sigmoid loss (open_clip SigLipLoss): per pair loss and logit gradient from the
+                                  // pair's own logit; writes the fp16 G tile (scaled by 2^SIG_GK) and row partials
+constexpr int SIG_GK = 14;        // SigLIP G is stored as G * 2^14: |G| < 1, and sigma down to 2^-28 stays normal fp16
 
 // scalar block computed on device by prep_scalars_kernel (no host sync on logit_scale)
 enum {
@@ -82,6 +85,10 @@ enum {
   SC_FAST_CLIP = 15,// 1.0: all CLIP log-sum-exps lie within 200 log2 units -> one exponential per pair
   SC_WBETA = 16,    // [2] beta = rho * median(row std) / c_clip of the weighted CE, image / text direction
   SC_WBETA2 = 18,   // [2] beta * log2(e)
+  SC_SIG_BIAS = 20, // SigLIP: logit bias beta (0 without one)
+  SC_SIG_GX = 21,   // SigLIP: sum over this rank's pairs of G x (d logit_scale, before gout / b), by the forward
+  SC_SIG_G = 22,    // SigLIP: sum of G (d logit_bias, before gout / b)
+  SC_TICKET_S = 23, // (int) SigLIP finalize tickets (forward, backward)
   SC_COUNT = 32
 };
 
@@ -375,6 +382,41 @@ __device__ __forceinline__ void store_g32(__half* dst, const float (&g)[32]) {
     st_cs_v8(dst + 16 * i, w);
   }
 }
+// SigLIP pair terms (MODE_SIGLIP).  z = s x + beta, l = +1 for the positive pair, -1 otherwise:
+//   loss = softplus(-l z) = max(-l z, 0) + log1p(e),  e = 2^(-|z| log2 e)  (the one MUFU op per pair)
+//   G = d loss / d z = -l sigma(-l z),  sigma(t) = r (t >= 0) or e r (t < 0),  r = 1 / (1 + e)
+// r and log1p(e) run on the FMA pipe: lg2.approx of 1 + e loses ~1e-3 of the typical negative's term (e ~ 5e-5 at
+// s = 10, beta = -10) to the rounding of 1 + e, and the CLIP logit-gradient kernel was MUFU-bound at one ex2 per
+// pair.  r: quadratic on [1, 2] (1e-2) + two Newton steps, 1.8e-7; log1p(e) = e P7(e), 3.2e-7 relative on [0, 1].
+__device__ __forceinline__ float2 sig_rcp1p(float2 e) {
+  const float2 y = pk_add(e, pk1(1.f));
+  float2 r = pk_fma(pk_fma(y, pk1(0.32323232f), pk1(-1.45454545f)), y, pk1(2.12121212f));
+#pragma unroll
+  for (int k = 0; k < 2; ++k) r = pk_fma(r, pk_fma(pk(-y.x, -y.y), r, pk1(1.f)), r);
+  return r;
+}
+__device__ __forceinline__ float2 sig_log1p(float2 e) {
+  float2 q = pk_fma(e, pk1(-0.00837115291506052f), pk1(0.04349390044808388f));
+  q = pk_fma(q, e, pk1(-0.1068500280380249f));
+  q = pk_fma(q, e, pk1(0.1768747717142105f));
+  q = pk_fma(q, e, pk1(-0.24474774301052094f));
+  q = pk_fma(q, e, pk1(0.3327192962169647f));
+  q = pk_fma(q, e, pk1(-0.49997174739837646f));
+  q = pk_fma(q, e, pk1(0.9999997615814209f));
+  return pk_mul(q, e);
+}
+// two pairs at once; pos.x / pos.y: the pair is a positive.  Returns the loss terms, G in g.
+__device__ __forceinline__ float2 siglip_pair2(float2 z, bool pos_x, bool pos_y, float2& g) {
+  const float L2E = 1.4426950408889634f;
+  const float2 e = pk_exp2(pk_mul(pk(fabsf(z.x), fabsf(z.y)), pk1(-L2E)));
+  const float2 r = sig_rcp1p(e);
+  const float2 er = pk_mul(e, r);
+  const float tx = pos_x ? -z.x : z.x, ty = pos_y ? -z.y : z.y;  // -l z
+  const float sx = tx >= 0.f ? r.x : er.x, sy = ty >= 0.f ? r.y : er.y;
+  g = pk(pos_x ? -sx : sx, pos_y ? -sy : sy);
+  return pk_add(pk(fmaxf(tx, 0.f), fmaxf(ty, 0.f)), sig_log1p(e));
+}
+
 // ================================================================================================
 // Forward: per-row soft-max statistics
 // ================================================================================================
@@ -427,10 +469,11 @@ dsoft_fwd_kernel(const __grid_constant__ TileMaps maps, const __grid_constant__ 
   const int stage_bytes = (resident ? 0 : TILE_BYTES) + brows * 128;
   // soft modes: 6 stages of 32 KiB (logit-gradient mode: 5); the 32 KiB behind them hold the staged per-column
   // vectors.  Logit-gradient modes keep 32 KiB (at 192 KiB; soft: at 160 KiB) for the G staging strips.
-  constexpr bool kGMode = (MODE == MODE_CLIP_G || MODE == MODE_SOFT_G || MODE == MODE_WCE_G);
+  constexpr bool kClipG = (MODE == MODE_CLIP_G || MODE == MODE_SIGLIP);  // one product, G staging behind the ring
+  constexpr bool kGMode = (kClipG || MODE == MODE_SOFT_G || MODE == MODE_WCE_G);
   constexpr bool kSoftG = (MODE == MODE_SOFT_G || MODE == MODE_WCE_G);
   const int nstages = kSoftG ? 5 : (kSoftMode ? 6 :
-                      min(MODE == MODE_CLIP_G ? (resident ? 4 : 6) : 8, (resident ? 6 : 14) * TILE_BYTES / stage_bytes));
+                      min(kClipG ? (resident ? 4 : 6) : 8, (resident ? 6 : 14) * TILE_BYTES / stage_bytes));
   // G staging: one 4 KiB strip (32 rows x 64 columns fp16, 128-byte swizzle) per epilogue warp.  A strip is written
   // with conflict-free 16-byte shared stores and leaves through ONE TMA tensor store; per-thread 32-byte global
   // stores (32 different lines per warp instruction) kept the L1TEX pipe at 78 % and the tensor pipe at 62 %.
@@ -1179,6 +1222,88 @@ dsoft_fwd_kernel(const __grid_constant__ TileMaps maps, const __grid_constant__ 
       }
       if (lane == 0) bulk_wait_group<0>();  // the stores have landed before the CTA may exit
       if (li < P.b) P.ds_part[sp * P.b + li] = dsacc + (dsacc2.x + dsacc2.y);
+    } else if constexpr (MODE == MODE_SIGLIP) {
+      // SigLIP (siglip_pair2): z = s x + beta per pair, positive where global row == global column.  The G tile
+      // (G 2^SIG_GK, fp16) goes to gout[0] unless that is null (no gradient wanted); the row partials sum loss, G x
+      // and G into part[3][npart][b] unless part is null (the text rows' launch at world > 1 only writes G).
+      const float2 s22 = pk1(P.scal[SC_SCALE]), b22 = pk1(P.scal[SC_SIG_BIAS]);
+      const bool want_g = P.gout[0] != nullptr;
+      const bool real_block = rb * BM < P.b;  // the odd pair member past the last row block owns no G rows
+      const bool live_row = li < P.b;         // rows past b are K entries of the transposed GEMM: keep them zero
+      float2 lacc = pk1(0.f), gxacc = pk1(0.f), gacc = pk1(0.f);
+      int it = 0;
+      for (int t = t0; t < t1; ++t, ++it) {
+        const int slot = it % nslots;
+        const uint32_t use = static_cast<uint32_t>(it / nslots);
+        mbar_wait(smem_u32(&s_full[slot]), use & 1);
+        tc_fence_after();
+        uint32_t rA[32], rB[32];
+        tmem_ld32_nowait(lane_addr + slot * 256 + half * 128, rA);
+#pragma unroll
+        for (int c = 0; c < 4; ++c) {
+          const int jrel0 = t * 256 + half * 128 + c * 32;
+          const int gj0 = P.col0 + jrel0;
+          uint32_t(&rcur)[32] = (c & 1) ? rB : rA;
+          uint32_t(&rnxt)[32] = (c & 1) ? rA : rB;
+          tmem_ld_wait(rcur);
+          if (c < 3) {
+            tmem_ld32_nowait(lane_addr + slot * 256 + half * 128 + (c + 1) * 32, rnxt);
+          } else {
+            tc_fence_before();
+            release_slot(slot);
+          }
+#pragma unroll
+          for (int e = 0; e < 32; ++e) v[e] = __uint_as_float(rcur[e]);
+          // positives, ragged columns, rows past b: only in the chunks that can hold them (warp-uniform)
+          const bool need_mask = (gw0 < gj0 + 32 && gj0 < gw0 + 32) || jrel0 + 32 > P.ncols || !real_block ||
+                                 rb * BM + q * 32 + 32 > P.b;
+          float g[32];
+          if (!need_mask) {
+#pragma unroll
+            for (int e = 0; e < 32; e += 2) {
+              const float2 vv = pk(v[e], v[e + 1]);
+              float2 gg;
+              lacc = pk_add(lacc, siglip_pair2(pk_fma(vv, s22, b22), false, false, gg));
+              gxacc = pk_fma(gg, vv, gxacc);
+              gacc = pk_add(gacc, gg);
+              g[e] = gg.x;
+              g[e + 1] = gg.y;
+            }
+          } else {
+#pragma unroll
+            for (int e = 0; e < 32; e += 2) {
+              const bool ok0 = live_row && jrel0 + e < P.ncols, ok1 = live_row && jrel0 + e + 1 < P.ncols;
+              const float2 vv = pk(v[e], v[e + 1]);
+              float2 gg;
+              float2 ll = siglip_pair2(pk_fma(vv, s22, b22), gj0 + e == gi, gj0 + e + 1 == gi, gg);
+              gg = pk(ok0 ? gg.x : 0.f, ok1 ? gg.y : 0.f);
+              ll = pk(ok0 ? ll.x : 0.f, ok1 ? ll.y : 0.f);
+              lacc = pk_add(lacc, ll);
+              gxacc = pk_fma(gg, vv, gxacc);
+              gacc = pk_add(gacc, gg);
+              g[e] = gg.x;
+              g[e + 1] = gg.y;
+            }
+          }
+          if (want_g && real_block && jrel0 + 32 <= P.g_pitch) {  // warp-uniform (the pitch is a multiple of 64)
+            uint32_t w16[16];
+            const float sk = static_cast<float>(1 << SIG_GK);
+#pragma unroll
+            for (int k = 0; k < 16; ++k) w16[k] = pack_f16x2(g[2 * k] * sk, g[2 * k + 1] * sk);
+            if ((c & 1) == 0) stage_begin();
+            stage_put32(w16, c & 1);
+            if (c & 1)
+              stage_store(&maps.g[0], (rb * (P.g_pitch >> 6) + (jrel0 >> 6)) * BM + q * 32);
+          }
+        }
+      }
+      if (lane == 0) bulk_wait_group<0>();  // the stores have landed before the CTA may exit
+      if (P.part && live_row) {
+        const int st = P.npart * P.b;
+        P.part[0 * st + sp * P.b + li] = lacc.x + lacc.y;
+        P.part[1 * st + sp * P.b + li] = gxacc.x + gxacc.y;
+        P.part[2 * st + sp * P.b + li] = gacc.x + gacc.y;
+      }
     } else if constexpr (MODE == MODE_SOFT_G) {
       // G_aj = [(2^(p-ls_a) + 2^(p-ls_j)) - (2^(q-lt_a) + 2^(q-lt_j))] * mant(1/||y_j||), j != a, for the
       // student (-> gout[0]) and the text term (-> gout[1]) from ONE teacher tile.

@@ -801,11 +801,13 @@ class ClipLossWithDINOEnhancements(nn.Module):
         # the reference returns None when output_dict is False (loss.py:598-607) - preserved
 
 
-def install_into_open_clip(open_clip_module=None):
+def install_into_open_clip(open_clip_module=None, siglip=False):
     """Make the reference's ``create_loss`` (factory.py:566-576) build this class.
 
     ``open_clip.factory`` imports the class by name at import time (factory.py:25-34), so both module
-    attributes are patched; ``train.py`` needs no change."""
+    attributes are patched; ``train.py`` needs no change.  ``siglip=True`` also patches every binding of
+    ``SigLipLoss`` (the ``--siglip`` objective) with ``siglip.SigLipLoss``; off by default, so that existing callers
+    keep upstream's SigLIP loss."""
     import importlib
 
     loss_mod = importlib.import_module("open_clip.loss") if open_clip_module is None else open_clip_module.loss
@@ -826,6 +828,17 @@ def install_into_open_clip(open_clip_module=None):
         train_mod = sys.modules.get("open_clip_train.train")  # train.py:16 binds the name at import, :316 isinstance
         if train_mod is not None and hasattr(train_mod, "CyCLIPLoss"):
             train_mod.CyCLIPLoss = CyCLIPLoss
+    if siglip and hasattr(loss_mod, "SigLipLoss"):
+        from .siglip import SigLipLoss
+        import sys
+
+        if not hasattr(loss_mod, "_reference_SigLipLoss"):
+            loss_mod._reference_SigLipLoss = loss_mod.SigLipLoss
+        loss_mod.SigLipLoss = SigLipLoss
+        factory_mod.SigLipLoss = SigLipLoss
+        train_mod = sys.modules.get("open_clip_train.train")
+        if train_mod is not None and hasattr(train_mod, "SigLipLoss"):
+            train_mod.SigLipLoss = SigLipLoss
     return ClipLossWithDINOEnhancements
 
 
@@ -848,4 +861,13 @@ def uninstall_from_open_clip(open_clip_module=None):
         train_mod = sys.modules.get("open_clip_train.train")
         if train_mod is not None and hasattr(train_mod, "CyCLIPLoss"):
             train_mod.CyCLIPLoss = cyc
+    sig = getattr(loss_mod, "_reference_SigLipLoss", None)
+    if sig is not None:
+        import sys
+
+        loss_mod.SigLipLoss = sig
+        factory_mod.SigLipLoss = sig
+        train_mod = sys.modules.get("open_clip_train.train")
+        if train_mod is not None and hasattr(train_mod, "SigLipLoss"):
+            train_mod.SigLipLoss = sig
     return ref
