@@ -533,18 +533,20 @@ class _DinoSoftFn(torch.autograd.Function):
         g_head = (None, None, None, None)
         if ctx.fused_head:
             # head backward in the arithmetic autocast gives the reference (bf16 operands, fp32 accumulation), on
-            # cuBLAS: dZ -> (dW2, db2, dH) -> ReLU mask -> (dW1, db1, dX); dX joins d_image
+            # cuBLAS: dZ -> (dW2, db2, dH) -> ReLU mask -> (dW1, db1, dX); dX joins d_image.  The parameter
+            # gradients keep the fp32 accumulator (autocast would round them to bf16, up to 2^-8 relative)
             s = plan.shape
             r0 = s.rank * b
             x = gathered[r0:r0 + b, :D]  # image columns of this rank's rows (strided view)
             dz = d_student.to(torch.bfloat16)
+            f32 = torch.float32
             if w2b is None:
-                g_head = ((dz.t() @ x).float(), d_student.sum(0), None, None)
+                g_head = (torch.mm(dz.t(), x, out_dtype=f32), d_student.sum(0), None, None)
                 d_image += (dz @ w1b).float()
             else:
                 dh = torch.ops.aten.threshold_backward(dz @ w2b, hidden, 0.0)
-                g_head = ((dh.t() @ x).float(), dh.sum(0, dtype=torch.float32), (dz.t() @ hidden).float(),
-                          d_student.sum(0))
+                g_head = (torch.mm(dh.t(), x, out_dtype=f32), dh.sum(0, dtype=f32),
+                          torch.mm(dz.t(), hidden, out_dtype=f32), d_student.sum(0))
                 d_image += (dh @ w1b).float()
         return (d_image.to(idt), d_text.to(tdt), d_scale.reshape(sshape).to(sdt), g_student, None, None) + g_head
 

@@ -56,7 +56,8 @@ def chunked_reference(img, txt, dino, scale, head=None, blocks=(), lambdas=(1.0,
     blocks = iterable of (row0, nrows).  Returns loss terms (python floats), d_logit_scale and per block
     d_image / d_text / d_student (fp64 tensors).  student_values [B, Dp]: the (bf16-rounded) student operand the
     implementation under test really used; replaces the VALUE of the head output (gradients still flow through
-    the head), see oracle.loss_and_grads."""
+    the head), see oracle.loss_and_grads.  With student_values and no head the student is a leaf: d_image and
+    d_text are the loss side alone and d_student is the gradient the head's backward starts from."""
     dt = torch.float64
     dev = img.device
     lam_o, lam_s, lam_x = (float(v) for v in lambdas)
@@ -123,6 +124,8 @@ def chunked_reference(img, txt, dino, scale, head=None, blocks=(), lambdas=(1.0,
             if student_values is not None:
                 st = st + (student_values[R].to(dt) - st).detach()
             st.retain_grad()
+        elif student_values is not None:  # the student as a leaf of its own: d_image is the loss side alone
+            st = student_values[R].to(dt).clone().requires_grad_(True)
         else:
             st = im
         z = _norm(_norm(st))
@@ -156,7 +159,7 @@ def chunked_reference(img, txt, dino, scale, head=None, blocks=(), lambdas=(1.0,
         Cc = s * ((tx * M_it).sum() + (im * M_ti).sum()) + (z * M_s).sum() / tau_s + (tn * M_x).sum() / tau_x
         (A + Cc).backward()
         out["blocks"].append(dict(row0=b0, rows=nb, d_image=im.grad.detach(), d_text=tx.grad.detach(),
-                                  d_student=None if hp is None else st.grad.detach()))
+                                  d_student=None if st is im else st.grad.detach()))
     return out
 
 

@@ -44,3 +44,24 @@ def test_chunked_weighted_loss_matches_oracle(oracle, sym):
     ref = oracle.loss_and_grads(img, txt, 30.0, dino, cfg)["ranks"][0]
     assert chunked_weighted_loss(img, txt, dino, 30.0, 0.2, 0.5, sym, slab=64) == pytest.approx(
         ref["weighted_loss"], rel=1e-9)
+
+
+def test_chunked_reference_student_leaf(oracle):
+    """student_values without a head: the student is a leaf, as in the oracle's rank_loss with a raw student."""
+    from test_gpu_multirank import oracle_ranks
+
+    B, D, Dd = 320, 64, 96
+    img, txt, dino = synth(6, B, D, Dd)
+    g = torch.Generator().manual_seed(2)
+    student = (img @ torch.randn(D, Dd, generator=g)).to(torch.bfloat16).float()
+    ref = oracle_ranks(oracle, img, txt, dino, student, 14.2857, 1, "global", False)[0]
+    got = chunked_reference(img, txt, dino, 14.2857, blocks=[(0, 128), (192, 128)], slab=96, student_values=student)
+    for k in ("classic_loss", "soft_loss", "total_loss"):
+        assert got[k] == pytest.approx(float(ref["terms"][k]), rel=1e-10), k
+    assert got["d_logit_scale"] == pytest.approx(ref["d_scale"], rel=1e-9)
+    for blk in got["blocks"]:
+        rows = slice(blk["row0"], blk["row0"] + blk["rows"])
+        for k in ("d_image", "d_text", "d_student"):
+            want = ref[k][rows]
+            err = (blk[k] - want).abs().max().item() / want.abs().max().item()
+            assert err < 1e-9, (k, blk["row0"], err)
