@@ -25,7 +25,9 @@
 extern "C" {
 #endif
 
-#define DSOFT_VERSION 260 /* 0.2.6: SigLIP loss (DSOFT_F_SIGLIP, dsoft_siglip_*); 0.2.5: retrieval ranks
+#define DSOFT_VERSION 260 /* 0.2.6: SigLIP loss (DSOFT_F_SIGLIP, dsoft_siglip_*), later extended without a number
+                             change by DistillClipLoss (DSOFT_F_DISTILL, dsoft_distill_*: additions only, nothing
+                             existing changed); 0.2.5: retrieval ranks
                              (dsoft_retrieval_ranks); 0.2.4: weighted plans accept the fused
                              backward (no DSOFT_F_GMAT); 0.2.3: weighted
                              CE branch at world > 1 (phases 5 / 6, dsoft_plan_lse_rows, dsoft_plan_wsigma_info) */
@@ -59,6 +61,12 @@ extern "C" {
                                   with Dp = Dd = 0 and no other flag (else DSOFT_EINVAL); runs through
                                   dsoft_siglip_forward / dsoft_siglip_backward, which dsoft_forward /
                                   dsoft_backward refuse.  dsoft_pack and the gathered layout are unchanged. */
+#define DSOFT_F_DISTILL 256u    /* DistillClipLoss (open_clip) instead of the DINO-Soft terms: Dd = the teacher width
+                                  and Dp = Dd; the packed row is image | text | teacher image | teacher text (dsoft_pack's
+                                  student and DINO arguments carry the teacher).  The only other flag it takes is
+                                  DSOFT_F_ROW_ONLY at world > 1 (else DSOFT_EINVAL); runs through
+                                  dsoft_distill_forward / dsoft_distill_backward, which dsoft_forward /
+                                  dsoft_backward refuse. */
 
 /* element types accepted by dsoft_pack */
 #define DSOFT_DT_F32 0
@@ -237,6 +245,35 @@ int dsoft_siglip_forward(const dsoft_plan_t* plan, const void* gathered_dev, con
 int dsoft_siglip_backward(const dsoft_plan_t* plan, const void* gathered_dev, const void* state_dev, void* scratch_dev,
                           const void* g_dev, const float* gout_dev, float* d_image_dev, float* d_text_dev,
                           float* d_scale_dev, float* d_bias_dev, void* stream);
+
+/* DistillClipLoss of a DSOFT_F_DISTILL plan (open_clip DistillClipLoss with local_loss).  x = s <I_i, T_j> (student),
+ * t = s_t <I_t_i, T_t_j> (teacher) over the bf16 columns of `gathered` (fp32 accumulation); p / q = their soft-maxes
+ * over this rank's rows of both directions (image rows x all B texts, text rows x all B images):
+ *   contrastive = 1/2 [mean_i CE(x_i., i) + mean_j CE(x_.j, j)]     (global index of the positive)
+ *   distill     = 1/2 [mean_i (lse(x_i.) - sum_j q_ij x_ij) + mean_j (lse(x_.j) - sum_i q_ij x_ij)]
+ * dsoft_distill_forward: logit_scale_dev = s, dist_logit_scale_dev = s_t (both already exp'd, one fp32 each on the
+ *   device).  losses_dev: [2] fp32 = contrastive, distill.  stats_dev: [4][b] fp32, this rank's row statistics -
+ *   the log-sum-exps (log2 units) of the student and teacher logits of its image rows, then of its text rows.
+ *   Scratch: dsoft_plan_forward_scratch_bytes.
+ * dsoft_distill_backward: the same gathered / state.  stats_all_dev: the [W][4][b] concatenation of every rank's
+ *   stats_dev (the caller all-gathers them; world 1: the forward's stats_dev); with DSOFT_F_ROW_ONLY this rank's
+ *   [4][b] alone.  g_dev: dsoft_distill_g_bytes(plan) bytes (16-byte aligned) for the fp16 logit-gradient matrix of a
+ *   [b x B] row block (world > 1: used by both directions in turn).  gout_dev: [2] fp32 upstream gradients g_c, g_d
+ *   of the two losses.  Outputs fp32, 16-byte aligned: d_image [b][D] and d_text [b][D] = the derivative of the SUM of
+ *   all ranks' losses with respect to this rank's rows (what an all-gather with gradient delivers; DSOFT_F_ROW_ONLY:
+ *   of this rank's loss only, the gathered copies being constants), d_scale [1] = the derivative of this rank's own
+ *   loss with respect to s; this assumes the same s, s_t and upstream gradients on every rank.  The teacher gets no
+ *   gradient.  Scratch: dsoft_plan_scratch_bytes.
+ * Profile slots: 0 / 1 = forward tile kernel (image / text rows), 7 = logit-gradient kernel, 3 / 4 = the gradient
+ * GEMMs (image / text rows).  Both calls are asynchronous on `stream`, make no host synchronisation and can be
+ * captured in a graph. */
+size_t dsoft_distill_g_bytes(const dsoft_plan_t* plan);
+int dsoft_distill_forward(const dsoft_plan_t* plan, const void* gathered_dev, const float* logit_scale_dev,
+                          const float* dist_logit_scale_dev, void* state_dev, void* scratch_dev, float* stats_dev,
+                          float* losses_dev, void* stream);
+int dsoft_distill_backward(const dsoft_plan_t* plan, const void* gathered_dev, const void* state_dev, void* scratch_dev,
+                           const float* stats_all_dev, void* g_dev, const float* gout_dev, float* d_image_dev,
+                           float* d_text_dev, float* d_scale_dev, void* stream);
 
 /* Column (in elements) of the DINO block inside a packed row: where dsoft_gather_rows must write when the caller
  * fills the DINO columns of `gathered` itself (dsoft_pack with dino_dev == NULL). */

@@ -13,6 +13,8 @@ Import as ``dinosoft_b200`` (see the shim at the repo root).  Contents:
     retrieval.py  retrieval ranks and R@K (open_clip get_clip_metrics) on the Gram-tile kernel, no N x N logits
     siglip.py    SigLipLoss drop-in (open_clip SigLipLoss): sigmoid loss and its logit gradient in one tile pass,
                  backward = the two gradient GEMMs, no B x B logit matrix
+    distill.py   DistillClipLoss drop-in (open_clip DistillClipLoss): student and teacher row statistics in the
+                 forward tile pass, one fp16 logit-gradient matrix + the two gradient GEMMs, no B x B logit matrix
     _cabi.py     ctypes binding of libdsoft.so (include/dsoft.h)
     _build.py    nvcc recipe for csrc/ (sm_100a only)
     csrc/        hand-written tcgen05 / TMEM / TMA kernels + the C ABI
@@ -25,6 +27,7 @@ from .graphed import make_graphed
 from .pair_stats import pair_stats
 from .retrieval import clip_metrics, retrieval_ranks
 from .siglip import SigLipLoss
+from .distill import DistillClipLoss
 from .loss import (
     ClipLossWithDINOEnhancements,
     CudaBackend,
@@ -52,5 +55,6 @@ __all__ = [
     "clip_metrics",
     "CyCLIPLoss",
     "SigLipLoss",
+    "DistillClipLoss",
     "make_graphed",
 ]

@@ -12,6 +12,7 @@ from . import _build
 DSOFT_F_SOFT, DSOFT_F_TEXT, DSOFT_F_SOFT_LOCAL, DSOFT_F_ROW_ONLY, DSOFT_F_GMAT = 1, 2, 4, 8, 16
 DSOFT_F_WEIGHTED, DSOFT_F_WSYM = 32, 64
 DSOFT_F_SIGLIP = 128
+DSOFT_F_DISTILL = 256
 DBG_N = 32
 DT_F32, DT_BF16, DT_F16 = 0, 1, 2
 
@@ -65,6 +66,9 @@ PROTOTYPES = {
     "dsoft_siglip_g_bytes": (C.c_size_t, [C.c_void_p]),
     "dsoft_siglip_forward": (C.c_int, [C.c_void_p] * 9),
     "dsoft_siglip_backward": (C.c_int, [C.c_void_p] * 11),
+    "dsoft_distill_g_bytes": (C.c_size_t, [C.c_void_p]),
+    "dsoft_distill_forward": (C.c_int, [C.c_void_p] * 9),
+    "dsoft_distill_backward": (C.c_int, [C.c_void_p] * 11),
     "dsoft_head_forward": (C.c_int, [C.c_void_p] * 6 + [C.c_int32, C.c_void_p, C.c_void_p]),
     "dsoft_forward": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(C.c_float)] + [C.c_void_p] * 6),
     "dsoft_backward": (C.c_int, [C.c_void_p] * 6 + [C.POINTER(C.c_float)] + [C.c_void_p] * 5),

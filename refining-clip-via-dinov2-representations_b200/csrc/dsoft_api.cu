@@ -99,6 +99,11 @@ struct dsoft_plan {
   int siglip;
   size_t sg_part, sg_blk;  // forward scratch: row partials [3][npart][b], per-block sums [3][blocks]
   size_t sg_Gt;            // backward scratch, world > 1: the text rows' fp16 G [bpad][pitch_c]
+  // DSOFT_F_DISTILL: DistillClipLoss on image | text | teacher image | teacher text (the student and DINO slots)
+  int distill;
+  size_t st_ddiag;         // state: raw diagonal dot products [2 directions][student, teacher][b]
+  size_t dl_part, dl_blk;  // forward scratch: row partials [2 directions][6][npart][b], per-block sums [4][blocks]
+  size_t dl_col;           // backward scratch: the column side's statistics by global column [4][Bcol]
 };
 
 static int ceil_div(int a, int b) { return (a + b - 1) / b; }
@@ -195,6 +200,14 @@ extern "C" int dsoft_plan_create(const dsoft_shape_t* sh, dsoft_plan_t** out) {
   }
   if ((sh->flags & DSOFT_F_SIGLIP) && (sh->flags != DSOFT_F_SIGLIP || sh->Dp != 0 || sh->Dd != 0))
     return fail(DSOFT_EINVAL, "DSOFT_F_SIGLIP takes no other flag and needs Dp = Dd = 0");
+  if (sh->flags & DSOFT_F_DISTILL) {
+    const uint32_t other = sh->flags & ~(DSOFT_F_DISTILL | (sh->world > 1 ? DSOFT_F_ROW_ONLY : 0u));
+    if (other)
+      return fail(DSOFT_EINVAL, "DSOFT_F_DISTILL takes no other flag than DSOFT_F_ROW_ONLY at world > 1 (flags %u)",
+                  sh->flags);
+    if (sh->Dd <= 0 || sh->Dp != sh->Dd)
+      return fail(DSOFT_EINVAL, "DSOFT_F_DISTILL needs Dp = Dd > 0, the teacher width (Dp=%d Dd=%d)", sh->Dp, sh->Dd);
+  }
   if (static_cast<long>(sh->b) * sh->world > (1L << 30)) return fail(DSOFT_EINVAL, "batch too large");
   if (sh->D > 2048 || sh->Dp > 2048) return fail(DSOFT_EINVAL, "feature dims above 2048 are not supported");
 
@@ -324,6 +337,39 @@ extern "C" int dsoft_plan_create(const dsoft_shape_t* sh, dsoft_plan_t** out) {
     *out = p;
     return 0;
   }
+  if (sh->flags & DSOFT_F_DISTILL) {
+    // packed row: image | text | teacher image | teacher text (dsoft_pack's student and DINO slots).  State: the
+    // scalar block and the diagonal dot products.  Forward scratch: the row partials of both directions.  Backward
+    // scratch: the column-side statistics, the gradient GEMMs' split partials and the fp16 text | image operands.
+    // The logit-gradient matrix is the caller's (dsoft_distill_g_bytes); at world > 1 the text rows reuse it.
+    const int pairs = ceil_div(rbs, 2);
+    p->distill = 1;
+    p->Dz = sh->Dd;
+    p->offZ = 2 * sh->D;
+    p->offD = 2 * sh->D + sh->Dd;
+    p->row_elems = 2 * sh->D + 2 * sh->Dd;
+    p->clip_tr = sh->world == 1;
+    p->g_clip = choose_gy_split(pairs * ceil_div(sh->D, GY_N), p->pitch_c / 64, sms, sh->b, sh->D);
+    p->g_clip_t = choose_gy_split(pairs * ceil_div(sh->D, GY_N), rbs * 2, sms, sh->b, sh->D);
+    p->st_scal = take(SC_COUNT);
+    p->st_ddiag = take(static_cast<size_t>(4) * sh->b);
+    p->st_total = o;
+    o = 0;
+    p->dl_part = take(static_cast<size_t>(2) * 6 * 2 * p->f_wce.nsplit * sh->b);
+    p->dl_blk = take(static_cast<size_t>(4) * ceil_div(2 * sh->b, 128));
+    p->sc_fwd_total = o;
+    const size_t ns_t = p->clip_tr ? p->g_clip_t.nsplit : p->g_clip.nsplit;
+    p->dl_col = take(static_cast<size_t>(4) * p->Bcol);
+    p->sc_acc1 = take(static_cast<size_t>(p->g_clip.nsplit) * sh->b * sh->D);
+    p->sc_acc2 = take(ns_t * sh->b * sh->D);
+    p->v_offT = 0;
+    p->v_offI = sh->D;
+    p->v_row = 2 * sh->D;
+    p->sc_v16 = take(static_cast<size_t>(p->B) * p->v_row / 2 + 1);
+    p->sc_total = o;
+    *out = p;
+    return 0;
+  }
   p->st_scal = take(SC_COUNT);
   p->st_rinv_t = take(p->Bcol);
   p->st_rinv_z = take(p->Bcol);
@@ -397,6 +443,10 @@ extern "C" size_t dsoft_plan_forward_scratch_bytes(const dsoft_plan_t* p) { retu
 extern "C" double dsoft_plan_algorithmic_flops(const dsoft_plan_t* p) {
   if (!p) return 0.0;
   if (p->siglip) return 2.0 * p->sh.b * p->B * (3.0 * p->sh.D);  // I . T^T, G . T, G^T . I
+  if (p->distill) {  // forward: both products per direction; G: both products once (world 1) or per direction
+    const double pr = p->sh.D + p->sh.Dd;
+    return 2.0 * p->sh.b * p->B * (2.0 * pr + (p->clip_tr ? 1.0 : 2.0) * pr + 2.0 * p->sh.D);
+  }
   // SURVEY.md 8(d): F_alg = 2 B^2 (3D + 2Dp + Dd [+ 2D]) for the whole job; this rank's share is 1/W.
   const double b = p->sh.b, cols_c = p->B, cols_s = p->sym_w ? p->B : p->s_ncols;
   double f = 2.0 * b * cols_c * (3.0 * p->sh.D);
@@ -414,6 +464,12 @@ extern "C" int dsoft_plan_kernel_flops(const dsoft_plan_t* p, double* algorithmi
   if (p->siglip) {  // [0] forward tile kernel, [3] / [4] gradient GEMMs, [7] world > 1: the text rows' G kernel
     algorithmic[0] = executed[0] = algorithmic[3] = executed[3] = algorithmic[4] = executed[4] = 2.0 * b * Bc * D;
     if (n > 7 && !p->clip_tr) executed[7] = 2.0 * b * Bc * D;
+    return 0;
+  }
+  if (p->distill) {  // [0] / [1] forward image / text rows, [3] / [4] gradient GEMMs, [7] the logit-gradient kernel
+    algorithmic[0] = executed[0] = algorithmic[1] = executed[1] = 2.0 * b * Bc * (D + Dd);
+    algorithmic[3] = executed[3] = algorithmic[4] = executed[4] = 2.0 * b * Bc * D;
+    if (n > 7) algorithmic[7] = executed[7] = (p->clip_tr ? 1.0 : 2.0) * 2.0 * b * Bc * (D + Dd);
     return 0;
   }
   // forward CLIP: the two directions are exact transposes -> one algorithmic product, two executed
@@ -453,12 +509,14 @@ extern "C" int dsoft_plan_kernel_flops(const dsoft_plan_t* p, double* algorithmi
 extern "C" int dsoft_plan_launches_forward(const dsoft_plan_t* p) {
   if (!p) return 0;
   if (p->siglip) return 3;  // scalars, tile kernel, finalize
+  if (p->distill) return 4;  // scalars, tile kernel x 2 directions, finalize
   return 1 /*pack*/ + 1 /*scalars*/ + 1 /*norms*/ + 2 /*clip x2*/ + (p->have_soft ? 1 : 0) + (p->fwd_sym ? 1 : 0) +
          1 /*finalize*/ + (p->weighted ? (p->wsym ? 2 : 1) * 7 + 1 : 0);
 }
 extern "C" int dsoft_plan_launches_backward(const dsoft_plan_t* p) {
   if (!p) return 0;
   if (p->siglip) return p->clip_tr ? 4 : 5;  // fp16 operands, [text rows' G,] two gradient GEMMs, finalize
+  if (p->distill) return p->clip_tr ? 6 : 7;  // scalars + relayout, fp16 operands, G (x 2), two GEMMs, finalize
   if (p->gmat)
     return 3 /*lse stats, relayout, fp16 operands*/ + (p->weighted && !p->clip_tr ? 1 : 0) /*weighted relayout*/ +
            (p->clip_tr ? 1 : 2) /*clip G*/ + 2 /*clip GEMMs*/ +
@@ -516,7 +574,7 @@ static int make_maps(const dsoft_plan* p, const void* gathered, TileMaps* tm, in
   if ((rc = make_map(&tm->m[0], g + p->offI, p->B, p->sh.D, p->row_elems, bf, box_rows))) return rc;
   if ((rc = make_map(&tm->m[1], g + p->offT, p->B, p->sh.D, p->row_elems, bf, box_rows))) return rc;
   if ((rc = make_map(&tm->m[2], g + p->offZ, p->B, p->Dz, p->row_elems, bf, box_rows))) return rc;
-  if (p->have_soft || p->weighted) {
+  if (p->have_soft || p->weighted || p->distill) {
     if ((rc = make_map(&tm->m[3], g + p->offD, p->B, p->sh.Dd, p->row_elems, bf, box_rows))) return rc;
   } else {
     tm->m[3] = tm->m[0];
@@ -1667,8 +1725,9 @@ extern "C" int dsoft_pack(const dsoft_plan_t* p, const void* image, int image_dt
   int rc;
   if ((rc = add(image, image_dt, ld_image, p->sh.D, p->offI))) return rc;
   if ((rc = add(text, text_dt, ld_text, p->sh.D, p->offT))) return rc;
-  if (p->have_proj && student && (rc = add(student, student_dt, ld_student, p->sh.Dp, p->offZ))) return rc;
-  if ((p->have_soft || p->weighted) && dino && (rc = add(dino, dino_dt, ld_dino, p->sh.Dd, p->offD))) return rc;
+  if ((p->have_proj || p->distill) && student && (rc = add(student, student_dt, ld_student, p->sh.Dp, p->offZ)))
+    return rc;
+  if ((p->have_soft || p->weighted || p->distill) && dino && (rc = add(dino, dino_dt, ld_dino, p->sh.Dd, p->offD))) return rc;
   bool vec8 = reinterpret_cast<uintptr_t>(base) % 16 == 0 && a.dst_ld % 8 == 0;
   for (int k = 0; k < a.nmat; ++k) {
     const PackSrc& m = a.m[k];
@@ -2388,6 +2447,7 @@ static int forward_impl(const dsoft_plan_t* p, const void* gathered, const float
   if (!p || !gathered || !logit_scale || !lambdas || !state || !scratch || !lse_local || !losses)
     return fail(DSOFT_EINVAL, "null argument");
   if (p->siglip) return fail(DSOFT_EINVAL, "a DSOFT_F_SIGLIP plan runs through dsoft_siglip_forward");
+  if (p->distill) return fail(DSOFT_EINVAL, "a DSOFT_F_DISTILL plan runs through dsoft_distill_forward");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   float* S = static_cast<float*>(state);
   float* X = static_cast<float*>(scratch);
@@ -2889,6 +2949,7 @@ static int backward_impl(const dsoft_plan_t* p, const void* gathered, const void
   if (!p || !gathered || !state || !scratch || !lse_all || !gout || !lambdas || !d_image || !d_text || !d_scale)
     return fail(DSOFT_EINVAL, "null argument");
   if (p->siglip) return fail(DSOFT_EINVAL, "a DSOFT_F_SIGLIP plan runs through dsoft_siglip_backward");
+  if (p->distill) return fail(DSOFT_EINVAL, "a DSOFT_F_DISTILL plan runs through dsoft_distill_backward");
   if (p->have_proj && !d_student) return fail(DSOFT_EINVAL, "d_student is null but the plan has Dp > 0");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   // state is logically const for the caller; the relayouted LSE columns live in it
@@ -3351,6 +3412,338 @@ extern "C" int dsoft_siglip_backward(const dsoft_plan_t* p, const void* gathered
   fa.d_bias = d_bias;
   const size_t work = static_cast<size_t>(b) * (p->sh.D / 4);
   siglip_finalize_bwd_kernel<<<static_cast<int>(std::min<size_t>((work + 255) / 256, p->num_sms * 8)), 256, 0, st>>>(fa);
+  CUDA_TRY(cudaGetLastError());
+  return 0;
+}
+
+// ------------------------------------------------------------------------------------------------
+// DistillClipLoss (open_clip) on the Gram-tile kernels.  x = s I T^T (student), t = s_t I_t T_t^T (teacher); p / q
+// their soft-maxes over rows (image -> text) or columns (text -> image):
+//   contrastive = 1/2 [CE_row(x, diag) + CE_col(x, diag)],  distill = 1/2 [CE_row(x, q_row) + CE_col(x, q_col)]
+//   dL/dx_ij = 1/(2b) [(g_c + g_d)(p_r + p_c) - g_d (q_r + q_c) - 2 g_c delta_ij]
+// Forward: dsoft_fwd_kernel<MODE_DIST_FWD> once per direction (its rows against all B columns), then a finalize that
+// merges the split partials into the per-row log-sum-exps (the [4][b] statistics the backward's column side needs)
+// and reduces the losses and the d(logit_scale) sums in fp64.  Backward: dsoft_fwd_kernel<MODE_DIST_G> writes the
+// fp16 G of one direction's rows (world 1: one matrix serves both directions, dT = G^T I), the gradient GEMMs, and a
+// finalize that applies the diagonal entries in fp32 and the s / (2b) factors.
+// ------------------------------------------------------------------------------------------------
+__global__ void dist_prep_kernel(const float* __restrict__ logit_scale, const float* __restrict__ dist_scale,
+                                 float* __restrict__ scal) {
+  if (threadIdx.x != 0 || blockIdx.x != 0) return;
+  const float L2E = 1.4426950408889634f;
+  const float s = *logit_scale;
+  scal[SC_SCALE] = s;
+  scal[SC_SCALE_L2] = s * L2E;
+  scal[SC_DST_TSCALE_L2] = *dist_scale * L2E;
+  scal[SC_DST_SPD] = scal[SC_DST_SPQ] = 0.f;
+  scal[SC_TICKET_DST] = 0.f;  // all-zero bits == integer 0
+}
+
+static void fill_dist(const dsoft_plan* p, FwdParams& P, int dir, float* S) {
+  memset(&P, 0, sizeof(P));
+  P.nprod = 2;
+  P.bn = 2 * BN;
+  P.a_map[0] = dir == 0 ? 0 : 1;  // student: image rows x text columns / text rows x image columns
+  P.b_map[0] = dir == 0 ? 1 : 0;
+  P.a_map[1] = dir == 0 ? 2 : 3;  // teacher: the same pairs of the teacher blocks
+  P.b_map[1] = dir == 0 ? 3 : 2;
+  P.kchunks[0] = ceil_div(p->sh.D, BK);
+  P.kchunks[1] = ceil_div(p->sh.Dd, BK);
+  P.row0 = p->sh.rank * p->sh.b;
+  P.b = p->sh.b;
+  P.col0 = 0;
+  P.ncols = p->B;
+  P.ntiles = ceil_div(p->B, 2 * BN);
+  P.tiles_per_split = p->f_wce.tps;
+  P.npart = 2 * p->f_wce.nsplit;
+  P.scal = S + p->st_scal;
+  P.wdir = dir;
+}
+
+struct DlFinFwdArgs {
+  int b, npart;
+  const float* part;  // [2][6][npart][b]: student m, sum, sum (x-m); teacher m_t, sum, sum (x-m) weighted by teacher
+  const float* diag;  // [2][2][b] raw diagonal dot products (direction, student / teacher)
+  float* stats;       // [4][b] out: student / teacher lse (log2) of the image rows, then of the text rows
+  float* blk;         // [4][gridDim.x]
+  float* scal;
+  float* losses;      // [2]: contrastive, distill
+  int* ticket;
+};
+
+// One thread per (direction, local row): merge the split partials, write the row's two log-sum-exps, and sum
+//   contrastive: lse - x_ii,  distill: lse - sum q x,  sum p x - x_ii,  sum p x - sum q x   (natural units)
+// per block in a fixed order; the last block adds the blocks in fp64 (deterministic, as finalize_fwd_kernel).
+__global__ void __launch_bounds__(128) dist_finalize_fwd_kernel(DlFinFwdArgs a) {
+  const float LN2 = 0.6931471805599453f;
+  const int r = blockIdx.x * blockDim.x + threadIdx.x;
+  float v[4] = {0.f, 0.f, 0.f, 0.f};
+  if (r < 2 * a.b) {
+    const int dir = r >= a.b, i = r - dir * a.b;
+    const size_t st = static_cast<size_t>(a.npart) * a.b;
+    const float* pp = a.part + dir * 6 * st + i;
+    float M = M_FLOOR, Mt = M_FLOOR;
+    for (int s = 0; s < a.npart; ++s) {
+      M = fmaxf(M, pp[0 * st + s * a.b]);
+      Mt = fmaxf(Mt, pp[3 * st + s * a.b]);
+    }
+    float S = 0.f, Ps = 0.f, St = 0.f, Q = 0.f;
+    for (int s = 0; s < a.npart; ++s) {
+      const size_t o = static_cast<size_t>(s) * a.b;
+      const float dm = pp[0 * st + o] - M;
+      const float f = exp2f(dm), ft = exp2f(pp[3 * st + o] - Mt);
+      S = fmaf(pp[1 * st + o], f, S);
+      Ps = fmaf(f, fmaf(dm, pp[1 * st + o], pp[2 * st + o]), Ps);
+      St = fmaf(pp[4 * st + o], ft, St);
+      Q = fmaf(ft, fmaf(dm, pp[4 * st + o], pp[5 * st + o]), Q);
+    }
+    const float l2s = log2f(S);
+    a.stats[(2 * dir + 0) * a.b + i] = M + l2s;
+    a.stats[(2 * dir + 1) * a.b + i] = Mt + log2f(St);
+    const float d2 = a.diag[(2 * dir) * a.b + i] * a.scal[SC_SCALE_L2];  // as the tile kernel scales it
+    const float px = Ps / S, qx = Q / St;  // sum p (x - M), sum q (x - M), log2 units
+    v[0] = LN2 * ((M - d2) + l2s);
+    v[1] = LN2 * (l2s - qx);
+    v[2] = LN2 * (px + (M - d2));
+    v[3] = LN2 * (px - qx);
+  }
+  __shared__ float shp[4][4];
+#pragma unroll
+  for (int k = 0; k < 4; ++k) {
+    float x = v[k];
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) x += __shfl_xor_sync(0xffffffffu, x, o);
+    if ((threadIdx.x & 31) == 0) shp[k][threadIdx.x >> 5] = x;
+  }
+  __syncthreads();
+  if (threadIdx.x < 4)
+    a.blk[threadIdx.x * gridDim.x + blockIdx.x] =
+        (shp[threadIdx.x][0] + shp[threadIdx.x][1]) + (shp[threadIdx.x][2] + shp[threadIdx.x][3]);
+  if (last_block_done(a.ticket)) {
+    __shared__ double sums[4];
+    block_reduce_rows(a.blk, gridDim.x, 4, sums);
+    if (threadIdx.x == 0) {
+      a.losses[0] = static_cast<float>(sums[0] * 0.5 / a.b);
+      a.losses[1] = static_cast<float>(sums[1] * 0.5 / a.b);
+      a.scal[SC_DST_SPD] = static_cast<float>(sums[2]);
+      a.scal[SC_DST_SPQ] = static_cast<float>(sums[3]);
+    }
+  }
+}
+
+// Backward scalars: gk = 2^(14 - max(0, e)) with |g_c| + |g_d| < 2^e, so that |G gk| < 2^15 (|G| <= 2 (|g_c| + |g_d|))
+// and probabilities down to 2^-28 stay normal fp16 numbers; and the column side's statistics by global column,
+// [4][Bcol] from the all-gathered [W][4][b] (zero past B).
+__global__ void __launch_bounds__(256) dist_relayout_kernel(const float* __restrict__ stats_all, int W, int b, int Bcol,
+                                                            const float* __restrict__ gout, float* __restrict__ scal,
+                                                            float* __restrict__ col) {
+  if (blockIdx.x == 0 && threadIdx.x == 0) {
+    const float gc = gout[0], gd = gout[1];
+    int e = 0;
+    frexpf(fabsf(gc) + fabsf(gd), &e);
+    const float gk = ldexpf(1.f, 14 - max(e, 0));
+    scal[SC_DST_GK] = gk;
+    scal[SC_DST_GC] = gc * gk;
+    scal[SC_DST_GD] = gd * gk;
+  }
+  if (!col) return;
+  const int B = W * b;
+  for (int idx = blockIdx.x * blockDim.x + threadIdx.x; idx < 4 * Bcol; idx += gridDim.x * blockDim.x) {
+    const int k = idx / Bcol, g = idx - k * Bcol;
+    float v = 0.f;
+    if (g < B) {
+      const int w = g / b;
+      v = stats_all[(static_cast<size_t>(w) * 4 + k) * b + (g - w * b)];
+    }
+    col[idx] = v;
+  }
+}
+
+struct DlFinBwdArgs {
+  int b, D, row0, row_elems, offI, offT, ns1, ns2, row_only;
+  const __nv_bfloat16* gathered;
+  const float* acc1;   // [ns1][b][D]  sum_j (G gk)_ij T_j   (image rows)
+  const float* acc2;   // [ns2][b][D]  sum_i (G gk)_ij I_i   (text rows)
+  const float* stats;  // [4][b] this rank's row statistics (log2 lse: image student / teacher, text student / teacher)
+  const float* diag;   // [2][2][b] raw diagonal dot products
+  const float* scal;
+  const float* gout;   // [2] g_c, g_d
+  float* d_image;
+  float* d_text;
+  float* d_scale;
+};
+
+// one term of the diagonal entry, in fp32: g_c (p - 1) + g_d (p - q) with p = 2^(x - lse), q = 2^(t - lse_t)
+__device__ __forceinline__ float dist_diag_term(float gc, float gd, float x2, float t2, float lse, float lset) {
+  const float LN2 = 0.6931471805599453f;
+  const float pm1 = expm1f(LN2 * (x2 - lse)), qm1 = expm1f(LN2 * (t2 - lset));
+  return fmaf(gc, pm1, gd * (pm1 - qm1));
+}
+
+// One warp per local row: d image = s / (2b) (sum of the split partials / gk + dg_I T_i), d text likewise with I_i;
+// dg = the pair (i, i)'s entry of dL/dx (2b), row side plus (unless row_only) column side.  d s from the forward's
+// sums: (g_c sum (p x - x_ii) + g_d sum (p x - q x)) / (2 b s).
+__global__ void __launch_bounds__(256) dist_finalize_bwd_kernel(DlFinBwdArgs a) {
+  const float gc = a.gout[0], gd = a.gout[1];
+  const float s = a.scal[SC_SCALE], s2 = a.scal[SC_SCALE_L2], st2 = a.scal[SC_DST_TSCALE_L2];
+  const float coef = s * 0.5f / static_cast<float>(a.b);
+  const float igk = 1.f / a.scal[SC_DST_GK];
+  const int lane = threadIdx.x & 31;
+  for (int i = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); i < a.b; i += gridDim.x * (blockDim.x >> 5)) {
+    const float* S = a.stats;
+    const float xI = a.diag[0 * a.b + i] * s2, tI = a.diag[1 * a.b + i] * st2;  // image row i, column i
+    const float xT = a.diag[2 * a.b + i] * s2, tT = a.diag[3 * a.b + i] * st2;  // text row i, column i
+    float dgI = dist_diag_term(gc, gd, xI, tI, S[0 * a.b + i], S[1 * a.b + i]);
+    float dgT = dist_diag_term(gc, gd, xT, tT, S[2 * a.b + i], S[3 * a.b + i]);
+    if (!a.row_only) {
+      dgI += dist_diag_term(gc, gd, xI, tI, S[2 * a.b + i], S[3 * a.b + i]);
+      dgT += dist_diag_term(gc, gd, xT, tT, S[0 * a.b + i], S[1 * a.b + i]);
+    }
+    const __nv_bfloat16* row = a.gathered + static_cast<size_t>(a.row0 + i) * a.row_elems;
+    for (int f = lane * 4; f < a.D; f += 128) {
+      const float4 ti = load_bf16x4(row + a.offT + f), ii = load_bf16x4(row + a.offI + f);
+      float4 u = sum_splits4(a.acc1, a.ns1, a.b, a.D, i, f);
+      *reinterpret_cast<float4*>(a.d_image + static_cast<size_t>(i) * a.D + f) =
+          make_float4(coef * fmaf(u.x, igk, dgI * ti.x), coef * fmaf(u.y, igk, dgI * ti.y),
+                      coef * fmaf(u.z, igk, dgI * ti.z), coef * fmaf(u.w, igk, dgI * ti.w));
+      u = sum_splits4(a.acc2, a.ns2, a.b, a.D, i, f);
+      *reinterpret_cast<float4*>(a.d_text + static_cast<size_t>(i) * a.D + f) =
+          make_float4(coef * fmaf(u.x, igk, dgT * ii.x), coef * fmaf(u.y, igk, dgT * ii.y),
+                      coef * fmaf(u.z, igk, dgT * ii.z), coef * fmaf(u.w, igk, dgT * ii.w));
+    }
+  }
+  if (blockIdx.x == 0 && threadIdx.x == 0)
+    a.d_scale[0] = (gc * a.scal[SC_DST_SPD] + gd * a.scal[SC_DST_SPQ]) * 0.5f / (static_cast<float>(a.b) * s);
+}
+
+extern "C" size_t dsoft_distill_g_bytes(const dsoft_plan_t* p) {
+  if (!p || !p->distill) return 0;
+  return static_cast<size_t>(ceil_div(p->sh.b, BM)) * BM * p->pitch_c * 2;
+}
+
+extern "C" int dsoft_distill_forward(const dsoft_plan_t* p, const void* gathered, const float* logit_scale,
+                                     const float* dist_logit_scale, void* state, void* scratch, float* stats,
+                                     float* losses, void* stream) {
+  if (!p || !gathered || !logit_scale || !dist_logit_scale || !state || !scratch || !stats || !losses)
+    return fail(DSOFT_EINVAL, "null argument");
+  if (!p->distill) return fail(DSOFT_EINVAL, "dsoft_distill_forward needs a DSOFT_F_DISTILL plan");
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  float* S = static_cast<float*>(state);
+  float* X = static_cast<float*>(scratch);
+  const int b = p->sh.b, rbs = ceil_div(b, BM);
+  const size_t dpart = static_cast<size_t>(6) * 2 * p->f_wce.nsplit * b;
+  TileMaps tm;
+  int rc = make_maps(p, gathered, &tm, 64);
+  if (rc) return rc;
+  dist_prep_kernel<<<1, 32, 0, st>>>(logit_scale, dist_logit_scale, S + p->st_scal);
+  CUDA_TRY(cudaGetLastError());
+  if ((rc = set_smem(dsoft_fwd_kernel<MODE_DIST_FWD, 2>, FWD_SMEM_BYTES))) return rc;
+  for (int d = 0; d < 2; ++d) {
+    FwdParams P;
+    fill_dist(p, P, d, S);
+    P.part = X + p->dl_part + d * dpart;
+    P.diag = S + p->st_ddiag + static_cast<size_t>(d) * 2 * b;
+    ProfScope ps(d == 0 ? PK_FWD_CLIP_IT : PK_FWD_CLIP_TI, st);
+    if ((rc = launch_fwd_pair(dsoft_fwd_kernel<MODE_DIST_FWD, 2>, rbs, p->f_wce.nsplit, st, tm, P))) return rc;
+  }
+  DlFinFwdArgs fa;
+  fa.b = b;
+  fa.npart = 2 * p->f_wce.nsplit;
+  fa.part = X + p->dl_part;
+  fa.diag = S + p->st_ddiag;
+  fa.stats = stats;
+  fa.blk = X + p->dl_blk;
+  fa.scal = S + p->st_scal;
+  fa.losses = losses;
+  fa.ticket = reinterpret_cast<int*>(S + p->st_scal + SC_TICKET_DST);
+  dist_finalize_fwd_kernel<<<ceil_div(2 * b, 128), 128, 0, st>>>(fa);
+  CUDA_TRY(cudaGetLastError());
+  return 0;
+}
+
+extern "C" int dsoft_distill_backward(const dsoft_plan_t* p, const void* gathered, const void* state, void* scratch,
+                                      const float* stats_all, void* g, const float* gout, float* d_image,
+                                      float* d_text, float* d_scale, void* stream) {
+  if (!p || !gathered || !state || !scratch || !stats_all || !g || !gout || !d_image || !d_text || !d_scale)
+    return fail(DSOFT_EINVAL, "null argument");
+  if (!p->distill) return fail(DSOFT_EINVAL, "dsoft_distill_backward needs a DSOFT_F_DISTILL plan");
+  if (reinterpret_cast<uintptr_t>(g) % 16 || reinterpret_cast<uintptr_t>(d_image) % 16 ||
+      reinterpret_cast<uintptr_t>(d_text) % 16)
+    return fail(DSOFT_EINVAL, "g, d_image and d_text must be 16-byte aligned");
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  float* S = const_cast<float*>(static_cast<const float*>(state));  // the backward's scalars live in the scalar block
+  float* X = static_cast<float*>(scratch);
+  const int b = p->sh.b, rbs = ceil_div(b, BM);
+  // row_only: the caller passes this rank's [4][b] only, and the column side is not read
+  const float* stats_loc = p->row_only ? stats_all : stats_all + static_cast<size_t>(p->sh.rank) * 4 * b;
+  float* col = p->row_only ? nullptr : X + p->dl_col;
+  __half* G = static_cast<__half*>(g);
+  __half* v16 = reinterpret_cast<__half*>(X + p->sc_v16);
+  TileMaps tm;
+  int rc = make_maps(p, gathered, &tm, 64);
+  if (rc) return rc;
+  dist_relayout_kernel<<<col ? std::min(ceil_div(4 * p->Bcol, 256), p->num_sms * 4) : 1, 256, 0, st>>>(
+      stats_all, p->sh.world, b, p->Bcol, gout, S + p->st_scal, col);
+  CUDA_TRY(cudaGetLastError());
+  make_v16_kernel<<<ceil_div(p->B, 8), 256, 0, st>>>(
+      static_cast<const __nv_bfloat16*>(gathered), p->row_elems, p->B, p->sh.D, p->Dz, p->offI, p->offT, p->offZ, 0, 0,
+      nullptr, nullptr, v16, p->v_row, p->v_offT, p->v_offI, 0, 0);
+  CUDA_TRY(cudaGetLastError());
+  if ((rc = set_smem(dsoft_gy_kernel<false>, GY_SMEM_BYTES))) return rc;
+  if ((rc = set_smem(dsoft_gy_kernel<true>, GY_SMEM_BYTES))) return rc;
+  if ((rc = set_smem(dsoft_fwd_kernel<MODE_DIST_G, 2>, FWD_SMEM_BYTES))) return rc;
+  if ((rc = make_gstore_map(p, &tm.g[0], G, p->pitch_c))) return rc;
+  tm.g[1] = tm.g[0];
+  // d = 0: image rows (dI = G . T; world 1 also dT = G^T . I), d = 1 (world > 1): text rows into the same buffer
+  for (int d = 0; d < (p->clip_tr ? 1 : 2); ++d) {
+    FwdParams P;
+    fill_dist(p, P, d, S);
+    P.wrow[0] = stats_loc + static_cast<size_t>(2 * d) * b;
+    P.wrow[1] = stats_loc + static_cast<size_t>(2 * d + 1) * b;
+    P.ncolvec = col ? 2 : 0;
+    if (col) {
+      P.colvec[0] = col + static_cast<size_t>(2 * (1 - d)) * p->Bcol;
+      P.colvec[1] = col + static_cast<size_t>(2 * (1 - d) + 1) * p->Bcol;
+    }
+    P.row_only = p->row_only;
+    P.gout[0] = G;
+    P.g_pitch = p->pitch_c;
+    {
+      ProfScope ps(PK_BWD_GCLIP, st);
+      if ((rc = launch_fwd_pair(dsoft_fwd_kernel<MODE_DIST_G, 2>, rbs, p->f_wce.nsplit, st, tm, P))) return rc;
+    }
+    if (d == 0) {
+      ProfScope ps(PK_BWD_CLIP_I, st);
+      if ((rc = launch_gy(p, G, p->pitch_c, v16, p->v_offT, p->sh.D, 0, p->g_clip, X + p->sc_acc1, st))) return rc;
+    }
+    if (p->clip_tr || d == 1) {
+      ProfScope ps(PK_BWD_CLIP_T, st);
+      if ((rc = launch_gy(p, G, p->pitch_c, v16, p->v_offI, p->sh.D, 0, p->clip_tr ? p->g_clip_t : p->g_clip,
+                          X + p->sc_acc2, st, p->clip_tr)))
+        return rc;
+    }
+  }
+  DlFinBwdArgs fa;
+  fa.b = b;
+  fa.D = p->sh.D;
+  fa.row0 = p->sh.rank * b;
+  fa.row_elems = p->row_elems;
+  fa.offI = p->offI;
+  fa.offT = p->offT;
+  fa.ns1 = p->g_clip.nsplit;
+  fa.ns2 = p->clip_tr ? p->g_clip_t.nsplit : p->g_clip.nsplit;
+  fa.row_only = p->row_only;
+  fa.gathered = static_cast<const __nv_bfloat16*>(gathered);
+  fa.acc1 = X + p->sc_acc1;
+  fa.acc2 = X + p->sc_acc2;
+  fa.stats = stats_loc;
+  fa.diag = S + p->st_ddiag;
+  fa.scal = S + p->st_scal;
+  fa.gout = gout;
+  fa.d_image = d_image;
+  fa.d_text = d_text;
+  fa.d_scale = d_scale;
+  dist_finalize_bwd_kernel<<<std::min(ceil_div(b, 8), p->num_sms * 8), 256, 0, st>>>(fa);
   CUDA_TRY(cudaGetLastError());
   return 0;
 }

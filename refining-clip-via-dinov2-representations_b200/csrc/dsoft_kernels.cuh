@@ -65,6 +65,9 @@ constexpr int MODE_RANKS = 14;    // retrieval ranks (open_clip get_clip_metrics
 constexpr int MODE_SIGLIP = 15;   // SigLIP sigmoid loss (open_clip SigLipLoss): per pair loss and logit gradient from the
                                   // pair's own logit; writes the fp16 G tile (scaled by 2^SIG_GK) and row partials
 constexpr int SIG_GK = 14;        // SigLIP G is stored as G * 2^14: |G| < 1, and sigma down to 2^-28 stays normal fp16
+constexpr int MODE_DIST_FWD = 16; // DistillClipLoss (open_clip): student and teacher row statistics of one direction
+                                  // from two products per tile (student logits, teacher logits)
+constexpr int MODE_DIST_G = 17;   // DistillClipLoss logit gradient of one direction's rows, both directions' terms
 
 // scalar block computed on device by prep_scalars_kernel (no host sync on logit_scale)
 enum {
@@ -89,6 +92,13 @@ enum {
   SC_SIG_GX = 21,   // SigLIP: sum over this rank's pairs of G x (d logit_scale, before gout / b), by the forward
   SC_SIG_G = 22,    // SigLIP: sum of G (d logit_bias, before gout / b)
   SC_TICKET_S = 23, // (int) SigLIP finalize tickets (forward, backward)
+  SC_DST_TSCALE_L2 = 24, // DistillClipLoss: teacher scale s_t * log2(e)
+  SC_DST_GC = 25,   // DistillClipLoss backward: g_c * gk (contrastive upstream gradient times the G scale)
+  SC_DST_GD = 26,   // g_d * gk (distill upstream gradient times the G scale)
+  SC_DST_GK = 27,   // gk: power-of-two scale of the fp16 G (2^14 while |g_c| + |g_d| <= 1)
+  SC_DST_SPD = 28,  // sum over this rank's rows of both directions of (sum_j p x - x_ii), by the forward
+  SC_DST_SPQ = 29,  // sum over the same rows of (sum_j p x - sum_j q x)
+  SC_TICKET_DST = 30, // (int) DistillClipLoss forward finalize ticket
   SC_COUNT = 32
 };
 
@@ -457,8 +467,9 @@ dsoft_fwd_kernel(const __grid_constant__ TileMaps maps, const __grid_constant__ 
   // "soft-like": 256-column tiles with several products per tile, staged per-column vectors, setmaxnreg
   constexpr bool kPairs = (MODE == MODE_PAIRS);  // two products per tile like the weighted-CE passes, no column vectors
   constexpr bool kRanks = (MODE == MODE_RANKS);  // one product per tile, column vectors from P.colvec
+  constexpr bool kDist = (MODE == MODE_DIST_FWD || MODE == MODE_DIST_G);  // two products, column vectors from P.colvec
   constexpr bool kSoftMode = (MODE == MODE_SOFT || MODE == MODE_SOFT_G || MODE == MODE_SOFT_SYM16 || kWce || kPairs ||
-                              kRanks);
+                              kRanks || kDist);
   static_assert(!kSoftMode || CG == 2, "the soft modes are written for CTA pairs");
   // streaming mode: stages of (A box | B boxes); resident mode: 8 A boxes, then B-only stages
   const bool resident = P.resident != 0;
@@ -470,8 +481,8 @@ dsoft_fwd_kernel(const __grid_constant__ TileMaps maps, const __grid_constant__ 
   // soft modes: 6 stages of 32 KiB (logit-gradient mode: 5); the 32 KiB behind them hold the staged per-column
   // vectors.  Logit-gradient modes keep 32 KiB (at 192 KiB; soft: at 160 KiB) for the G staging strips.
   constexpr bool kClipG = (MODE == MODE_CLIP_G || MODE == MODE_SIGLIP);  // one product, G staging behind the ring
-  constexpr bool kGMode = (kClipG || MODE == MODE_SOFT_G || MODE == MODE_WCE_G);
-  constexpr bool kSoftG = (MODE == MODE_SOFT_G || MODE == MODE_WCE_G);
+  constexpr bool kGMode = (kClipG || MODE == MODE_SOFT_G || MODE == MODE_WCE_G || MODE == MODE_DIST_G);
+  constexpr bool kSoftG = (MODE == MODE_SOFT_G || MODE == MODE_WCE_G || MODE == MODE_DIST_G);
   const int nstages = kSoftG ? 5 : (kSoftMode ? 6 :
                       min(kClipG ? (resident ? 4 : 6) : 8, (resident ? 6 : 14) * TILE_BYTES / stage_bytes));
   // G staging: one 4 KiB strip (32 rows x 64 columns fp16, 128-byte swizzle) per epilogue warp.  A strip is written
@@ -547,7 +558,8 @@ dsoft_fwd_kernel(const __grid_constant__ TileMaps maps, const __grid_constant__ 
   // the register hand-over sits INSIDE the role branches: ptxas budgets the code dominated by a setmaxnreg with
   // its value (placed before the branch it compiled the whole kernel, epilogues included, for 56 registers)
   if (warp < EPI_WARP0) {
-  if constexpr (kSoftMode && !kRanks) setmaxnreg_dec<40>();  // the ranks epilogue fits the even split: no spills
+  // the ranks and distill epilogues fit the even split (168 registers): no hand-over, no spills
+  if constexpr (kSoftMode && !kRanks && !kDist) setmaxnreg_dec<40>();
   if (warp == 0) {
     // ------------------------------------------------------------------ TMA producer (warp-uniform loop)
     int stage = 0;
@@ -578,11 +590,11 @@ dsoft_fwd_kernel(const __grid_constant__ TileMaps maps, const __grid_constant__ 
         mbar_wait(smem_u32(&col_empty[cb]), ((static_cast<uint32_t>(n / COL_BUFS)) & 1) ^ 1);
         if (elect_one()) {
           const uint32_t full = smem_u32(&col_full[cb]);
-          const int nvec = (kWce || kPairs || kRanks) ? P.ncolvec : (MODE == MODE_SOFT_G ? 2 : 1) * P.nprod;
+          const int nvec = (kWce || kPairs || kRanks || kDist) ? P.ncolvec : (MODE == MODE_SOFT_G ? 2 : 1) * P.nprod;
           mbar_arrive_expect_tx(full, nvec * CT * 4);
           float* dst = colbuf + cb * COL_VECS * CT;
           const size_t c0 = static_cast<size_t>(gcol(t));  // CT == bn == 256 in the soft modes
-          if constexpr (kWce || kPairs || kRanks) {
+          if constexpr (kWce || kPairs || kRanks || kDist) {
             for (int k = 0; k < P.ncolvec; ++k) bulk_copy_g2s(smem_u32(dst + k * CT), P.colvec[k] + c0, CT * 4, full);
           } else {
             for (int p = 0; p < P.nprod; ++p) {
@@ -659,7 +671,7 @@ dsoft_fwd_kernel(const __grid_constant__ TileMaps maps, const __grid_constant__ 
   }
   } else {
     // ------------------------------------------------------------------ epilogue
-    if constexpr (kSoftMode && !kRanks) setmaxnreg_inc<232>();
+    if constexpr (kSoftMode && !kRanks && !kDist) setmaxnreg_inc<232>();
     const int q = warp & 3;
     const int half = (warp - EPI_WARP0) >> 2;
     const int row = q * 32 + lane;
@@ -1674,6 +1686,166 @@ dsoft_fwd_kernel(const __grid_constant__ TileMaps maps, const __grid_constant__ 
         } else {
 #pragma unroll
           for (int k = 0; k < 11; ++k) P.part[k * st + o] = acc[k];
+        }
+      }
+    } else if constexpr (kDist) {
+      // ---------------------------------------------------------------- DistillClipLoss (open_clip)
+      // Products per 256-column tile: [0] student logits x = s <row, col> (image rows x text columns, or text rows x
+      // image columns), [1] teacher logits t = s_t <row_t, col_t> of the same pairs; both in log2 units.  The rows are
+      // this rank's block [row0, row0 + b), the columns all B; the diagonal of local row li is column row0 + li.
+      // Both TMEM slots of a tile are read chunk by chunk side by side (holding the student strip in registers while
+      // the teacher tile arrives, as the weighted-CE modes do, does not fit the register budget without spills).
+      //   FWD: per row, with online maxima (neither diagonal bounds its row): student m, sum 2^(x-m), sum 2^(x-m) (x-m);
+      //        teacher m_t, sum 2^(t-m_t) and sum 2^(t-m_t) (x-m) (relative to the CURRENT student maximum, so that
+      //        the distill term comes out as a difference of small numbers) -> part[6][npart][b]; the raw diagonal dot
+      //        products -> diag[0 / 1][b] (student / teacher).
+      //   G  : (2b gk) dL/dx off the diagonal, without the diagonal's one-hot term (applied in fp32 afterwards):
+      //          a_c (p_r + p_c) + a_d ((p_r - q_r) + (p_c - q_c)),   a_c = g_c gk, a_d = g_d gk
+      //        p_r / q_r from this row's student / teacher lse (wrow[0 / 1]), p_c / q_c from the column's (the other
+      //        direction's row statistics by global column, colvec[0 / 1]); row_only drops the column side.
+      const int lic = min(li, P.b - 1);
+      const float s2 = P.scal[SC_SCALE_L2], st2 = P.scal[SC_DST_TSCALE_L2];
+      const bool real_block = rb * BM < P.b;
+      const bool live_row = li < P.b;
+      float ms = M_FLOOR, ss = 0.f, ps = 0.f, mt = M_FLOOR, stt = 0.f, qa = 0.f, dgx = 0.f, dgt = 0.f;
+      bool have_dg = false;
+      float lse_r = 0.f, lset_r = 0.f, ac = 0.f, ad = 0.f;
+      if constexpr (MODE == MODE_DIST_G) {
+        lse_r = P.wrow[0][lic];
+        lset_r = P.wrow[1][lic];
+        ac = P.scal[SC_DST_GC];
+        ad = P.scal[SC_DST_GD];
+      }
+      int it = 0;
+      for (int t = t0; t < t1; ++t, it += 2) {
+        const int jt0 = t * CT + half * 128;
+        const int cb = (t - t0) % COL_BUFS;
+        mbar_wait(smem_u32(&col_full[cb]), static_cast<uint32_t>((t - t0) / COL_BUFS) & 1);
+        const float* cv = colbuf + cb * COL_VECS * CT + half * 128;
+        const int slot_x = it % 2, slot_t = (it + 1) % 2;
+        mbar_wait(smem_u32(&s_full[slot_x]), static_cast<uint32_t>(it / 2) & 1);
+        mbar_wait(smem_u32(&s_full[slot_t]), static_cast<uint32_t>((it + 1) / 2) & 1);
+        tc_fence_after();
+#pragma unroll 1
+        for (int c = 0; c < 4; ++c) {
+          const int jrel0 = jt0 + c * 32;
+          uint32_t rX[32], rT[32];
+          tmem_ld32_nowait(lane_addr + slot_x * CT + half * 128 + c * 32, rX);
+          tmem_ld32_nowait(lane_addr + slot_t * CT + half * 128 + c * 32, rT);
+          tmem_ld_wait(rX);
+          tmem_ld_wait(rT);
+          if (c == 3) {
+            tc_fence_before();
+            release_slot(slot_x);
+            release_slot(slot_t);
+          }
+          const bool has_diag = gw0 < jrel0 + 32 && jrel0 < gw0 + 32;  // warp-uniform
+          const bool ragged = jrel0 + 32 > P.ncols;
+          if constexpr (MODE == MODE_DIST_FWD) {
+            if (has_diag) {
+#pragma unroll
+              for (int e = 0; e < 32; ++e)
+                if (jrel0 + e == gi) {
+                  dgx = __uint_as_float(rX[e]);  // raw dot products: the finalize scales them as below
+                  dgt = __uint_as_float(rT[e]);
+                  have_dg = true;
+                }
+            }
+            float cm = NEG_BIG, cmt = NEG_BIG;
+#pragma unroll
+            for (int e = 0; e < 32; ++e) {
+              float x = __uint_as_float(rX[e]) * s2, tt = __uint_as_float(rT[e]) * st2;
+              if (ragged && jrel0 + e >= P.ncols) x = tt = NEG_BIG;
+              rX[e] = __float_as_uint(x);
+              rT[e] = __float_as_uint(tt);
+              cm = fmaxf(cm, x);
+              cmt = fmaxf(cmt, tt);
+            }
+            const float mnew = fmaxf(ms, cm);
+            const float dl = mnew - ms;
+            const float al = fast_exp2(-dl);
+            ps = al * fmaf(-dl, ss, ps);  // sum 2^(x-m) (x-m) relative to the new maximum
+            ss *= al;
+            qa = fmaf(-dl, stt, qa);      // sum 2^(t-m_t) (x-m): the student reference moves
+            ms = mnew;
+            const float mtn = fmaxf(mt, cmt);
+            const float alt = fast_exp2(mt - mtn);
+            stt *= alt;
+            qa *= alt;
+            mt = mtn;
+            float2 sacc = pk1(0.f), pacc = pk1(0.f), tacc = pk1(0.f), qacc = pk1(0.f);
+#pragma unroll
+            for (int e = 0; e < 32; e += 2) {
+              const float2 d = pk_add(pk(__uint_as_float(rX[e]), __uint_as_float(rX[e + 1])), pk1(-ms));
+              const float2 ex = pk_exp2(d);
+              const float2 w = pk_exp2(pk_add(pk(__uint_as_float(rT[e]), __uint_as_float(rT[e + 1])), pk1(-mt)));
+              sacc = pk_add(sacc, ex);
+              pacc = pk_fma(ex, d, pacc);
+              tacc = pk_add(tacc, w);
+              qacc = pk_fma(w, d, qacc);
+            }
+            ss += sacc.x + sacc.y;
+            ps += pacc.x + pacc.y;
+            stt += tacc.x + tacc.y;
+            qa += qacc.x + qacc.y;
+          } else {  // MODE_DIST_G
+            const float4* lsc = reinterpret_cast<const float4*>(cv + 0 * CT + c * 32);  // column's student lse
+            const float4* ltc = reinterpret_cast<const float4*>(cv + 1 * CT + c * 32);  // column's teacher lse
+            const bool need_mask = has_diag || ragged || !real_block || rb * BM + q * 32 + 32 > P.b;
+            uint32_t w16[16];
+#pragma unroll
+            for (int e4 = 0; e4 < 8; ++e4) {
+              float4 l4 = make_float4(0.f, 0.f, 0.f, 0.f), m4 = l4;
+              if (!P.row_only) {
+                l4 = lsc[e4];
+                m4 = ltc[e4];
+              }
+              const float lcol[4] = {l4.x, l4.y, l4.z, l4.w}, tcol[4] = {m4.x, m4.y, m4.z, m4.w};
+              float g4[4];
+#pragma unroll
+              for (int k = 0; k < 4; ++k) {
+                const int e = 4 * e4 + k;
+                const float x = __uint_as_float(rX[e]) * s2;
+                const float tt = __uint_as_float(rT[e]) * st2;
+                const float pr = fast_exp2(x - lse_r);
+                const float qr = fast_exp2(tt - lset_r);
+                float psum = pr, dpq = pr - qr;  // p - q formed in fp32
+                if (!P.row_only) {
+                  const float pc = fast_exp2(x - lcol[k]);
+                  const float qc = fast_exp2(tt - tcol[k]);
+                  psum += pc;
+                  dpq += pc - qc;
+                }
+                float g = fmaf(ac, psum, ad * dpq);
+                if (need_mask && ((jrel0 + e == gi) || (jrel0 + e >= P.ncols) || !live_row)) g = 0.f;
+                g4[k] = g;
+              }
+              w16[2 * e4 + 0] = pack_f16x2(g4[0], g4[1]);
+              w16[2 * e4 + 1] = pack_f16x2(g4[2], g4[3]);
+            }
+            if (real_block && jrel0 + 32 <= P.g_pitch) {
+              if ((c & 1) == 0) stage_begin();
+              stage_put32(w16, c & 1);
+              if (c & 1) stage_store(&maps.g[0], (rb * (P.g_pitch >> 6) + (jrel0 >> 6)) * BM + q * 32);
+            }
+          }
+        }
+        mbar_arrive(smem_u32(&col_empty[cb]));
+      }
+      if constexpr (MODE == MODE_DIST_G) {
+        if (lane == 0) bulk_wait_group<0>();  // the stores have landed before the CTA may exit
+      } else if (live_row) {
+        const int o = sp * P.b + li;
+        const int st = P.npart * P.b;
+        P.part[0 * st + o] = ms;
+        P.part[1 * st + o] = ss;
+        P.part[2 * st + o] = ps;
+        P.part[3 * st + o] = mt;
+        P.part[4 * st + o] = stt;
+        P.part[5 * st + o] = qa;
+        if (have_dg) {
+          P.diag[li] = dgx;
+          P.diag[P.b + li] = dgt;
         }
       }
     } else if constexpr (MODE == MODE_SOFT_SYM16) {

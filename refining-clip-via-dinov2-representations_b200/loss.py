@@ -803,13 +803,14 @@ class ClipLossWithDINOEnhancements(nn.Module):
         # the reference returns None when output_dict is False (loss.py:598-607) - preserved
 
 
-def install_into_open_clip(open_clip_module=None, siglip=False):
+def install_into_open_clip(open_clip_module=None, siglip=False, distill=False):
     """Make the reference's ``create_loss`` (factory.py:566-576) build this class.
 
     ``open_clip.factory`` imports the class by name at import time (factory.py:25-34), so both module
     attributes are patched; ``train.py`` needs no change.  ``siglip=True`` also patches every binding of
     ``SigLipLoss`` (the ``--siglip`` objective) with ``siglip.SigLipLoss``; off by default, so that existing callers
-    keep upstream's SigLIP loss."""
+    keep upstream's SigLIP loss.  ``distill=True`` likewise patches ``DistillClipLoss`` (the ``--distill`` objective)
+    with ``distill.DistillClipLoss``; off by default."""
     import importlib
 
     loss_mod = importlib.import_module("open_clip.loss") if open_clip_module is None else open_clip_module.loss
@@ -841,6 +842,17 @@ def install_into_open_clip(open_clip_module=None, siglip=False):
         train_mod = sys.modules.get("open_clip_train.train")
         if train_mod is not None and hasattr(train_mod, "SigLipLoss"):
             train_mod.SigLipLoss = SigLipLoss
+    if distill and hasattr(loss_mod, "DistillClipLoss"):
+        from .distill import DistillClipLoss
+        import sys
+
+        if not hasattr(loss_mod, "_reference_DistillClipLoss"):
+            loss_mod._reference_DistillClipLoss = loss_mod.DistillClipLoss
+        loss_mod.DistillClipLoss = DistillClipLoss
+        factory_mod.DistillClipLoss = DistillClipLoss
+        train_mod = sys.modules.get("open_clip_train.train")
+        if train_mod is not None and hasattr(train_mod, "DistillClipLoss"):
+            train_mod.DistillClipLoss = DistillClipLoss
     return ClipLossWithDINOEnhancements
 
 
@@ -872,4 +884,13 @@ def uninstall_from_open_clip(open_clip_module=None):
         train_mod = sys.modules.get("open_clip_train.train")
         if train_mod is not None and hasattr(train_mod, "SigLipLoss"):
             train_mod.SigLipLoss = sig
+    dcl = getattr(loss_mod, "_reference_DistillClipLoss", None)
+    if dcl is not None:
+        import sys
+
+        loss_mod.DistillClipLoss = dcl
+        factory_mod.DistillClipLoss = dcl
+        train_mod = sys.modules.get("open_clip_train.train")
+        if train_mod is not None and hasattr(train_mod, "DistillClipLoss"):
+            train_mod.DistillClipLoss = dcl
     return ref
