@@ -282,13 +282,6 @@ __device__ __forceinline__ void issue_s_stage(uint32_t tmem_d, uint32_t a_smem, 
   }
 }
 
-// 8 packed fp16 pairs -> one 32-byte evict-first store
-__device__ __forceinline__ void st_cs_v8(void* dst, const uint32_t (&w)[8]) {
-  asm volatile("st.global.cs.v8.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};" ::"l"(dst), "r"(w[0]), "r"(w[1]),
-               "r"(w[2]), "r"(w[3]), "r"(w[4]), "r"(w[5]), "r"(w[6]), "r"(w[7])
-               : "memory");
-}
-
 // Packed fp32 pairs (sm_100 FFMA2 / FMUL2 / FADD2: one issue slot and one pass through the FMA pipe for two lanes'
 // worth of work).  The epilogues are issue-bound (two epilogue warps per scheduler next to the MMA stream), so their
 // element loops are written over column PAIRS.
@@ -375,23 +368,6 @@ __device__ __forceinline__ float warp_colmax32(float (&x)[32], int lane) {
   return x[0];
 }
 
-// element (local row li, column j) of a blocked fp16 logit-gradient matrix: K tiles of 64 columns, each
-// (row block, K tile) = one 16 KiB TMA box of the gradient GEMM's A operand
-__device__ __forceinline__ size_t g_index(int li, int j, int pitch) {
-  return ((static_cast<size_t>(li >> 7) * (pitch >> 6) + (j >> 6)) * BM + (li & 127)) * 64 + (j & 63);
-}
-
-// 32 consecutive logit gradients of one row -> fp16 -> global memory as two 32-byte stores (full sectors),
-// evict-first: read back once by the gradient GEMM, must not displace the operands in L2
-__device__ __forceinline__ void store_g32(__half* dst, const float (&g)[32]) {
-#pragma unroll
-  for (int i = 0; i < 2; ++i) {
-    uint32_t w[8];
-#pragma unroll
-    for (int k = 0; k < 8; ++k) w[k] = pack_f16x2(g[16 * i + 2 * k], g[16 * i + 2 * k + 1]);
-    st_cs_v8(dst + 16 * i, w);
-  }
-}
 // SigLIP pair terms (MODE_SIGLIP).  z = s x + beta, l = +1 for the positive pair, -1 otherwise:
 //   loss = softplus(-l z) = max(-l z, 0) + log1p(e),  e = 2^(-|z| log2 e)  (the one MUFU op per pair)
 //   G = d loss / d z = -l sigma(-l z),  sigma(t) = r (t >= 0) or e r (t < 0),  r = 1 / (1 + e)
@@ -433,9 +409,9 @@ __device__ __forceinline__ float2 siglip_pair2(float2 z, bool pos_x, bool pos_y,
 //  MODE_CLIP partials (2): running max m (log2 units), sum 2^(x-m)        [+ diag dot product]
 //  MODE_SOFT partials (7): teacher m, Zt, Aq=sum w*q, Ap=sum w*p, Ar=sum w*r, student Zs, text Ztt
 //  (w = 2^(q-m); student/text use the fixed maximum log2(e)/tau, reached on the diagonal.)
-// CG = 2: the kernel runs as clusters of two CTAs (consecutive row blocks) that drive cta_group::2 MMAs
-// (M = 256): each CTA loads its own 128 rows of the row-side operand and HALF of the column-side tile, the
-// leader issues one MMA for both.
+// The kernel runs as clusters of two CTAs (consecutive row blocks) that drive cta_group::2 MMAs (M = 256): each
+// CTA loads its own 128 rows of the row-side operand and HALF of the column-side tile, the leader issues one MMA for
+// both.
 //
 // Tile width.  What bounds these kernels is the L2 -> SM operand stream (~6300 B/clk for the whole chip, i.e.
 // ~42 B/clk per SM): an M=256 x N=128 pair tile with a streamed row operand pulls 24 KiB per CTA per 64-deep K
@@ -452,9 +428,45 @@ __device__ __forceinline__ float2 siglip_pair2(float2 z, bool pos_x, bool pos_y,
 // MMA time.  It runs SIXTEEN epilogue warps (four per quadrant, 64-column strips, 640 threads per CTA, <= 96
 // registers) so that four warps per scheduler hide each other's latencies.  (Tried for MODE_CLIP_G as well, with
 // 32-column half-box G stores so that the staging strips still fit: 1.17 ms against 1.04 ms - dropped.)
-__host__ __device__ constexpr int fwd_epi_warps(int mode) {
-  return mode == MODE_CLIP_SYM ? 16 : 8;
+
+// Per-column vectors the producer stages per tile for the epilogue (bulk copies into shared memory, COL_BUFS tiles
+// deep, read as shared-memory broadcasts instead of dependent global loads per 32-column chunk)
+enum FwdCols {
+  COLS_NONE,
+  COLS_RINV,         // P.rinv[p] per product: inverse column norms
+  COLS_RINV_COLFAC,  // P.rinv[p] and P.colfac[p] (at vector 3 + p): the soft logit gradient
+  COLS_COLVEC        // P.colvec[0 .. ncolvec)
+};
+struct FwdMode {
+  int stages;     // operand ring depth in 32 KiB stages, with the column buffers (and the G strips) behind the ring;
+                  // 0: as deep as the shared memory allows (see the kernel)
+  int g_stage;    // the G staging strips start at g_stage * 32 KiB, behind the ring (modes that write G)
+  FwdCols cols;
+  bool writes_g;  // streams fp16 logit-gradient tiles through TMA stores (maps.g, L2 policies)
+  bool regsplit;  // setmaxnreg hand-over (40 / 232) from the producer / MMA / allocator warps to the epilogue; the
+                  // ranks and distill epilogues fit the even split (168 registers) without spills
+  int epi_warps;
+};
+__host__ __device__ constexpr FwdMode fwd_mode(int mode) {
+  switch (mode) {
+    case MODE_SOFT:
+    case MODE_SOFT_SYM16: return {6, 6, COLS_RINV, false, true, 8};
+    case MODE_SOFT_G: return {5, 5, COLS_RINV_COLFAC, true, true, 8};
+    case MODE_WCE_STAT:
+    case MODE_WCE_LSE:
+    case MODE_WCE_DBG:
+    case MODE_PAIRS: return {6, 6, COLS_COLVEC, false, true, 8};
+    case MODE_WCE_G: return {5, 5, COLS_COLVEC, true, true, 8};
+    case MODE_RANKS:
+    case MODE_DIST_FWD: return {6, 6, COLS_COLVEC, false, false, 8};
+    case MODE_DIST_G: return {5, 5, COLS_COLVEC, true, false, 8};
+    case MODE_CLIP_G:
+    case MODE_SIGLIP: return {0, 6, COLS_NONE, true, false, 8};
+    case MODE_CLIP_SYM: return {0, 6, COLS_NONE, false, false, 16};
+    default: return {0, 6, COLS_NONE, false, false, 8};  // MODE_CLIP, MODE_RAW, MODE_LINEAR
+  }
 }
+__host__ __device__ constexpr int fwd_epi_warps(int mode) { return fwd_mode(mode).epi_warps; }
 __host__ __device__ constexpr int fwd_threads(int mode) { return 32 * (EPI_WARP0 + fwd_epi_warps(mode)); }
 
 template <int MODE, int CG>
@@ -462,45 +474,43 @@ __global__ void __launch_bounds__(fwd_threads(MODE), 1)
 dsoft_fwd_kernel(const __grid_constant__ TileMaps maps, const __grid_constant__ FwdParams P) {
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = align_1024(smem_raw);
-  constexpr int kEpiThreads = 32 * fwd_epi_warps(MODE);
+  static_assert(CG == 2, "the forward kernel runs as CTA pairs");
+  constexpr FwdMode kM = fwd_mode(MODE);
+  constexpr int kEpiThreads = 32 * kM.epi_warps;
+  // epilogue families (the shared part below reads only kM)
   constexpr bool kWce = (MODE >= MODE_WCE_STAT && MODE <= MODE_WCE_G);
-  // "soft-like": 256-column tiles with several products per tile, staged per-column vectors, setmaxnreg
-  constexpr bool kPairs = (MODE == MODE_PAIRS);  // two products per tile like the weighted-CE passes, no column vectors
-  constexpr bool kRanks = (MODE == MODE_RANKS);  // one product per tile, column vectors from P.colvec
-  constexpr bool kDist = (MODE == MODE_DIST_FWD || MODE == MODE_DIST_G);  // two products, column vectors from P.colvec
-  constexpr bool kSoftMode = (MODE == MODE_SOFT || MODE == MODE_SOFT_G || MODE == MODE_SOFT_SYM16 || kWce || kPairs ||
-                              kRanks || kDist);
-  static_assert(!kSoftMode || CG == 2, "the soft modes are written for CTA pairs");
+  constexpr bool kDist = (MODE == MODE_DIST_FWD || MODE == MODE_DIST_G);
   // streaming mode: stages of (A box | B boxes); resident mode: 8 A boxes, then B-only stages
   const bool resident = P.resident != 0;
   const int bn = P.bn;
-  const int brows = bn / CG;                 // column-operand rows this CTA stages per tile
-  const int boxr = (CG == 2) ? 64 : BM;      // rows per TMA box (maps are built accordingly)
+  const int brows = bn / CG;  // column-operand rows this CTA stages per tile
+  const int boxr = 64;        // rows per TMA box (maps are built accordingly)
   const int box_bytes = boxr * 128;
   const int stage_bytes = (resident ? 0 : TILE_BYTES) + brows * 128;
-  // soft modes: 6 stages of 32 KiB (logit-gradient mode: 5); the 32 KiB behind them hold the staged per-column
-  // vectors.  Logit-gradient modes keep 32 KiB (at 192 KiB; soft: at 160 KiB) for the G staging strips.
-  constexpr bool kClipG = (MODE == MODE_CLIP_G || MODE == MODE_SIGLIP);  // one product, G staging behind the ring
-  constexpr bool kGMode = (kClipG || MODE == MODE_SOFT_G || MODE == MODE_WCE_G || MODE == MODE_DIST_G);
-  constexpr bool kSoftG = (MODE == MODE_SOFT_G || MODE == MODE_WCE_G || MODE == MODE_DIST_G);
-  const int nstages = kSoftG ? 5 : (kSoftMode ? 6 :
-                      min(kClipG ? (resident ? 4 : 6) : 8, (resident ? 6 : 14) * TILE_BYTES / stage_bytes));
+  // Ring depth.  Modes with column vectors: 6 stages of 32 KiB with the staged vectors behind them (logit-gradient
+  // modes: 5 stages, the G staging strips right behind them).  The others: as many stages as fit (at most 8); the
+  // logit-gradient ones stop at the G staging strips (g_stage * 2 boxes of 16 KiB: streaming stages take two boxes,
+  // resident ones one box of the 256-column tile behind the 8 resident boxes).
+  static_assert(!kM.writes_g || kM.stages == 0 || kM.stages == kM.g_stage, "G strips right behind the ring");
+  const int nstages = kM.stages ? kM.stages
+                                : min(kM.writes_g ? (resident ? 2 * kM.g_stage - 8 : kM.g_stage) : 8,
+                                      (resident ? 6 : 14) * TILE_BYTES / stage_bytes);
   // G staging: one 4 KiB strip (32 rows x 64 columns fp16, 128-byte swizzle) per epilogue warp.  A strip is written
   // with conflict-free 16-byte shared stores and leaves through ONE TMA tensor store; per-thread 32-byte global
   // stores (32 different lines per warp instruction) kept the L1TEX pipe at 78 % and the tensor pipe at 62 %.
-  uint8_t* gstage = smem + (kSoftG ? 5 : 6) * 2 * TILE_BYTES;
+  uint8_t* gstage = smem + kM.g_stage * 2 * TILE_BYTES;
   const int nslots = TMEM_COLS / bn;  // 4 x 128 or 2 x 256 columns
   uint8_t* ring = resident ? smem + 8 * TILE_BYTES : smem;
   uint64_t* bars = reinterpret_cast<uint64_t*>(smem + F_STAGES * 2 * TILE_BYTES + 2 * TILE_BYTES);
-  uint64_t* ring_full = bars;        // [8]  (CG = 2: the leader's copy collects both CTAs' bytes)
+  uint64_t* ring_full = bars;        // [8]  (the leader's copy collects both CTAs' bytes)
   uint64_t* ring_empty = bars + 8;   // [8]
   uint64_t* s_full = bars + 16;
-  uint64_t* s_empty = s_full + F_SLOTS;  // (CG = 2: the leader's copy collects both CTAs' epilogues)
+  uint64_t* s_empty = s_full + F_SLOTS;  // (the leader's copy collects both CTAs' epilogues)
   uint64_t* a_full = s_empty + F_SLOTS;
   uint32_t* tmem_holder = reinterpret_cast<uint32_t*>(a_full + 1);
-  // soft modes: the per-column vectors of a tile (inverse norms; column soft-max factors in the G mode; 256
-  // columns each) are staged by the producer with bulk copies, COL_BUFS tiles deep.  The epilogue reads them as
-  // shared-memory broadcasts instead of dependent global loads per 32-column chunk.
+  // the per-column vectors of a tile (kM.cols; 256 columns each) are staged by the producer with bulk copies,
+  // COL_BUFS tiles deep.  The epilogue reads them as shared-memory broadcasts instead of dependent global loads per
+  // 32-column chunk.
   constexpr int COL_VECS = 6, COL_BUFS = 2, CT = 256;
   float* colbuf = reinterpret_cast<float*>(smem + 6 * 2 * TILE_BYTES);            // [COL_BUFS][COL_VECS][256]
   uint64_t* col_full = reinterpret_cast<uint64_t*>(colbuf + COL_BUFS * COL_VECS * CT);  // [COL_BUFS]
@@ -523,12 +533,12 @@ dsoft_fwd_kernel(const __grid_constant__ TileMaps maps, const __grid_constant__ 
   }
   // global column of the first column of (primed) tile t; without wrap the two coincide up to col0
   auto gcol = [&](int t) { return P.wrap ? (P.col0 + t * P.bn) % P.wrap : P.col0 + t * P.bn; };
-  const int prank = (CG == 2) ? (rb & 1) : 0;  // rank in the pair (== cluster rank)
+  const int prank = rb & 1;  // rank in the pair (== cluster rank)
   const bool leader = prank == 0;
 
   if (warp == 0 && lane == 0) {
     for (int i = 0; i < 4; ++i) tma_prefetch_desc(&maps.m[i]);
-    if constexpr (kGMode) {
+    if constexpr (kM.writes_g) {
       tma_prefetch_desc(&maps.g[0]);
       tma_prefetch_desc(&maps.g[1]);
     }
@@ -541,7 +551,7 @@ dsoft_fwd_kernel(const __grid_constant__ TileMaps maps, const __grid_constant__ 
       mbar_init(smem_u32(&s_empty[i]), CG * kEpiThreads);
     }
     mbar_init(smem_u32(a_full), 1);
-    if constexpr (kSoftMode) {
+    if constexpr (kM.cols != COLS_NONE) {
       for (int i = 0; i < COL_BUFS; ++i) {
         mbar_init(smem_u32(&col_full[i]), 1);
         mbar_init(smem_u32(&col_empty[i]), NUM_EPI_THREADS);
@@ -551,28 +561,24 @@ dsoft_fwd_kernel(const __grid_constant__ TileMaps maps, const __grid_constant__ 
   }
   if (warp == 2) tmem_alloc_cg<CG>(smem_u32(tmem_holder), TMEM_COLS);
   tc_fence_before();
-  if constexpr (CG == 2) cluster_sync_all(); else __syncthreads();
+  cluster_sync_all();
   tc_fence_after();
   const uint32_t tmem_base = *tmem_holder;
 
   // the register hand-over sits INSIDE the role branches: ptxas budgets the code dominated by a setmaxnreg with
   // its value (placed before the branch it compiled the whole kernel, epilogues included, for 56 registers)
   if (warp < EPI_WARP0) {
-  // the ranks and distill epilogues fit the even split (168 registers): no hand-over, no spills
-  if constexpr (kSoftMode && !kRanks && !kDist) setmaxnreg_dec<40>();
+  if constexpr (kM.regsplit) setmaxnreg_dec<40>();
   if (warp == 0) {
     // ------------------------------------------------------------------ TMA producer (warp-uniform loop)
     int stage = 0;
     uint32_t phase = 0;
     // logit-gradient modes: the operands must survive the G store stream in L2
-    const uint64_t pol_keep = kGMode ? l2_policy_evict_last() : 0ull;
+    const uint64_t pol_keep = kM.writes_g ? l2_policy_evict_last() : 0ull;
     auto load = [&](uint32_t dst, const CUtensorMap* m, uint32_t bar_local, int c0, int c1) {
-      if constexpr (CG == 2) {
-        if constexpr (kGMode) tma_load_2d_2sm_hint(dst, m, mapa_shared(bar_local, 0), c0, c1, pol_keep);
-        else tma_load_2d_2sm(dst, m, mapa_shared(bar_local, 0), c0, c1);
-      } else {
-        tma_load_2d(dst, m, bar_local, c0, c1);
-      }
+      // fwd_mode(MODE), not kM: nvcc rejects a member of the enclosing constexpr local in this lambda's if constexpr
+      if constexpr (fwd_mode(MODE).writes_g) tma_load_2d_2sm_hint(dst, m, mapa_shared(bar_local, 0), c0, c1, pol_keep);
+      else tma_load_2d_2sm(dst, m, mapa_shared(bar_local, 0), c0, c1);
     };
     if (resident && elect_one()) {
       const uint32_t af = smem_u32(a_full);
@@ -584,22 +590,22 @@ dsoft_fwd_kernel(const __grid_constant__ TileMaps maps, const __grid_constant__ 
     }
     __syncwarp();
     for (int t = t0; t < t1; ++t) {
-      if constexpr (kSoftMode) {
+      if constexpr (kM.cols != COLS_NONE) {
         const int n = t - t0;
         const int cb = n % COL_BUFS;
         mbar_wait(smem_u32(&col_empty[cb]), ((static_cast<uint32_t>(n / COL_BUFS)) & 1) ^ 1);
         if (elect_one()) {
           const uint32_t full = smem_u32(&col_full[cb]);
-          const int nvec = (kWce || kPairs || kRanks || kDist) ? P.ncolvec : (MODE == MODE_SOFT_G ? 2 : 1) * P.nprod;
+          const int nvec = kM.cols == COLS_COLVEC ? P.ncolvec : (kM.cols == COLS_RINV_COLFAC ? 2 : 1) * P.nprod;
           mbar_arrive_expect_tx(full, nvec * CT * 4);
           float* dst = colbuf + cb * COL_VECS * CT;
-          const size_t c0 = static_cast<size_t>(gcol(t));  // CT == bn == 256 in the soft modes
-          if constexpr (kWce || kPairs || kRanks || kDist) {
+          const size_t c0 = static_cast<size_t>(gcol(t));  // CT == bn == 256 in the modes with column vectors
+          if constexpr (kM.cols == COLS_COLVEC) {
             for (int k = 0; k < P.ncolvec; ++k) bulk_copy_g2s(smem_u32(dst + k * CT), P.colvec[k] + c0, CT * 4, full);
           } else {
             for (int p = 0; p < P.nprod; ++p) {
               bulk_copy_g2s(smem_u32(dst + p * CT), P.rinv[p] + c0, CT * 4, full);
-              if constexpr (MODE == MODE_SOFT_G)
+              if constexpr (kM.cols == COLS_RINV_COLFAC)
                 bulk_copy_g2s(smem_u32(dst + (3 + p) * CT), P.colfac[p] + c0, CT * 4, full);
             }
           }
@@ -671,7 +677,7 @@ dsoft_fwd_kernel(const __grid_constant__ TileMaps maps, const __grid_constant__ 
   }
   } else {
     // ------------------------------------------------------------------ epilogue
-    if constexpr (kSoftMode && !kRanks && !kDist) setmaxnreg_inc<232>();
+    if constexpr (kM.regsplit) setmaxnreg_inc<232>();
     const int q = warp & 3;
     const int half = (warp - EPI_WARP0) >> 2;
     const int row = q * 32 + lane;
@@ -683,7 +689,7 @@ dsoft_fwd_kernel(const __grid_constant__ TileMaps maps, const __grid_constant__ 
     float v[32];
     // ---- G staging (logit-gradient modes): this warp's strip, its swizzled row, and the TMA store of a finished
     // 64-column box.  Strip reuse: the issuing lane waits until its previous store has read the strip.
-    const uint64_t pol_stream = kGMode ? l2_policy_evict_first() : 0ull;  // G tiles: written once, read once later
+    const uint64_t pol_stream = kM.writes_g ? l2_policy_evict_first() : 0ull;  // G tiles: written once, read once later
     const uint32_t gs_base = smem_u32(gstage) + static_cast<uint32_t>(warp - EPI_WARP0) * 4096u;
     const uint32_t gs_row = gs_base + static_cast<uint32_t>(lane) * 128u;
     const int gsw = lane & 7;
@@ -706,15 +712,11 @@ dsoft_fwd_kernel(const __grid_constant__ TileMaps maps, const __grid_constant__ 
       }
     };
     auto release_slot = [&](int slot) {  // the MMA issuer lives in the pair's leader
-      if constexpr (CG == 2) {
-        // relaxed: a .release arrive is a MEMBAR that waits for every earlier memory operation of the thread
-        // (ncu: "membar" was the top stall of the soft epilogue, and with the G stores in flight it serialised
-        // the G kernels).  The barrier only hands back TMEM, whose reads are complete (tcgen05.wait::ld) and
-        // ordered by fence::before_thread_sync.
-        mbar_arrive_cluster_relaxed(mapa_shared(smem_u32(&s_empty[slot]), 0));
-      } else {
-        mbar_arrive(smem_u32(&s_empty[slot]));
-      }
+      // relaxed: a .release arrive is a MEMBAR that waits for every earlier memory operation of the thread (ncu:
+      // "membar" was the top stall of the soft epilogue, and with the G stores in flight it serialised the G
+      // kernels).  The barrier only hands back TMEM, whose reads are complete (tcgen05.wait::ld) and ordered by
+      // fence::before_thread_sync.
+      mbar_arrive_cluster_relaxed(mapa_shared(smem_u32(&s_empty[slot]), 0));
     };
 
     if constexpr (MODE == MODE_RAW) {
@@ -791,7 +793,7 @@ dsoft_fwd_kernel(const __grid_constant__ TileMaps maps, const __grid_constant__ 
         P.part[(1 * P.npart + sp) * P.b + li] = sum;
         if (have_dg && P.diag) P.diag[li] = dg;
       }
-    } else if constexpr (kPairs) {
+    } else if constexpr (MODE == MODE_PAIRS) {
       // ---------------------------------------------------------------- CLIP-blind pair statistics
       // helpers.py:221-285 (_pair_stats): cs = Z Z^T, ds = D D^T for L2-normalised rows, over the pairs i < j:
       // how many have cs >= cmin, how many of those have ds <= dmax ("blind": CLIP calls them similar, DINOv2 does
@@ -886,7 +888,7 @@ dsoft_fwd_kernel(const __grid_constant__ TileMaps maps, const __grid_constant__ 
           }
         }
       }
-    } else if constexpr (kRanks) {
+    } else if constexpr (MODE == MODE_RANKS) {
       // ---------------------------------------------------------------- retrieval ranks
       // open_clip get_clip_metrics as counts over s = I . T^T (rows = images, columns = captions): a pair (i, j) is
       // the positive when t(j) == i (1:1: the diagonal, warp-uniform per 32 x 32 chunk); every other pair counts
@@ -2143,7 +2145,7 @@ dsoft_fwd_kernel(const __grid_constant__ TileMaps maps, const __grid_constant__ 
   }
 
   tc_fence_before();
-  if constexpr (CG == 2) cluster_sync_all(); else __syncthreads();
+  cluster_sync_all();
   if (warp == 2) tmem_dealloc_cg<CG>(tmem_base, TMEM_COLS);
 }
 

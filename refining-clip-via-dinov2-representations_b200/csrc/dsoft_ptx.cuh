@@ -113,18 +113,6 @@ __device__ __forceinline__ void tma_load_2d(uint32_t smem_dst, const CUtensorMap
       : "memory");
 }
 
-// Multicast variant: the box is written to the same shared-memory offset of every CTA in `cta_mask`
-// and complete_tx is signalled on the mbarrier at the same offset in each of them.
-__device__ __forceinline__ void tma_load_2d_mc(uint32_t smem_dst, const CUtensorMap* map, uint32_t bar,
-                                               int32_t c0, int32_t c1, uint16_t cta_mask) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster"
-      " [%0], [%1, {%3, %4}], [%2], %5;"
-      :
-      : "r"(smem_dst), "l"(reinterpret_cast<uint64_t>(map)), "r"(bar), "r"(c0), "r"(c1), "h"(cta_mask)
-      : "memory");
-}
-
 // ----------------------------------------------------------------------------------------------
 // Thread-block cluster
 // ----------------------------------------------------------------------------------------------
@@ -310,14 +298,10 @@ __device__ __forceinline__ void tma_load_2d_2sm(uint32_t smem_dst, const CUtenso
       : "r"(smem_dst), "l"(reinterpret_cast<uint64_t>(map)), "r"(bar_cluster), "r"(c0), "r"(c1)
       : "memory");
 }
-// arrive on an mbarrier of another CTA of the cluster (address from mapa_shared)
-__device__ __forceinline__ void mbar_arrive_cluster(uint32_t bar_cluster) {
-  asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(bar_cluster) : "memory");
-}
-
-// Same without release semantics: a .release arrive waits until every earlier global store of the thread has
-// been performed at cluster scope (MEMBAR), which stalls an epilogue that streams tiles to HBM.  Valid when the
-// barrier only hands back TMEM (reads completed by tcgen05.wait::ld + fence::before_thread_sync), not memory.
+// Arrive on an mbarrier of another CTA of the cluster (address from mapa_shared) without release semantics: a
+// .release arrive waits until every earlier global store of the thread has been performed at cluster scope (MEMBAR),
+// which stalls an epilogue that streams tiles to HBM.  Valid when the barrier only hands back TMEM (reads completed
+// by tcgen05.wait::ld + fence::before_thread_sync), not memory.
 __device__ __forceinline__ void mbar_arrive_cluster_relaxed(uint32_t bar_cluster) {
   asm volatile("mbarrier.arrive.relaxed.cluster.shared::cluster.b64 _, [%0];" ::"r"(bar_cluster) : "memory");
 }
@@ -427,12 +411,6 @@ __device__ __forceinline__ void tma_store_2d_hint(const CUtensorMap* map, uint32
                : "memory");
 }
 
-// TMA tensor store: one swizzled shared-memory box -> global memory (bulk async group of the issuing thread)
-__device__ __forceinline__ void tma_store_2d(const CUtensorMap* map, uint32_t smem_src, int c0, int c1) {
-  asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group [%0, {%2, %3}], [%1];"
-               :: "l"(reinterpret_cast<uint64_t>(map)), "r"(smem_src), "r"(c0), "r"(c1)
-               : "memory");
-}
 __device__ __forceinline__ void bulk_commit_group() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
 // all but the N most recent bulk groups of this thread have finished READING their shared-memory source
 template <int N>
@@ -482,12 +460,6 @@ __device__ __forceinline__ float warp_min_f32(float x) {
   float r;
   asm volatile("redux.sync.min.f32 %0, %1, 0xffffffff;" : "=f"(r) : "f"(x));
   return r;
-}
-
-__device__ __forceinline__ float fast_log2(float x) {
-  float y;
-  asm("lg2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
-  return y;
 }
 
 // two fp32 -> packed bf16x2 (lo = first argument), round-to-nearest-even
