@@ -27,7 +27,8 @@ extern "C" {
 
 #define DSOFT_VERSION 260 /* 0.2.6: SigLIP loss (DSOFT_F_SIGLIP, dsoft_siglip_*), later extended without a number
                              change by DistillClipLoss (DSOFT_F_DISTILL, dsoft_distill_*: additions only, nothing
-                             existing changed); 0.2.5: retrieval ranks
+                             existing changed) and by kNN top-k (dsoft_knn_scratch_bytes, dsoft_knn_topk:
+                             additions only); 0.2.5: retrieval ranks
                              (dsoft_retrieval_ranks); 0.2.4: weighted plans accept the fused
                              backward (no DSOFT_F_GMAT); 0.2.3: weighted
                              CE branch at world > 1 (phases 5 / 6, dsoft_plan_lse_rows, dsoft_plan_wsigma_info) */
@@ -220,6 +221,24 @@ size_t dsoft_retrieval_scratch_bytes(int32_t n_img, int32_t n_txt);
 int dsoft_retrieval_ranks(const void* img_dev, const void* txt_dev, int32_t k, int32_t n_img, int32_t n_txt,
                           const int32_t* text_image_dev, int32_t* rank_img_dev, int32_t* rank_txt_dev,
                           void* scratch_dev, void* stream);
+
+/* kNN top-k (the neighbour search of DINO's knn_classifier) without the [n_q x n_k] score matrix.
+ *   s_ij = <q_i, k_j> * key_scale_dev[j] * query_scale_dev[i]   (bf16 operands [n][width] row-major, fp32
+ *   accumulation; a NULL scale is 1; pass 1/||k_j|| and 1/||q_i|| for cosine scores, so that the operands are never
+ *   re-rounded after a normalisation)
+ * values_dev [n_q][k] fp32 / indices_dev [n_q][k] int32: row i holds the k largest s_ij over j < n_k by decreasing
+ * value, equal values by increasing key index (stable and deterministic).  Exact for any key order: the tile pass keeps
+ * the best 32 (k <= 32) or 64 keys of every 128-column strip of every column split per query, and a merge selects the
+ * top-k of those lists.  Both scales are applied before any comparison, so the order is that of the returned values.
+ * Pass split operands q = [hi | lo | hi], k = [hi | hi | lo] (width = 3 d) for fp32 features, as for
+ * dsoft_retrieval_ranks.  1 <= k <= 64 and k <= n_k (else DSOFT_EINVAL); operands and scratch 16-byte aligned, width
+ * a multiple of 8; the scales hold n_k and n_q fp32 (any alignment).  scratch_dev holds
+ * dsoft_knn_scratch_bytes(n_q, n_k, k) bytes for the current device, O(n_q k + n_k) (0: invalid arguments or no
+ * sm_100 device).  Asynchronous on `stream`, no host synchronisation (graph-capturable). */
+size_t dsoft_knn_scratch_bytes(int32_t n_q, int32_t n_k, int32_t k);
+int dsoft_knn_topk(const void* q_dev, const void* k_dev, int32_t width, int32_t n_q, int32_t n_k, int32_t k,
+                   const float* key_scale_dev, const float* query_scale_dev, float* values_dev, int32_t* indices_dev,
+                   void* scratch_dev, void* stream);
 
 /* SigLIP sigmoid loss of a DSOFT_F_SIGLIP plan (open_clip SigLipLoss).  z_ij = s <I_i, T_j> + beta over the bf16
  * image | text columns of `gathered` (fp32 accumulation, s and beta applied in fp32), l_ij = +1 for j == i (global

@@ -11,6 +11,8 @@ Import as ``dinosoft_b200`` (see the shim at the repo root).  Contents:
     graphed.py   CUDA-graph capture of the loss forward + backward (launch-bound small batches)
     pair_stats.py  CLIP-blind pair statistics on the Gram-tile kernel (helpers.py:221-285, SURVEY 8f-4)
     retrieval.py  retrieval ranks and R@K (open_clip get_clip_metrics) on the Gram-tile kernel, no N x N logits
+    knn.py       kNN top-k neighbours and DINO's weighted kNN classifier on the Gram-tile kernel: per-strip top-k
+                 lists in registers + a merge, no N_query x N_key score matrix
     siglip.py    SigLipLoss drop-in (open_clip SigLipLoss): sigmoid loss and its logit gradient in one tile pass,
                  backward = the two gradient GEMMs, no B x B logit matrix
     distill.py   DistillClipLoss drop-in (open_clip DistillClipLoss): student and teacher row statistics in the
@@ -26,6 +28,7 @@ from .cyclip import CyCLIPLoss
 from .graphed import make_graphed
 from .pair_stats import pair_stats
 from .retrieval import clip_metrics, retrieval_ranks
+from .knn import knn_classify, knn_topk
 from .siglip import SigLipLoss
 from .distill import DistillClipLoss
 from .loss import (
@@ -53,6 +56,8 @@ __all__ = [
     "pair_stats",
     "retrieval_ranks",
     "clip_metrics",
+    "knn_topk",
+    "knn_classify",
     "CyCLIPLoss",
     "SigLipLoss",
     "DistillClipLoss",

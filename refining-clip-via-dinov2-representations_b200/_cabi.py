@@ -63,6 +63,9 @@ PROTOTYPES = {
     "dsoft_retrieval_scratch_bytes": (C.c_size_t, [C.c_int32, C.c_int32]),
     "dsoft_retrieval_ranks": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_void_p,
                                         C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "dsoft_knn_scratch_bytes": (C.c_size_t, [C.c_int32, C.c_int32, C.c_int32]),
+    "dsoft_knn_topk": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_void_p,
+                                 C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "dsoft_siglip_g_bytes": (C.c_size_t, [C.c_void_p]),
     "dsoft_siglip_forward": (C.c_int, [C.c_void_p] * 9),
     "dsoft_siglip_backward": (C.c_int, [C.c_void_p] * 11),

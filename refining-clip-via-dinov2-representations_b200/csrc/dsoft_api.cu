@@ -2410,6 +2410,163 @@ extern "C" int dsoft_retrieval_ranks(const void* img, const void* txt, int32_t k
   return launch_fwd_pair(dsoft_fwd_kernel<MODE_RANKS, 2>, rbs, sp.nsplit, st, tm, P);
 }
 
+// ------------------------------------------------------------------------------------------------
+// kNN top-k (DINO's knn_classifier) on the Gram-tile kernel: MODE_TOPK keeps, per query, the KL best keys of each
+// 128-column strip of each column split in registers (KL = 32 for k <= 32, else 64); knn_merge_kernel selects the
+// top-k of those 2 nsplit sorted lists.  Nothing of size n_q x n_k exists.
+// Scratch: key scale [n_k padded to 256] fp32 | partial scores [2 nsplit][n_q][KL] fp32 | their key indices int32
+// ------------------------------------------------------------------------------------------------
+static int knn_list(int k) { return k <= 32 ? 32 : 64; }
+static bool knn_args_ok(int n_q, int n_k, int k) { return n_q > 0 && n_k > 0 && k >= 1 && k <= 64 && k <= n_k; }
+static SplitPlan knn_split(int n_q, int n_k, int sms) {
+  return choose_split(ceil_div(n_q, BM), 1, ceil_div(n_k, 2 * BN), sms);
+}
+static size_t knn_list_elems(int n_q, int k, const SplitPlan& sp) {
+  return static_cast<size_t>(2 * sp.nsplit) * static_cast<size_t>(n_q) * knn_list(k);
+}
+
+extern "C" size_t dsoft_knn_scratch_bytes(int32_t n_q, int32_t n_k, int32_t k) {
+  if (!knn_args_ok(n_q, n_k, k)) return 0;
+  int sms = 0;
+  if (query_num_sms(&sms)) return 0;
+  return 4 * rk_cols(n_k) + 8 * knn_list_elems(n_q, k, knn_split(n_q, n_k, sms));
+}
+
+// the key scale padded to whole tiles (1 where none is given; columns past n_k never enter a list)
+__global__ void knn_scale_kernel(const float* __restrict__ in, int n_k, int ncols_pad, float* __restrict__ out) {
+  for (int j = blockIdx.x * blockDim.x + threadIdx.x; j < ncols_pad; j += gridDim.x * blockDim.x)
+    out[j] = (in && j < n_k) ? in[j] : 1.f;
+}
+
+// one warp per query: k steps of a merge of the 2 nsplit partial lists (each sorted by decreasing score, ties by
+// increasing key index; a key lies in exactly one list).  Lane l holds the heads of lists l, l + 32, ..; per step the
+// warp reduces the lanes' best heads to the winner and its lane advances that list.
+template <int KL>
+__global__ void __launch_bounds__(256) knn_merge_kernel(const float* __restrict__ pv, const int* __restrict__ pi,
+                                                        int nlists, int n_q, int k, float* __restrict__ out_v,
+                                                        int* __restrict__ out_i) {
+  constexpr int R = 4;  // lists per lane: nlists = 2 nsplit <= 128
+  const int q = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  const int lane = threadIdx.x & 31;
+  if (q >= n_q) return;
+  const float neg_inf = __int_as_float(static_cast<int>(0xff800000u));
+  auto better = [](float a, int ai, float b, int bi) { return a > b || (a == b && ai < bi); };
+  int pos[R] = {0, 0, 0, 0};
+  float hv[R];
+  int hi[R];
+  auto head = [&](int r) {
+    const int l = lane + 32 * r;
+    if (l < nlists && pos[r] < KL) {
+      const size_t o = (static_cast<size_t>(l) * n_q + q) * KL + pos[r];
+      hv[r] = pv[o];
+      hi[r] = pi[o];
+    } else {
+      hv[r] = neg_inf;
+      hi[r] = 0x7fffffff;
+    }
+  };
+#pragma unroll
+  for (int r = 0; r < R; ++r) head(r);
+  for (int n = 0; n < k; ++n) {
+    float bv = hv[0];
+    int bi = hi[0], br = 0;
+#pragma unroll
+    for (int r = 1; r < R; ++r)
+      if (better(hv[r], hi[r], bv, bi)) {
+        bv = hv[r];
+        bi = hi[r];
+        br = r;
+      }
+    float wv = bv;
+    int wi = bi;
+#pragma unroll
+    for (int o = 16; o; o >>= 1) {
+      const float ov = __shfl_xor_sync(0xffffffffu, wv, o);
+      const int oi = __shfl_xor_sync(0xffffffffu, wi, o);
+      if (better(ov, oi, wv, wi)) {
+        wv = ov;
+        wi = oi;
+      }
+    }
+    if (lane == 0) {
+      out_v[static_cast<size_t>(q) * k + n] = wv;
+      out_i[static_cast<size_t>(q) * k + n] = wi;
+    }
+    if (bi == wi) {  // key indices are unique, so exactly one lane holds the winner
+#pragma unroll
+      for (int r = 0; r < R; ++r)
+        if (r == br) {
+          ++pos[r];
+          head(r);
+        }
+    }
+  }
+}
+
+template <int MODE>
+static int knn_launch(const TileMaps& tm, const FwdParams& P, int rbs, int nsplit, int n_q, int k, float* values,
+                      int32_t* indices, cudaStream_t st) {
+  int rc;
+  if ((rc = set_smem(dsoft_fwd_kernel<MODE, 2>, FWD_SMEM_BYTES))) return rc;
+  if ((rc = launch_fwd_pair(dsoft_fwd_kernel<MODE, 2>, rbs, nsplit, st, tm, P))) return rc;
+  knn_merge_kernel<topk_list(MODE)><<<ceil_div(n_q, 8), 256, 0, st>>>(P.tk_val, P.tk_idx, 2 * nsplit, n_q, k, values,
+                                                                      indices);
+  CUDA_TRY(cudaGetLastError());
+  return 0;
+}
+
+extern "C" int dsoft_knn_topk(const void* q_dev, const void* k_dev, int32_t width, int32_t n_q, int32_t n_k,
+                              int32_t k, const float* key_scale_dev, const float* query_scale_dev, float* values_dev,
+                              int32_t* indices_dev, void* scratch_dev, void* stream) {
+  if (!q_dev || !k_dev || !values_dev || !indices_dev || !scratch_dev) return fail(DSOFT_EINVAL, "null argument");
+  if (n_q <= 0 || n_k <= 0 || width <= 0 || width % 8)
+    return fail(DSOFT_EINVAL, "need n_q, n_k > 0 and a feature width that is a positive multiple of 8 "
+                              "(n_q=%d n_k=%d width=%d)", n_q, n_k, width);
+  if (!knn_args_ok(n_q, n_k, k)) return fail(DSOFT_EINVAL, "need 1 <= k <= 64 and k <= n_k (k=%d n_k=%d)", k, n_k);
+  for (const void* p : {q_dev, k_dev, static_cast<const void*>(scratch_dev)})
+    if (reinterpret_cast<uintptr_t>(p) % 16) return fail(DSOFT_EINVAL, "operands and scratch must be 16-byte aligned");
+  int sms = 0, rc = query_num_sms(&sms);
+  if (rc) return rc;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const SplitPlan sp = knn_split(n_q, n_k, sms);
+  const int ncols_pad = static_cast<int>(rk_cols(n_k));
+  float* kscale = static_cast<float*>(scratch_dev);
+  float* pv = kscale + ncols_pad;
+  int* pi = reinterpret_cast<int*>(pv + knn_list_elems(n_q, k, sp));
+  knn_scale_kernel<<<std::min(ceil_div(ncols_pad, 256), 4 * sms), 256, 0, st>>>(key_scale_dev, n_k, ncols_pad,
+                                                                                kscale);
+  CUDA_TRY(cudaGetLastError());
+
+  TileMaps tm;
+  const CUtensorMapDataType bf = CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
+  if ((rc = make_map(&tm.m[0], q_dev, n_q, width, static_cast<size_t>(width), bf, 64))) return rc;
+  if ((rc = make_map(&tm.m[1], k_dev, n_k, width, static_cast<size_t>(width), bf, 64))) return rc;
+  tm.m[2] = tm.m[3] = tm.g[0] = tm.g[1] = tm.m[0];
+  FwdParams P;
+  memset(&P, 0, sizeof(P));
+  P.nprod = 1;
+  P.a_map[0] = 0;
+  P.b_map[0] = 1;
+  P.kchunks[0] = ceil_div(width, BK);
+  P.bn = 2 * BN;
+  P.row0 = 0;
+  P.b = n_q;
+  P.col0 = 0;
+  P.ncols = n_k;
+  P.ntiles = ceil_div(n_k, 2 * BN);
+  P.tiles_per_split = sp.tps;
+  P.npart = 2 * sp.nsplit;
+  P.ncolvec = 1;
+  P.colvec[0] = kscale;
+  P.tk_qscale = query_scale_dev;
+  P.tk_val = pv;
+  P.tk_idx = pi;
+  const int rbs = ceil_div(n_q, BM);
+  if (knn_list(k) == 32)
+    return knn_launch<MODE_TOPK32>(tm, P, rbs, sp.nsplit, n_q, k, values_dev, indices_dev, st);
+  return knn_launch<MODE_TOPK>(tm, P, rbs, sp.nsplit, n_q, k, values_dev, indices_dev, st);
+}
+
 // phase 0: the whole forward; of a DSOFT_SYM_W plan: 4 = operand statistics, 1 = the soft part up to the column-sum
 // exchange, 3 = the CLIP part (independent of 1 and of the exchange), 2 = finalize; of a weighted plan: 5 = up to the
 // weighted row statistics (row stds), 6 = median onward

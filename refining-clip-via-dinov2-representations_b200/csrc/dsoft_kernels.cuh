@@ -68,6 +68,9 @@ constexpr int SIG_GK = 14;        // SigLIP G is stored as G * 2^14: |G| < 1, an
 constexpr int MODE_DIST_FWD = 16; // DistillClipLoss (open_clip): student and teacher row statistics of one direction
                                   // from two products per tile (student logits, teacher logits)
 constexpr int MODE_DIST_G = 17;   // DistillClipLoss logit gradient of one direction's rows, both directions' terms
+constexpr int MODE_TOPK = 18;     // kNN top-k (DINO knn_classifier): per query row and 128-column strip of a column
+constexpr int MODE_TOPK32 = 19;   // split, the 64 (MODE_TOPK32: 32) best (score, key index) in registers
+__host__ __device__ constexpr int topk_list(int mode) { return mode == MODE_TOPK32 ? 32 : 64; }
 
 // scalar block computed on device by prep_scalars_kernel (no host sync on logit_scale)
 enum {
@@ -191,6 +194,11 @@ struct FwdParams {
   int* rk_img;              // += #{j : t(j) != i, s_ij > p_i}   (caller-zeroed)
   int* rk_txt;              // += #{i : i != t(j), s_ij > s_t(j),j}
   int rk_mapped;            // 0: t(j) = j (the positives are the diagonal), 1: t(j) from colvec[1]
+  // ---- kNN top-k (MODE_TOPK, MODE_TOPK32): rows = queries (b = n_q), columns = keys (ncols = n_k); colvec[0] = the
+  // key scale (1/||k_j||, or 1), padded to whole tiles
+  const float* tk_qscale;   // per query: 1/||q_i||, or null (1)
+  float* tk_val;            // [npart][b][topk_list(MODE)] partial lists, by decreasing score (ties: increasing index)
+  int* tk_idx;              // their key indices (INT_MAX in slots no key filled)
 };
 
 struct BwdParams {
@@ -444,7 +452,7 @@ struct FwdMode {
   FwdCols cols;
   bool writes_g;  // streams fp16 logit-gradient tiles through TMA stores (maps.g, L2 policies)
   bool regsplit;  // setmaxnreg hand-over (40 / 232) from the producer / MMA / allocator warps to the epilogue; the
-                  // ranks and distill epilogues fit the even split (168 registers) without spills
+                  // ranks, distill and kNN epilogues fit the even split (168 registers) without spills
   int epi_warps;
 };
 __host__ __device__ constexpr FwdMode fwd_mode(int mode) {
@@ -458,6 +466,8 @@ __host__ __device__ constexpr FwdMode fwd_mode(int mode) {
     case MODE_PAIRS: return {6, 6, COLS_COLVEC, false, true, 8};
     case MODE_WCE_G: return {5, 5, COLS_COLVEC, true, true, 8};
     case MODE_RANKS:
+    case MODE_TOPK:
+    case MODE_TOPK32:
     case MODE_DIST_FWD: return {6, 6, COLS_COLVEC, false, false, 8};
     case MODE_DIST_G: return {5, 5, COLS_COLVEC, true, false, 8};
     case MODE_CLIP_G:
@@ -957,6 +967,92 @@ dsoft_fwd_kernel(const __grid_constant__ TileMaps maps, const __grid_constant__ 
         }
       }
       if (live_row && rcount) atomicAdd(P.rk_img + li, static_cast<int>(rcount));
+    } else if constexpr (MODE == MODE_TOPK || MODE == MODE_TOPK32) {
+      // ---------------------------------------------------------------- kNN top-k
+      // s_ij = <q_i, k_j> (rows = queries, columns = keys) times the staged key scale and this row's query scale.
+      // Each thread keeps the KL best (score, key index) of its row and 128-column strip in registers, sorted by
+      // decreasing score.  Keys reach a thread in increasing index order, so a score enters only when it is strictly
+      // above the list's last entry, and a listed equal score stays ahead of it: ties keep the smaller key index.
+      // One compare per score builds the chunk's survivor mask (usually empty once the list has filled).  A chunk
+      // with survivors is parked in this thread's slice of shared memory, which frees u[] for the insertion; each
+      // survivor is read back and inserted with static list indices only, so the list never leaves the registers.
+      // Chunks are CW columns wide, 16 for a 32-entry list and 8 for a 64-entry one: next to the 2 KL list registers,
+      // wider chunks do not fit the even register split (168) without spills.  Both scales are applied here, before
+      // any comparison, so that the lists and the merge order exactly the values that are returned.
+      constexpr int KL = topk_list(MODE);
+      constexpr int CW = KL == 64 ? 8 : 16;
+      float tv[KL], u[CW];
+      int ti[KL];
+#pragma unroll
+      for (int k = 0; k < KL; ++k) {
+        tv[k] = __int_as_float(static_cast<int>(0xff800000u));  // -inf: no score is below it
+        ti[k] = 0x7fffffff;
+      }
+      const float qs = (P.tk_qscale && li < P.b) ? P.tk_qscale[li] : 1.f;
+      // 256-column tiles: two TMEM slots and two column buffers, both picked by the parity of the tile's position
+      for (int t = t0; t < t1; ++t) {
+        const int n = t - t0, par = n & 1;
+        mbar_wait(smem_u32(&col_full[par]), static_cast<uint32_t>(n >> 1) & 1);
+        mbar_wait(smem_u32(&s_full[par]), static_cast<uint32_t>(n >> 1) & 1);
+        tc_fence_after();
+        const float* ks = colbuf + par * COL_VECS * CT + half * 128;
+        const uint32_t taddr = lane_addr + par * CT + half * 128;
+        const int gcol0 = t * CT + half * 128;
+#pragma unroll 1
+        for (int c = 0; c < 128 / CW; ++c) {
+          const int gj0 = gcol0 + c * CW;
+          if constexpr (CW == 16) tmem_ld16(taddr + c * CW, u);
+          else tmem_ld8(taddr + c * CW, u);
+          if (c == 128 / CW - 1) {
+            tc_fence_before();
+            release_slot(par);
+          }
+          if (gj0 >= P.ncols) continue;  // warp-uniform
+          const float lo = tv[KL - 1];
+          unsigned int m = 0;
+#pragma unroll
+          for (int e = 0; e < CW; ++e) {
+            u[e] = (u[e] * ks[c * CW + e]) * qs;
+            m |= (u[e] > lo) ? (1u << e) : 0u;
+          }
+          if (gj0 + CW > P.ncols) m &= (1u << (P.ncols - gj0)) - 1u;  // columns past n_k never enter
+          float* stash = reinterpret_cast<float*>(smem + 6 * 2 * TILE_BYTES + 16384)  // [256][CW], behind colbuf
+                         + (threadIdx.x - 32 * EPI_WARP0) * CW;
+          if (m) {
+#pragma unroll
+            for (int e = 0; e < CW; e += 4)
+              reinterpret_cast<float4*>(stash)[e / 4] = make_float4(u[e], u[e + 1], u[e + 2], u[e + 3]);
+          }
+          while (m) {
+            const int e = __ffs(m) - 1;
+            m &= m - 1u;
+            const float x = stash[e];
+            const int xj = gj0 + e;
+            // new[i] = old[i-1] if old[i-1] < x, else x if old[i] < x, else old[i] (a no-op when x <= old[KL-1])
+#pragma unroll
+            for (int i = KL - 1; i > 0; --i) {
+              const bool up = tv[i - 1] < x, here = tv[i] < x;
+              tv[i] = up ? tv[i - 1] : (here ? x : tv[i]);
+              ti[i] = up ? ti[i - 1] : (here ? xj : ti[i]);
+            }
+            if (tv[0] < x) {
+              tv[0] = x;
+              ti[0] = xj;
+            }
+          }
+        }
+        mbar_arrive(smem_u32(&col_empty[par]));
+      }
+      if (li < P.b) {
+        const size_t o = (static_cast<size_t>(sp) * P.b + li) * KL;
+        float4* dv = reinterpret_cast<float4*>(P.tk_val + o);
+        int4* di = reinterpret_cast<int4*>(P.tk_idx + o);
+#pragma unroll
+        for (int k = 0; k < KL / 4; ++k) {
+          dv[k] = make_float4(tv[4 * k], tv[4 * k + 1], tv[4 * k + 2], tv[4 * k + 3]);
+          di[k] = make_int4(ti[4 * k], ti[4 * k + 1], ti[4 * k + 2], ti[4 * k + 3]);
+        }
+      }
     } else if constexpr (MODE == MODE_LINEAR) {
       // ---------------------------------------------------------------- projection-head layer
       // Row operand = the samples (image rows of the packed buffer, or the hidden activations), column operand =

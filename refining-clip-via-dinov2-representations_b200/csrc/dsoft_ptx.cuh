@@ -333,6 +333,32 @@ __device__ __forceinline__ void tmem_ld32(uint32_t taddr, float (&v)[32]) {
   for (int i = 0; i < 32; ++i) v[i] = __uint_as_float(r[i]);
 }
 
+// Same for 16 and 8 consecutive columns (epilogues whose other live registers leave no room for 32).
+__device__ __forceinline__ void tmem_ld16(uint32_t taddr, float (&v)[16]) {
+  uint32_t r[16];
+  asm volatile(
+      "tcgen05.ld.sync.aligned.32x32b.x16.b32 "
+      "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
+      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]),
+        "=r"(r[8]), "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
+      : "r"(taddr)
+      : "memory");
+  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+#pragma unroll
+  for (int i = 0; i < 16; ++i) v[i] = __uint_as_float(r[i]);
+}
+
+__device__ __forceinline__ void tmem_ld8(uint32_t taddr, float (&v)[8]) {
+  uint32_t r[8];
+  asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];"
+               : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7])
+               : "r"(taddr)
+               : "memory");
+  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+#pragma unroll
+  for (int i = 0; i < 8; ++i) v[i] = __uint_as_float(r[i]);
+}
+
 // Split form for software pipelining: issue the load of the NEXT 32-column chunk, compute on the current one, and
 // only then wait.  tcgen05.wait::ld covers every earlier tcgen05.ld of the thread; the registers are passed through
 // the wait as in/out operands so that the compiler cannot move a consumer above it.
