@@ -1173,9 +1173,10 @@ __device__ __forceinline__ float4 load_bf16x4(const __nv_bfloat16* p) {
 // small residual), the coefficient of the CLIP part and the diagonal's share of d(logit_scale).
 //   classic:  dg = (p_it_aa - 1) + (p_ti_aa - 1); the matrix is unscaled, g_c s / (2b) is applied here; the row
 //             partials of d(logit_scale) include the diagonal's probabilities, hence the - 2 dot_aa
-//   weighted: the matrix already carries g_c and g_w and has no diagonal;
+//   weighted: the matrix already carries g_c gk and g_w gk and has no diagonal;
 //             dg = g_c [(p_it_aa - 1) + (p_ti_aa - 1)] + g_w [(p~_it_aa - 1 + beta A_a p_it_aa c_a) + text direction]
-//             (d CE~_a / d x_aa = p~_aa - 1 - beta A_a p_aa (r_aa - c_a) with r_aa = 0, loss.py:416-471)
+//             (d CE~_a / d x_aa = p~_aa - 1 - beta A_a p_aa (r_aa - c_a) with r_aa = 0, loss.py:416-471), taken
+//             times gk like the GEMM partials and the d(logit_scale) row partials; s / (2b gk) divides gk out
 struct ClipDiag { float dg_img, dg_txt, coefc, ds_diag; };
 __device__ __forceinline__ ClipDiag clip_diag(const FinBwdArgs& a, int i, float gc, float inv_b) {
   const float LN2 = 0.6931471805599453f;
@@ -1198,13 +1199,14 @@ __device__ __forceinline__ ClipDiag clip_diag(const FinBwdArgs& a, int i, float 
     const float g_txt = a.wsym ? expm1f(LN2 * (xd - wt[1 * a.Bcol + j])) +
                                      a.scal[SC_WBETA + 1] * wt[2 * a.Bcol + j] * (dm_ti + 1.f) * wt[0 * a.Bcol + j]
                                : dm_ti;
-    const float dg = gc * (dm_it + dm_ti) + gw * (g_img + g_txt);
+    const float gk = a.scal[SC_WCE_GK];
+    const float dg = (gc * (dm_it + dm_ti) + gw * (g_img + g_txt)) * gk;
     r.dg_img = r.dg_txt = dg;
     if (a.row_only) {  // world > 1, gathered columns detached: each direction's own row term only
-      r.dg_img = gc * dm_it + gw * g_img;
-      r.dg_txt = gc * dm_ti + gw * g_txt;
+      r.dg_img = (gc * dm_it + gw * g_img) * gk;
+      r.dg_txt = (gc * dm_ti + gw * g_txt) * gk;
     }
-    r.coefc = a.scal[SC_SCALE] * 0.5f * inv_b;
+    r.coefc = a.scal[SC_SCALE] * 0.5f * inv_b * a.scal[SC_WCE_IGK];
     r.ds_diag = dg * a.diag[i];
   }
   return r;
@@ -1333,7 +1335,8 @@ __global__ void __launch_bounds__(128) finalize_bwd_kernel(FinBwdArgs a) {
   if (last_block_done(a.ticket)) {
     __shared__ double sum1[1];
     block_reduce_rows(a.dsrow, gridDim.x, 1, sum1);
-    const float gc = a.weighted ? 1.f : a.gout[0] + a.lam_orig * a.gout[4];
+    // weighted: the row terms carry g_c, g_w and gk already
+    const float gc = a.weighted ? a.scal[SC_WCE_IGK] : a.gout[0] + a.lam_orig * a.gout[4];
     if (threadIdx.x == 0) a.d_scale[0] = static_cast<float>(sum1[0] * static_cast<double>(gc) * 0.5 / a.b);
   }
 }
@@ -1469,8 +1472,8 @@ __global__ void __launch_bounds__(256, 2) finalize_bwd_warp_kernel(FinBwdArgs a)
   if (last_block_done(a.ticket)) {
     __shared__ double sum1[1];
     block_reduce_rows(a.dsrow, gridDim.x, 1, sum1);
-    if (threadIdx.x == 0)
-      a.d_scale[0] = static_cast<float>(sum1[0] * static_cast<double>(a.weighted ? 1.f : gc) * 0.5 / a.b);
+    if (threadIdx.x == 0)  // weighted: the row terms carry g_c, g_w and gk already
+      a.d_scale[0] = static_cast<float>(sum1[0] * static_cast<double>(a.weighted ? a.scal[SC_WCE_IGK] : gc) * 0.5 / a.b);
   }
 }
 
@@ -2053,6 +2056,22 @@ __global__ void __launch_bounds__(1024) wce_final_kernel(WceFinalArgs a) {
   g[17] = static_cast<float>(ce_txt_mod);
   g[24] = a.rho;
   g[25] = a.cc;
+}
+
+// Backward scalar of the weighted CE branch: gk = 2^(14 - e) with |G| < 2^e, so that the fp16 logit gradient of
+// MODE_WCE_G / MODE_WCE_X holds G gk with |G gk| < 2^15 at any upstream gradient (a GradScaler's 2^16 and more) and
+// keeps its precision at small ones.  From wce_pair: e1, e2, p~ <= 1, A in [0, 1] and |r - c| <= 2, so
+// |G| <= 2 |g_c| + |g_w| (2 + 2 beta_img + 2 beta_txt), beta_txt only when the text direction is modulated.  e is
+// clamped only so that 1/gk, folded into the finalize's s / (2b gk), stays a normal fp32 number (gk <= 2^64).
+__global__ void wce_gscale_kernel(const float* __restrict__ gout, float lam_orig, float lam_w, int wsym,
+                                  float* __restrict__ scal) {
+  const float gc = gout[0] + lam_orig * gout[4], gw = gout[5] + lam_w * gout[4];
+  const float bsum = scal[SC_WBETA + 0] + (wsym ? scal[SC_WBETA + 1] : 0.f);
+  int e = 0;
+  frexpf(2.f * fabsf(gc) + fabsf(gw) * (2.f + 2.f * bsum), &e);
+  e = max(e, -50);
+  scal[SC_WCE_GK] = ldexpf(1.f, 14 - e);
+  scal[SC_WCE_IGK] = ldexpf(1.f, e - 14);
 }
 
 // world > 1, backward: c, lse~ and A of every rank's rows ([W][nr][b] rows 5 + 3 d + k, as all-gathered) -> the
@@ -3135,6 +3154,10 @@ static int backward_impl(const dsoft_plan_t* p, const void* gathered, const void
   if (p->weighted && p->sh.world > 1) {
     wce_relayout_kernel<<<ceil_div(3 * p->wnd * p->Bcol, 1024), 256, 0, st>>>(lse_all, p->sh.world, b, p->lse_rows,
                                                                              p->Bcol, p->wnd, S + p->st_wstat);
+    CUDA_TRY(cudaGetLastError());
+  }
+  if (p->weighted) {
+    wce_gscale_kernel<<<1, 1, 0, st>>>(gout, lambdas[0], lambdas[3], p->wsym, S + p->st_scal);
     CUDA_TRY(cudaGetLastError());
   }
   make_v16_kernel<<<ceil_div(p->B, 8), 256, 0, st>>>(

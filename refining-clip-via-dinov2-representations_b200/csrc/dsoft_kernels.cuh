@@ -85,6 +85,7 @@ enum {
   SC_RMIN_T = 8,    // min_j 1/||text_j||    (atomicMin by rinv_kernel; +inf until then)
   SC_RMIN_Z = 9,    // min_j 1/||student_j||
   SC_RMIN_D = 10,   // min_j 1/||dino_j||
+  SC_WCE_IGK = 11,  // weighted CE backward: 1/gk (SC_WCE_GK)
   SC_TICKET_F = 12, // (int) blocks of finalize_fwd_kernel that are done: the last one reduces the row losses
   SC_TICKET_B = 13, // (int) same for finalize_bwd_kernel
   SC_C_CLIP = 14,   // reference exponent c of the factorised CLIP logit gradients (lse_prepare_kernel)
@@ -102,6 +103,7 @@ enum {
   SC_DST_SPD = 28,  // sum over this rank's rows of both directions of (sum_j p x - x_ii), by the forward
   SC_DST_SPQ = 29,  // sum over the same rows of (sum_j p x - sum_j q x)
   SC_TICKET_DST = 30, // (int) DistillClipLoss forward finalize ticket
+  SC_WCE_GK = 31,   // weighted CE backward: gk, power-of-two scale of its fp16 logit gradient (wce_gscale_kernel)
   SC_COUNT = 32
 };
 
@@ -239,12 +241,13 @@ struct BwdParams {
 // e1 / gimg are the row side's classic / modulated terms, e2 / gtxt the column side's (the other direction's entry of
 // the same pair, statistics by column); x is the CLIP logit in log2 units, r the DINO dissimilarity.  The switches
 // (wrow_plain, wsym, wsplit, row_only) are read from the kernel parameters P (FwdParams or BwdParams) at each use, as
-// the kernel-parameter bank costs no registers.
+// the kernel-parameter bank costs no registers.  g_c and g_w arrive multiplied by gk = scal[SC_WCE_GK], so that g and
+// gr are the pair's entry times gk (|g gk| < 2^15 at any upstream gradient); the finalize kernel divides gk out.
 struct WceRowK {
   float lse, c, lset, aa;      // row side: lse, c_a, lse~, A_a
   float beta, beta2;           // row side: beta, beta log2(e)
   float beta_t, beta2_t;       // column side
-  float cc, gcl, gwt;          // c_clip, g_c, g_w
+  float cc, gcl, gwt;          // c_clip, g_c gk, g_w gk
 };
 struct WcePair { float g, gr; };
 template <class Params>
@@ -1569,9 +1572,10 @@ dsoft_fwd_kernel(const __grid_constant__ TileMaps maps, const __grid_constant__ 
       //   LSE  : log-sum-exp of x~ = x + beta clamp(r - c_a, +-c_clip) (diagonal unshifted, loss.py:445-447) and
       //          A_a = sum_{j != a} p~_aj [ |r_aj - c_a| <= c_clip ] (the share of the row that feels d c_a)
       //   DBG  : the row statistics behind the reference's diagnostics (loss.py:479-595)
-      //   G    : the fp16 logit gradient of  g_c * classic CE  +  g_w * weighted CE  for BOTH directions in one
-      //          matrix (rows = image, columns = text; the text direction's entry is the transposed one and reads
-      //          its row statistics per column):  d CE~_a / d x_ak = p~_ak - delta_ak - beta A_a p_ak (r_ak - c_a).
+      //   G    : the fp16 logit gradient of  g_c * classic CE  +  g_w * weighted CE, times gk (SC_WCE_GK), for
+      //          BOTH directions in one matrix (rows = image, columns = text; the text direction's entry is the
+      //          transposed one and reads its row statistics per column):
+      //          d CE~_a / d x_ak = p~_ak - delta_ak - beta A_a p_ak (r_ak - c_a).
       //          World > 1: one launch per direction (wdir = row side); the column side reads the other
       //          direction's all-gathered row statistics by global column, as MODE_CLIP_G does.
       const int lic = min(li, P.b - 1);
@@ -1602,8 +1606,8 @@ dsoft_fwd_kernel(const __grid_constant__ TileMaps maps, const __grid_constant__ 
         wk.beta_t = P.scal[SC_WBETA + 1 - P.wdir];
         wk.beta2_t = P.scal[SC_WBETA2 + 1 - P.wdir];
         wk.cc = cc;
-        wk.gcl = P.wgout[0] + P.wlam[0] * P.wgout[4];
-        wk.gwt = P.wgout[5] + P.wlam[1] * P.wgout[4];
+        wk.gcl = (P.wgout[0] + P.wlam[0] * P.wgout[4]) * P.scal[SC_WCE_GK];
+        wk.gwt = (P.wgout[5] + P.wlam[1] * P.wgout[4]) * P.scal[SC_WCE_GK];
       }
       int it = 0;
       for (int t = t0; t < t1; ++t, it += 2) {
@@ -1769,7 +1773,7 @@ dsoft_fwd_kernel(const __grid_constant__ TileMaps maps, const __grid_constant__ 
       }
       if constexpr (MODE == MODE_WCE_G) {
         if (lane == 0) bulk_wait_group<0>();
-        if (li < P.b) P.ds_part[sp * P.b + li] = acc[0] / s2;  // back to raw dot-product units
+        if (li < P.b) P.ds_part[sp * P.b + li] = acc[0] / s2;  // back to raw dot-product units (still times gk)
       } else if (li < P.b) {
         const int o = sp * P.b + li;
         const int st = P.npart * P.b;
@@ -2252,8 +2256,8 @@ dsoft_fwd_kernel(const __grid_constant__ TileMaps maps, const __grid_constant__ 
 //             -2 one-hot part and the s/(2b) factor are applied in fp32 by the finalize kernel)
 //  MODE_SOFT: G_aj = [(2^(p-ls_a) + 2^(p-ls_j)) - (2^(q-lt_a) + 2^(q-lt_j))] / (||y_j|| sigma), j != a
 //             (diagonal dropped: it is parallel to y_a and vanishes in the normalise backward)
-//  MODE_WCE_X: G_aj = the weighted CE entry of MODE_WCE_G (wce_pair) for the rows of one direction, from a CLIP
-//             tile and a DINO tile per column tile (diagonal dropped, applied in fp32 by the finalize kernel); one
+//  MODE_WCE_X: G_aj = the weighted CE entry of MODE_WCE_G (wce_pair, times gk) for the rows of one direction, from a
+//             CLIP tile and a DINO tile per column tile (diagonal dropped, applied in fp32 by the finalize kernel); one
 //             launch per direction, each with the row-side d(logit_scale) term only (wsplit), as MODE_CLIP
 //  row_only drops the *_j (column-side) terms: gathered features are constants (gather_with_grad=0).
 //  G is stored as fp16 (10-bit mantissa) and multiplied with an EXACT fp16 copy of the gradient operand
@@ -2516,8 +2520,8 @@ dsoft_bwd_kernel(const __grid_constant__ TileMaps maps, const __grid_constant__ 
       wk.beta_t = P.scal[SC_WBETA + 1 - P.wdir];
       wk.beta2_t = P.scal[SC_WBETA2 + 1 - P.wdir];
       wk.cc = P.wcc;
-      wk.gcl = P.wgout[0] + P.wlam[0] * P.wgout[4];
-      wk.gwt = P.wgout[5] + P.wlam[1] * P.wgout[4];
+      wk.gcl = (P.wgout[0] + P.wlam[0] * P.wgout[4]) * P.scal[SC_WCE_GK];
+      wk.gwt = (P.wgout[5] + P.wlam[1] * P.wgout[4]) * P.scal[SC_WCE_GK];
     }
 
     // 32 fp32 -> fp16, 4 x 16-byte swizzled stores into the K-major SW128 A-operand layout

@@ -24,8 +24,19 @@ LAMBDAS = (1.0, 0.5, 0.5, 0.0)  # lambda_original, lambda_soft, text_lambda, lam
 TEACHER_TEMP, TEXT_TEMP = 0.15, 0.02
 
 
-def oracle_ranks(oracle, img, txt, dino, student, scale, W, scope, gwg):
-    """Per-rank losses and gradients of the reference semantics (fp64), student given as a raw leaf tensor."""
+TERMS = ("classic_loss", "soft_img", "soft_txt", "soft_loss", "total_loss", "weighted_loss")  # order of gout / losses
+
+
+def seeded(terms, gout):
+    """sum_k gout[k] * term_k: what the backward of upstream gradients gout differentiates (None: total_loss)."""
+    if gout is None:
+        return terms["total_loss"]
+    return sum(float(g) * terms[k] for g, k in zip(gout, TERMS) if g != 0.0)
+
+
+def oracle_ranks(oracle, img, txt, dino, student, scale, W, scope, gwg, gout=None):
+    """Per-rank losses and gradients of the reference semantics (fp64), student given as a raw leaf tensor; the
+    gradients are those of sum_k gout[k] * term_k (default: of total_loss)."""
     cfg = oracle.OracleConfig(lambda_original=LAMBDAS[0], lambda_soft=LAMBDAS[1], soft_mode="kl_teacher",
                               teacher_temp=TEACHER_TEMP, soft_dino_to_text=True, text_lambda=LAMBDAS[2],
                               text_student_temp=TEXT_TEMP, world_size=W, local_loss=True, gather_with_grad=gwg,
@@ -47,8 +58,8 @@ def oracle_ranks(oracle, img, txt, dino, student, scale, W, scope, gwg):
         # logit_scale: each rank's own loss
         im, tx, sc, st = leafs()
         per = [oracle.rank_loss(im, tx, sc, dino.to(dt), st, cfg, rank=r) for r in range(W)]
-        g_sc = [torch.autograd.grad(p["total_loss"], sc, retain_graph=True)[0] for p in per]
-        sum(p["total_loss"] for p in per).backward()
+        g_sc = [torch.autograd.grad(seeded(p, gout), sc, retain_graph=True)[0] for p in per]
+        sum(seeded(p, gout) for p in per).backward()
         for r in range(W):
             rows = slice(r * b, (r + 1) * b)
             out.append(dict(terms=per[r], d_image=im.grad[rows], d_text=tx.grad[rows],
@@ -57,14 +68,15 @@ def oracle_ranks(oracle, img, txt, dino, student, scale, W, scope, gwg):
         for r in range(W):
             im, tx, sc, st = leafs()
             p = oracle.rank_loss(im, tx, sc, dino.to(dt), st, cfg, rank=r)
-            p["total_loss"].backward()
+            seeded(p, gout).backward()
             rows = slice(r * b, (r + 1) * b)
             out.append(dict(terms=p, d_image=im.grad[rows], d_text=tx.grad[rows],
                             d_student=None if st is None else st.grad[rows], d_scale=float(sc.grad)))
     return out
 
 
-def cuda_ranks(pkg, img, txt, dino, student, scale, W, scope, gwg, gmat):
+def cuda_ranks(pkg, img, txt, dino, student, scale, W, scope, gwg, gmat, gout=None):
+    """Every rank through the C ABI on cuda:0; gout: the six upstream gradients (default: d total_loss = 1)."""
     from dinosoft_b200 import _cabi
     from dinosoft_b200.loss import CudaBackend
 
@@ -98,7 +110,8 @@ def cuda_ranks(pkg, img, txt, dino, student, scale, W, scope, gwg, gmat):
         be.forward(pl, gathered, ls, LAMBDAS, st, sc, lse_all[r], lo)
         states.append(st)
         losses.append(lo)
-    gout = torch.tensor([0.0, 0.0, 0.0, 0.0, 1.0, 0.0], dtype=torch.float32, device=dev)  # d total_loss = 1
+    gout = torch.tensor([0.0, 0.0, 0.0, 0.0, 1.0, 0.0] if gout is None else list(gout), dtype=torch.float32,
+                        device=dev)
     out = []
     for r, pl in enumerate(plans):
         scratch = torch.empty(pl.scratch_numel, dtype=torch.float32, device=dev)

@@ -22,9 +22,10 @@ pytestmark = pytest.mark.gpu
 PAIR_RTOL = 5e-4
 
 
-def cuda_ranks(img, txt, dino, student, scale, W, gwg, wsym, soft, gmat):
+def cuda_ranks(img, txt, dino, student, scale, W, gwg, wsym, soft, gmat, gout=None):
     """Every rank of a W-rank weighted job through the C ABI on cuda:0 (the two collectives done by hand), with or
-    without DSOFT_F_GMAT.  Returns per rank the losses and the four gradients."""
+    without DSOFT_F_GMAT, for the six upstream gradients gout (default: d total_loss = 1).  Returns per rank the
+    losses and the four gradients."""
     from dinosoft_b200 import _cabi
     from dinosoft_b200.loss import CudaBackend
 
@@ -62,7 +63,8 @@ def cuda_ranks(img, txt, dino, student, scale, W, gwg, wsym, soft, gmat):
         for r, pl in enumerate(plans):
             states[r][off:off + W * n] = full
             be.forward(pl, gathered, ls, lam, states[r], scratch[r], lse_all[r], losses[r], None, phase=6)
-    gout = torch.tensor([0.0, 0.0, 0.0, 0.0, 1.0, 0.0], dtype=torch.float32, device=dev)  # d total_loss = 1
+    gout = torch.tensor([0.0, 0.0, 0.0, 0.0, 1.0, 0.0] if gout is None else list(gout), dtype=torch.float32,
+                        device=dev)
     out = []
     for r, pl in enumerate(plans):
         sc = torch.empty(pl.scratch_numel, dtype=torch.float32, device=dev)

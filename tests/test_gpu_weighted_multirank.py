@@ -15,6 +15,7 @@ import pytest
 import torch
 
 from gpu_util import rel_err, synth
+from test_gpu_multirank import seeded
 from weighted_rows_ref import weighted_ce_global_rows, weighted_ce_rows_branch
 
 pytestmark = pytest.mark.gpu
@@ -39,8 +40,9 @@ def student_of(img, Dd, seed):
     return ((img @ mix) * 2.5 + 0.1 * torch.randn(img.shape[0], Dd, generator=g)).to(torch.bfloat16).float()
 
 
-def oracle_ranks(oracle, img, txt, dino, student, scale, W, gwg, wsym, soft):
-    """Per-rank loss terms and gradients in fp64 (per-rank gradient convention of test_gpu_multirank.py)."""
+def oracle_ranks(oracle, img, txt, dino, student, scale, W, gwg, wsym, soft, gout=None):
+    """Per-rank loss terms and gradients in fp64 (per-rank gradient convention of test_gpu_multirank.py), of
+    sum_k gout[k] * term_k (default: of total_loss)."""
     lam = lambdas(soft)
     cfg = oracle.OracleConfig(lambda_original=lam[0], lambda_soft=lam[1], soft_mode="kl_teacher" if soft else "none",
                               teacher_temp=TEACHER_TEMP, soft_dino_to_text=soft, text_lambda=lam[2],
@@ -75,8 +77,8 @@ def oracle_ranks(oracle, img, txt, dino, student, scale, W, gwg, wsym, soft):
     if gwg:
         im, tx, sc, st = leafs()
         per = [rank_terms(im, tx, sc, st, r) for r in range(W)]
-        g_sc = [torch.autograd.grad(p["total_loss"], sc, retain_graph=True)[0] for p in per]
-        sum(p["total_loss"] for p in per).backward()
+        g_sc = [torch.autograd.grad(seeded(p, gout), sc, retain_graph=True)[0] for p in per]
+        sum(seeded(p, gout) for p in per).backward()
         for r in range(W):
             rows = slice(r * b, (r + 1) * b)
             out.append(dict(terms=per[r], d_image=im.grad[rows], d_text=tx.grad[rows],
@@ -85,15 +87,16 @@ def oracle_ranks(oracle, img, txt, dino, student, scale, W, gwg, wsym, soft):
         for r in range(W):
             im, tx, sc, st = leafs()
             p = rank_terms(im, tx, sc, st, r)
-            p["total_loss"].backward()
+            seeded(p, gout).backward()
             rows = slice(r * b, (r + 1) * b)
             out.append(dict(terms=p, d_image=im.grad[rows], d_text=tx.grad[rows],
                             d_student=None if st is None else st.grad[rows], d_scale=float(sc.grad)))
     return out
 
 
-def cuda_ranks(img, txt, dino, student, scale, W, gwg, wsym, soft, want_dbg=True):
-    """Every rank of a W-rank job through the C ABI on cuda:0, the two collectives done by hand."""
+def cuda_ranks(img, txt, dino, student, scale, W, gwg, wsym, soft, want_dbg=True, gout=None):
+    """Every rank of a W-rank job through the C ABI on cuda:0, the two collectives done by hand; gout: the six
+    upstream gradients (default: d total_loss = 1)."""
     from dinosoft_b200 import _cabi
     from dinosoft_b200.loss import CudaBackend
 
@@ -137,7 +140,8 @@ def cuda_ranks(img, txt, dino, student, scale, W, gwg, wsym, soft, want_dbg=True
             states[r][off:off + W * n] = full
             be.forward(pl, gathered, ls, lam, states[r], scratch[r], lse_all[r], losses[r],
                        dbgs[r] if want_dbg else None, phase=6)
-    gout = torch.tensor([0.0, 0.0, 0.0, 0.0, 1.0, 0.0], dtype=torch.float32, device=dev)  # d total_loss = 1
+    gout = torch.tensor([0.0, 0.0, 0.0, 0.0, 1.0, 0.0] if gout is None else list(gout), dtype=torch.float32,
+                        device=dev)
     out = []
     for r, pl in enumerate(plans):
         sc = torch.empty(pl.scratch_numel, dtype=torch.float32, device=dev)
