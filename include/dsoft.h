@@ -27,8 +27,9 @@ extern "C" {
 
 #define DSOFT_VERSION 260 /* 0.2.6: SigLIP loss (DSOFT_F_SIGLIP, dsoft_siglip_*), later extended without a number
                              change by DistillClipLoss (DSOFT_F_DISTILL, dsoft_distill_*: additions only, nothing
-                             existing changed) and by kNN top-k (dsoft_knn_scratch_bytes, dsoft_knn_topk:
-                             additions only); 0.2.5: retrieval ranks
+                             existing changed), by kNN top-k (dsoft_knn_scratch_bytes, dsoft_knn_topk:
+                             additions only) and by embedding geometry (dsoft_geometry_scratch_bytes,
+                             dsoft_geometry: additions only); 0.2.5: retrieval ranks
                              (dsoft_retrieval_ranks); 0.2.4: weighted plans accept the fused
                              backward (no DSOFT_F_GMAT); 0.2.3: weighted
                              CE branch at world > 1 (phases 5 / 6, dsoft_plan_lse_rows, dsoft_plan_wsigma_info) */
@@ -239,6 +240,33 @@ size_t dsoft_knn_scratch_bytes(int32_t n_q, int32_t n_k, int32_t k);
 int dsoft_knn_topk(const void* q_dev, const void* k_dev, int32_t width, int32_t n_q, int32_t n_k, int32_t k,
                    const float* key_scale_dev, const float* query_scale_dev, float* values_dev, int32_t* indices_dev,
                    void* scratch_dev, void* stream);
+
+/* Embedding geometry (Wang & Isola's uniformity and alignment, cosine histograms) without an [n_a x n_b] matrix.
+ *   cos_ij = <a_i, b_j> * b_scale_dev[j] * a_scale_dev[i]   (bf16 operands [n][width] row-major, fp32 accumulation, a
+ *   NULL scale is 1; pass 1/||row|| of the values the kernel multiplies for cosines)
+ * One set: n_b = 0, the pairs i < j of the n_a >= 2 rows; b_dev is the column operand of the same rows (NULL: a_dev)
+ * and the column scale is a_scale_dev.  Two sets: n_a, n_b >= 1; t(j) = text_image_dev[j], the row of a that column j
+ * belongs to (NULL: t(j) = j, which needs n_a == n_b); the positives are the pairs (t(j), j), the negatives all others.
+ * Split operands a = [hi | lo | hi], b = [hi | hi | lo] (width = 3 d) serve fp32 / fp16 features, as for
+ * dsoft_knn_topk.
+ *   sums_dev (fp64 [2], written): [0] = sum over the one set's pairs, or the negatives, of 2^(kappa (cos - 1)) with
+ *     kappa = 2 t log2(e), i.e. exp(2 t (cos - 1)); 0 when t == 0 (0 <= t <= 20, else DSOFT_EINVAL)
+ *     [1] = two sets: sum over the positives of max(2 - 2 cos, 0)^(alpha / 2) (alpha > 0); one set: 0
+ *   hist_dev (uint64, written; may be NULL when bins == 0): [bins + 2] per histogram, the bins equal-width over
+ *     [lo, hi) with the last one closed (numpy.histogram's convention), then the counts below lo and above hi.  One
+ *     set: one histogram over the pairs; two sets: [0] the positives, [1] the negatives.  0 <= bins <= 256.
+ *   pos_cos_dev (fp32 [n_b], or NULL; two sets only): the positives' cosines.
+ * The positives come from an fp32 pre-pass over the same operands, and the tile pass masks them, so each is counted
+ * once.  Map entries must lie in [0, n_a) (not checked on the device: a column whose entry is out of range counts
+ * nothing).  Both sums reduce fixed-size fp64 partials in a fixed order: repeated calls are bit-identical.
+ * Operands and scratch 16-byte aligned, width a multiple of 8; scratch_dev holds dsoft_geometry_scratch_bytes(n_a,
+ * n_b, bins) bytes for the current device, O(n_a + n_b) (0: invalid arguments or no sm_100 device).  Asynchronous on
+ * `stream`, no host synchronisation (graph-capturable). */
+size_t dsoft_geometry_scratch_bytes(int32_t n_a, int32_t n_b, int32_t bins);
+int dsoft_geometry(const void* a_dev, const void* b_dev, int32_t width, int32_t n_a, int32_t n_b,
+                   const float* a_scale_dev, const float* b_scale_dev, const int32_t* text_image_dev, float t,
+                   float alpha, float lo, float hi, int32_t bins, double* sums_dev, unsigned long long* hist_dev,
+                   float* pos_cos_dev, void* scratch_dev, void* stream);
 
 /* SigLIP sigmoid loss of a DSOFT_F_SIGLIP plan (open_clip SigLipLoss).  z_ij = s <I_i, T_j> + beta over the bf16
  * image | text columns of `gathered` (fp32 accumulation, s and beta applied in fp32), l_ij = +1 for j == i (global

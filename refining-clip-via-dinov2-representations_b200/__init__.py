@@ -13,6 +13,8 @@ Import as ``dinosoft_b200`` (see the shim at the repo root).  Contents:
     retrieval.py  retrieval ranks and R@K (open_clip get_clip_metrics) on the Gram-tile kernel, no N x N logits
     knn.py       kNN top-k neighbours and DINO's weighted kNN classifier on the Gram-tile kernel: per-strip top-k
                  lists in registers + a merge, no N_query x N_key score matrix
+    geometry.py  embedding geometry (Wang & Isola uniformity and alignment, anisotropy, pairwise-cosine histograms)
+                 on the Gram-tile kernel, no N x N matrix
     siglip.py    SigLipLoss drop-in (open_clip SigLipLoss): sigmoid loss and its logit gradient in one tile pass,
                  backward = the two gradient GEMMs, no B x B logit matrix
     distill.py   DistillClipLoss drop-in (open_clip DistillClipLoss): student and teacher row statistics in the
@@ -29,6 +31,7 @@ from .graphed import make_graphed
 from .pair_stats import pair_stats
 from .retrieval import clip_metrics, retrieval_ranks
 from .knn import knn_classify, knn_topk
+from .geometry import embedding_geometry, image_text_geometry
 from .siglip import SigLipLoss
 from .distill import DistillClipLoss
 from .loss import (
@@ -58,6 +61,8 @@ __all__ = [
     "clip_metrics",
     "knn_topk",
     "knn_classify",
+    "embedding_geometry",
+    "image_text_geometry",
     "CyCLIPLoss",
     "SigLipLoss",
     "DistillClipLoss",

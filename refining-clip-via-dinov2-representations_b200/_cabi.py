@@ -66,6 +66,10 @@ PROTOTYPES = {
     "dsoft_knn_scratch_bytes": (C.c_size_t, [C.c_int32, C.c_int32, C.c_int32]),
     "dsoft_knn_topk": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_void_p,
                                  C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "dsoft_geometry_scratch_bytes": (C.c_size_t, [C.c_int32, C.c_int32, C.c_int32]),
+    "dsoft_geometry": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p,
+                                 C.c_void_p, C.c_float, C.c_float, C.c_float, C.c_float, C.c_int32, C.c_void_p,
+                                 C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "dsoft_siglip_g_bytes": (C.c_size_t, [C.c_void_p]),
     "dsoft_siglip_forward": (C.c_int, [C.c_void_p] * 9),
     "dsoft_siglip_backward": (C.c_int, [C.c_void_p] * 11),

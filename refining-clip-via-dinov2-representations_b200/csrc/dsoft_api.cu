@@ -2586,6 +2586,217 @@ extern "C" int dsoft_knn_topk(const void* q_dev, const void* k_dev, int32_t widt
   return knn_launch<MODE_TOPK>(tm, P, rbs, sp.nsplit, n_q, k, values_dev, indices_dev, st);
 }
 
+// ------------------------------------------------------------------------------------------------
+// Embedding geometry (Wang & Isola's uniformity, cosine histograms, alignment) on the Gram-tile kernel: MODE_GEOM sums
+// the exponentials and counts the histogram of the pairs in scope.  Two sets take their positives from an fp32
+// pre-pass (gm_pos_kernel) and the tile pass masks them, so every positive is counted once.  Nothing of size
+// n_a x n_b exists.
+// Scratch: column scale [ncols padded to 256] fp32 | t(j) [same] int32 | tile partials [CTAs] fp64 |
+//          positives' partials [pos_blocks] fp64
+// ------------------------------------------------------------------------------------------------
+struct GeomPlan {
+  int ncols, ncols_pad, tps, nsplit, ctas, pos_blocks;
+};
+static bool geom_args_ok(int n_a, int n_b, int bins) {
+  return (n_b == 0 ? n_a >= 2 : (n_a >= 1 && n_b >= 1)) && bins >= 0 && bins <= GEOM_BINS_MAX;
+}
+static GeomPlan geom_plan(int n_a, int n_b, int sms) {
+  GeomPlan g;
+  const bool one = n_b == 0;
+  g.ncols = one ? n_a : n_b;
+  g.ncols_pad = static_cast<int>(rk_cols(g.ncols));
+  const int rbs = ceil_div(n_a, BM), ntiles = ceil_div(g.ncols, 2 * BN);
+  // one set: the upper block triangle in chunks from the row's end, as dsoft_pair_stats; two sets: the rectangle
+  const int tps = one ? std::max(4, ceil_div(ntiles, 10)) : choose_split(rbs, 1, ntiles, sms).tps;
+  g.tps = std::min(tps, 1 << 16);  // a CTA's 32-bit histogram counts: 8 warps x 32 rows x 128 columns per tile
+  g.nsplit = ceil_div(ntiles, g.tps);
+  g.ctas = (rbs + 1) / 2 * 2 * g.nsplit;
+  g.pos_blocks = one ? 0 : std::min(ceil_div(n_b, 8), 1024);
+  return g;
+}
+
+extern "C" size_t dsoft_geometry_scratch_bytes(int32_t n_a, int32_t n_b, int32_t bins) {
+  if (!geom_args_ok(n_a, n_b, bins)) return 0;
+  int sms = 0;
+  if (query_num_sms(&sms)) return 0;
+  const GeomPlan g = geom_plan(n_a, n_b, sms);
+  return 8 * static_cast<size_t>(g.ncols_pad) + 8 * static_cast<size_t>(g.ctas + g.pos_blocks);
+}
+
+// t(j) padded to whole tiles with -1 (mapped two sets), and the histograms zeroed
+__global__ void gm_init_kernel(const int32_t* __restrict__ tmap_in, int n, int ncols_pad, int* __restrict__ tmap,
+                               unsigned long long* __restrict__ hist, int nhist) {
+  for (int j = blockIdx.x * blockDim.x + threadIdx.x; j < max(ncols_pad, nhist); j += gridDim.x * blockDim.x) {
+    if (tmap_in && j < ncols_pad) tmap[j] = j < n ? tmap_in[j] : -1;
+    if (j < nhist) hist[j] = 0ull;
+  }
+}
+
+// Two sets, the positives: one warp per caption j over a fixed grid (so the partials always add in the same order).
+// cos = <a_t(j), b_j> b_scale[j] a_scale[t(j)] in fp32 from the bf16 operands, as rk_thr_kernel; the positive
+// histogram in shared memory, flushed once per block into the 64-bit counters; (2 - 2 cos)^(alpha / 2) in fp64 into
+// the block's partial.  A map entry outside [0, n_a) counts nothing.
+__global__ void __launch_bounds__(256) gm_pos_kernel(const __nv_bfloat16* __restrict__ a,
+                                                     const __nv_bfloat16* __restrict__ b, int k, int n_a, int n_b,
+                                                     const int32_t* __restrict__ tmap, const float* __restrict__ a_scale,
+                                                     const float* __restrict__ b_scale, float alpha, float lo, float hi,
+                                                     float bscale, int bins, unsigned long long* __restrict__ hist,
+                                                     float* __restrict__ pos_cos, double* __restrict__ part) {
+  __shared__ uint32_t h[GEOM_BINS_MAX + 2];
+  __shared__ double ws[8];
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, nh = bins + 2;
+  for (int q = threadIdx.x; q < nh; q += blockDim.x) h[q] = 0u;
+  __syncthreads();
+  double al = 0.0;
+  for (int j = blockIdx.x * 8 + warp; j < n_b; j += gridDim.x * 8) {
+    const int i = tmap ? tmap[j] : j;
+    if (i < 0 || i >= n_a) continue;  // warp-uniform
+    const uint4* x4 = reinterpret_cast<const uint4*>(a + static_cast<size_t>(i) * k);
+    const uint4* y4 = reinterpret_cast<const uint4*>(b + static_cast<size_t>(j) * k);
+    float acc = 0.f;
+    for (int c = lane; c < k / 8; c += 32) {
+      const uint4 x = __ldg(x4 + c), y = __ldg(y4 + c);
+      const __nv_bfloat162* xa = reinterpret_cast<const __nv_bfloat162*>(&x);
+      const __nv_bfloat162* ya = reinterpret_cast<const __nv_bfloat162*>(&y);
+#pragma unroll
+      for (int hh = 0; hh < 4; ++hh) {
+        const float2 xf = __bfloat1622float2(xa[hh]), yf = __bfloat1622float2(ya[hh]);
+        acc = fmaf(xf.x, yf.x, acc);
+        acc = fmaf(xf.y, yf.y, acc);
+      }
+    }
+#pragma unroll
+    for (int o = 16; o; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
+    if (lane == 0) {
+      const float cs = (acc * (b_scale ? b_scale[j] : 1.f)) * (a_scale ? a_scale[i] : 1.f);
+      if (pos_cos) pos_cos[j] = cs;
+      al += pow(fmax(2.0 - 2.0 * static_cast<double>(cs), 0.0), 0.5 * static_cast<double>(alpha));
+      if (bins) atomicAdd(&h[geom_bin(cs, lo, hi, bscale, bins)], 1u);
+    }
+  }
+  if (lane == 0) ws[warp] = al;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    double s = 0.0;
+    for (int w = 0; w < 8; ++w) s += ws[w];
+    part[blockIdx.x] = s;
+  }
+  if (bins)
+    for (int q = threadIdx.x; q < nh; q += blockDim.x)
+      if (h[q]) atomicAdd(hist + q, static_cast<unsigned long long>(h[q]));
+}
+
+// one block: sums[0] = the tile partials, sums[1] = the positives' partials, each reduced in a fixed order
+__global__ void __launch_bounds__(256) gm_finalize_kernel(const double* __restrict__ tile, int ntile,
+                                                          const double* __restrict__ pos, int npos,
+                                                          double* __restrict__ sums) {
+  __shared__ double s[2][256];
+  double x = 0.0, y = 0.0;
+  for (int q = threadIdx.x; q < ntile; q += 256) x += tile[q];
+  for (int q = threadIdx.x; q < npos; q += 256) y += pos[q];
+  s[0][threadIdx.x] = x;
+  s[1][threadIdx.x] = y;
+  __syncthreads();
+  for (int o = 128; o; o >>= 1) {
+    if (threadIdx.x < o) {
+      s[0][threadIdx.x] += s[0][threadIdx.x + o];
+      s[1][threadIdx.x] += s[1][threadIdx.x + o];
+    }
+    __syncthreads();
+  }
+  if (threadIdx.x == 0) {
+    sums[0] = s[0][0];
+    sums[1] = s[1][0];
+  }
+}
+
+extern "C" int dsoft_geometry(const void* a_dev, const void* b_dev, int32_t width, int32_t n_a, int32_t n_b,
+                              const float* a_scale_dev, const float* b_scale_dev, const int32_t* text_image_dev,
+                              float t, float alpha, float lo, float hi, int32_t bins, double* sums_dev,
+                              unsigned long long* hist_dev, float* pos_cos_dev, void* scratch_dev, void* stream) {
+  if (!a_dev || !sums_dev || !scratch_dev || (bins > 0 && !hist_dev)) return fail(DSOFT_EINVAL, "null argument");
+  const bool one = n_b == 0;
+  if (width <= 0 || width % 8)
+    return fail(DSOFT_EINVAL, "the feature width must be a positive multiple of 8 (width=%d)", width);
+  if (!geom_args_ok(n_a, n_b, bins))
+    return fail(DSOFT_EINVAL, "need n_a >= 2 for one set (n_b = 0) or n_a, n_b >= 1 for two, and 0 <= bins <= %d "
+                              "(n_a=%d n_b=%d bins=%d)", GEOM_BINS_MAX, n_a, n_b, bins);
+  if (!(t >= 0.f && t <= 20.f)) return fail(DSOFT_EINVAL, "t must lie in [0, 20] (t=%g)", t);
+  if (bins > 0 && !(std::isfinite(lo) && std::isfinite(hi) && lo < hi))
+    return fail(DSOFT_EINVAL, "the histogram range needs finite lo < hi (lo=%g hi=%g)", lo, hi);
+  if (one && (text_image_dev || pos_cos_dev))
+    return fail(DSOFT_EINVAL, "one set (n_b = 0) has no positives: text_image and pos_cos must be NULL");
+  if (!one && !(alpha > 0.f && std::isfinite(alpha))) return fail(DSOFT_EINVAL, "alpha must be > 0 (alpha=%g)", alpha);
+  if (!one && !b_dev) return fail(DSOFT_EINVAL, "two sets need b_dev");
+  if (!one && !text_image_dev && n_a != n_b)
+    return fail(DSOFT_EINVAL, "without a caption -> image map n_a must equal n_b (%d, %d)", n_a, n_b);
+  const void* bcol = b_dev ? b_dev : a_dev;
+  for (const void* q : {a_dev, bcol, static_cast<const void*>(scratch_dev)})
+    if (reinterpret_cast<uintptr_t>(q) % 16) return fail(DSOFT_EINVAL, "operands and scratch must be 16-byte aligned");
+  int sms = 0, rc = query_num_sms(&sms);
+  if (rc) return rc;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const GeomPlan g = geom_plan(n_a, n_b, sms);
+  float* cscale = static_cast<float*>(scratch_dev);
+  int* tmap = reinterpret_cast<int*>(cscale + g.ncols_pad);
+  double* tpart = reinterpret_cast<double*>(tmap + g.ncols_pad);
+  double* ppart = tpart + g.ctas;
+  const int nh = bins + 2, nhist = bins ? (one ? nh : 2 * nh) : 0;
+  const float bscale = bins ? static_cast<float>(static_cast<double>(bins) / (static_cast<double>(hi) - lo)) : 0.f;
+  const int grid = std::min(ceil_div(std::max(g.ncols_pad, nhist), 256), 4 * sms);
+  knn_scale_kernel<<<grid, 256, 0, st>>>(one ? a_scale_dev : b_scale_dev, g.ncols, g.ncols_pad, cscale);
+  CUDA_TRY(cudaGetLastError());
+  gm_init_kernel<<<grid, 256, 0, st>>>(one ? nullptr : text_image_dev, g.ncols, g.ncols_pad, tmap, hist_dev, nhist);
+  CUDA_TRY(cudaGetLastError());
+  if (!one) {
+    gm_pos_kernel<<<g.pos_blocks, 256, 0, st>>>(static_cast<const __nv_bfloat16*>(a_dev),
+                                                static_cast<const __nv_bfloat16*>(b_dev), width, n_a, n_b,
+                                                text_image_dev, a_scale_dev, b_scale_dev, alpha, lo, hi, bscale, bins,
+                                                hist_dev, pos_cos_dev, ppart);
+    CUDA_TRY(cudaGetLastError());
+  }
+  const bool tiles = bins > 0 || t > 0.f;  // two sets without a histogram: the pre-pass is the whole result
+  if (tiles) {
+    TileMaps tm;
+    const CUtensorMapDataType bf = CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
+    if ((rc = make_map(&tm.m[0], a_dev, n_a, width, static_cast<size_t>(width), bf, 64))) return rc;
+    if ((rc = make_map(&tm.m[1], bcol, g.ncols, width, static_cast<size_t>(width), bf, 64))) return rc;
+    tm.m[2] = tm.m[3] = tm.g[0] = tm.g[1] = tm.m[0];
+    FwdParams P;
+    memset(&P, 0, sizeof(P));
+    P.nprod = 1;
+    P.a_map[0] = 0;
+    P.b_map[0] = 1;
+    P.kchunks[0] = ceil_div(width, BK);
+    P.bn = 2 * BN;
+    P.row0 = 0;
+    P.b = n_a;
+    P.col0 = 0;
+    P.ncols = g.ncols;
+    P.ntiles = ceil_div(g.ncols, 2 * BN);
+    P.tiles_per_split = g.tps;
+    P.npart = 2 * g.nsplit;
+    P.tri = one ? 1 : 0;  // one set: upper block triangle, pairs i < j
+    P.gm_mapped = (!one && text_image_dev) ? 1 : 0;
+    P.ncolvec = P.gm_mapped ? 2 : 1;
+    P.colvec[0] = cscale;
+    P.colvec[1] = reinterpret_cast<const float*>(tmap);
+    P.gm_rscale = a_scale_dev;
+    P.gm_kappa = static_cast<float>(2.0 * t * 1.4426950408889634);
+    P.gm_bins = bins;
+    P.gm_lo = lo;
+    P.gm_hi = hi;
+    P.gm_bscale = bscale;
+    P.gm_hist = (bins && !one) ? hist_dev + nh : hist_dev;
+    P.gm_part = tpart;
+    if ((rc = set_smem(dsoft_fwd_kernel<MODE_GEOM, 2>, FWD_SMEM_BYTES))) return rc;
+    if ((rc = launch_fwd_pair(dsoft_fwd_kernel<MODE_GEOM, 2>, ceil_div(n_a, BM), g.nsplit, st, tm, P))) return rc;
+  }
+  gm_finalize_kernel<<<1, 256, 0, st>>>(tpart, tiles ? g.ctas : 0, ppart, g.pos_blocks, sums_dev);
+  CUDA_TRY(cudaGetLastError());
+  return 0;
+}
+
 // phase 0: the whole forward; of a DSOFT_SYM_W plan: 4 = operand statistics, 1 = the soft part up to the column-sum
 // exchange, 3 = the CLIP part (independent of 1 and of the exchange), 2 = finalize; of a weighted plan: 5 = up to the
 // weighted row statistics (row stds), 6 = median onward

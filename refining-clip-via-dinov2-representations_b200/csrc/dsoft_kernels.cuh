@@ -71,6 +71,9 @@ constexpr int MODE_DIST_G = 17;   // DistillClipLoss logit gradient of one direc
 constexpr int MODE_TOPK = 18;     // kNN top-k (DINO knn_classifier): per query row and 128-column strip of a column
 constexpr int MODE_TOPK32 = 19;   // split, the 64 (MODE_TOPK32: 32) best (score, key index) in registers
 __host__ __device__ constexpr int topk_list(int mode) { return mode == MODE_TOPK32 ? 32 : 64; }
+constexpr int MODE_GEOM = 20;     // embedding geometry (Wang & Isola uniformity, cosine histograms): per pair of a Gram
+                                  // matrix of scaled rows, one exponential and one histogram count
+constexpr int GEOM_BINS_MAX = 256;  // histogram bins; each epilogue warp counts into [bins + 2] (below, above) in smem
 
 // scalar block computed on device by prep_scalars_kernel (no host sync on logit_scale)
 enum {
@@ -201,6 +204,15 @@ struct FwdParams {
   const float* tk_qscale;   // per query: 1/||q_i||, or null (1)
   float* tk_val;            // [npart][b][topk_list(MODE)] partial lists, by decreasing score (ties: increasing index)
   int* tk_idx;              // their key indices (INT_MAX in slots no key filled)
+  // ---- embedding geometry (MODE_GEOM): cos_ij = <a_i, b_j> * colvec[0][j] * gm_rscale[i]; one set (tri): the pairs
+  // i < j; two sets: every pair but the positives (t(j) == i: colvec[1] as int bits when gm_mapped, else j == i)
+  const float* gm_rscale;   // per row: 1/||a_i||
+  int gm_mapped;
+  float gm_kappa;           // 2 t log2(e): the pair adds 2^(kappa (cos - 1)); 0: no uniformity sum
+  int gm_bins;              // 0: no histogram
+  float gm_lo, gm_hi, gm_bscale;         // bin = floor((cos - lo) * bscale), bscale = bins / (hi - lo)
+  unsigned long long* gm_hist;           // [bins + 2]: the bins, below lo, above hi (+= per CTA)
+  double* gm_part;          // [CTAs]: this CTA's sum of the exponentials, by blockIdx.y * gridDim.x + blockIdx.x
 };
 
 struct BwdParams {
@@ -455,7 +467,7 @@ struct FwdMode {
   FwdCols cols;
   bool writes_g;  // streams fp16 logit-gradient tiles through TMA stores (maps.g, L2 policies)
   bool regsplit;  // setmaxnreg hand-over (40 / 232) from the producer / MMA / allocator warps to the epilogue; the
-                  // ranks, distill and kNN epilogues fit the even split (168 registers) without spills
+                  // ranks, distill, kNN and geometry epilogues fit the even split (168 registers) without spills
   int epi_warps;
 };
 __host__ __device__ constexpr FwdMode fwd_mode(int mode) {
@@ -471,6 +483,7 @@ __host__ __device__ constexpr FwdMode fwd_mode(int mode) {
     case MODE_RANKS:
     case MODE_TOPK:
     case MODE_TOPK32:
+    case MODE_GEOM:
     case MODE_DIST_FWD: return {6, 6, COLS_COLVEC, false, false, 8};
     case MODE_DIST_G: return {5, 5, COLS_COLVEC, true, false, 8};
     case MODE_CLIP_G:
@@ -480,6 +493,12 @@ __host__ __device__ constexpr FwdMode fwd_mode(int mode) {
   }
 }
 __host__ __device__ constexpr int fwd_epi_warps(int mode) { return fwd_mode(mode).epi_warps; }
+
+// Histogram slot of a cosine (MODE_GEOM and the positives' pre-pass): bins equal-width over [lo, hi), the last one
+// closed (numpy.histogram's convention); nb: below lo, nb + 1: above hi
+__device__ __forceinline__ int geom_bin(float x, float lo, float hi, float bscale, int nb) {
+  return x < lo ? nb : (x > hi ? nb + 1 : min(static_cast<int>((x - lo) * bscale), nb - 1));
+}
 __host__ __device__ constexpr int fwd_threads(int mode) { return 32 * (EPI_WARP0 + fwd_epi_warps(mode)); }
 
 template <int MODE, int CG>
@@ -1054,6 +1073,80 @@ dsoft_fwd_kernel(const __grid_constant__ TileMaps maps, const __grid_constant__ 
         for (int k = 0; k < KL / 4; ++k) {
           dv[k] = make_float4(tv[4 * k], tv[4 * k + 1], tv[4 * k + 2], tv[4 * k + 3]);
           di[k] = make_int4(ti[4 * k], ti[4 * k + 1], ti[4 * k + 2], ti[4 * k + 3]);
+        }
+      }
+    } else if constexpr (MODE == MODE_GEOM) {
+      // ---------------------------------------------------------------- embedding geometry
+      // cos = <a_i, b_j> times the staged column scale and this row's scale, over the pairs in scope: one set (P.tri,
+      // upper block triangle) the pairs i < j, two sets every pair but the positives (masked as in MODE_RANKS).  Per
+      // pair, 2^(kappa (cos - 1)) goes into fp32 sums per tile (at most 128 terms <= 1 per thread), promoted to fp64
+      // across tiles: a thread sees 10^5 - 10^6 terms, and one fp32 sum would lose ~1e-3 relative.  The exponent's
+      // maximum is 0 (cos <= 1), so no running maximum is needed.  And one count goes into this warp's histogram in
+      // shared memory.  At the end the CTA writes its fp64 sum to its own slot, which a finalize kernel reduces in a
+      // fixed order (no float atomics: bit-identical across calls), and adds its histogram, summed over the warps, to
+      // the 64-bit counters.  A warp's 32-bit counters take at most 32 x 128 columns per tile of its split.
+      static_assert(8 * (GEOM_BINS_MAX + 2) * 4 + 8 * 8 <= 16384, "histograms behind colbuf, in front of the barriers");
+      const int nb = P.gm_bins, nh = nb + 2;
+      const int et = threadIdx.x - 32 * EPI_WARP0;                                       // 0 .. 255
+      uint32_t* hist = reinterpret_cast<uint32_t*>(smem + 6 * 2 * TILE_BYTES + 16384);  // [8][nh], behind colbuf
+      double* wsum = reinterpret_cast<double*>(hist + 8 * (GEOM_BINS_MAX + 2));         // [8]
+      for (int k = et; k < 8 * nh; k += NUM_EPI_THREADS) hist[k] = 0u;
+      named_bar_sync(1, NUM_EPI_THREADS);
+      uint32_t* whist = hist + (warp - EPI_WARP0) * nh;
+      const bool live_row = li < P.b;
+      const bool rows_edge = rb * BM + q * 32 + 32 > P.b;  // warp-uniform: some rows of the warp are past b
+      const float rs = (P.gm_rscale && live_row) ? P.gm_rscale[li] : 1.f;
+      const float kap = P.gm_kappa, lo = P.gm_lo, hi = P.gm_hi, bscale = P.gm_bscale;
+      const bool tri = P.tri != 0, mapped = P.gm_mapped != 0;
+      double usum = 0.0;
+      // 256-column tiles: two TMEM slots and two column buffers, both picked by the parity of the tile's position
+      for (int t = t0; t < t1; ++t) {
+        const int n = t - t0, par = n & 1;
+        mbar_wait(smem_u32(&col_full[par]), static_cast<uint32_t>(n >> 1) & 1);
+        mbar_wait(smem_u32(&s_full[par]), static_cast<uint32_t>(n >> 1) & 1);
+        tc_fence_after();
+        const float* cs = colbuf + par * COL_VECS * CT + half * 128;
+        const int* tmap = reinterpret_cast<const int*>(cs + CT);
+        const uint32_t taddr = lane_addr + par * CT + half * 128;
+        float tsum[2] = {0.f, 0.f};
+#pragma unroll 1
+        for (int c = 0; c < 4; ++c) {
+          const int gj0 = t * CT + half * 128 + c * 32;
+          tmem_ld32(taddr + c * 32, v);
+          if (c == 3) {
+            tc_fence_before();
+            release_slot(par);
+          }
+          if (gj0 >= P.ncols || (tri && gj0 + 31 <= gw0)) continue;  // warp-uniform: no pair of the chunk in scope
+          // warp-uniform: some entries need the mask (rows and chunks are both 32-aligned: gj0 == gw0 holds the diagonal)
+          const bool edge = rows_edge || gj0 + 32 > P.ncols || (tri ? gj0 <= gw0 + 31 : gj0 == gw0);
+#pragma unroll
+          for (int e = 0; e < 32; ++e) {
+            const int gj = gj0 + e;
+            const float x = (v[e] * cs[c * 32 + e]) * rs;
+            bool ok = !edge || (live_row && gj < P.ncols && (tri ? gj > gi : (mapped || gj != gi)));
+            if (mapped) ok = ok && tmap[c * 32 + e] != gi;
+            if (kap != 0.f) tsum[e & 1] += ok ? fast_exp2(fmaf(kap, x, -kap)) : 0.f;
+            if (nb && ok) atomicAdd(whist + geom_bin(x, lo, hi, bscale, nb), 1u);
+          }
+        }
+        usum += static_cast<double>(tsum[0] + tsum[1]);
+        mbar_arrive(smem_u32(&col_empty[par]));
+      }
+#pragma unroll
+      for (int o = 16; o; o >>= 1) usum += __shfl_xor_sync(0xffffffffu, usum, o);
+      if (lane == 0) wsum[warp - EPI_WARP0] = usum;
+      named_bar_sync(1, NUM_EPI_THREADS);
+      if (et == 0) {
+        double s = 0.0;
+        for (int w = 0; w < 8; ++w) s += wsum[w];
+        P.gm_part[blockIdx.y * gridDim.x + blockIdx.x] = s;
+      }
+      if (nb) {
+        for (int k = et; k < nh; k += NUM_EPI_THREADS) {
+          uint32_t s = 0u;
+          for (int w = 0; w < 8; ++w) s += hist[w * nh + k];
+          if (s) atomicAdd(P.gm_hist + k, static_cast<unsigned long long>(s));
         }
       }
     } else if constexpr (MODE == MODE_LINEAR) {
